@@ -41,7 +41,15 @@ def parse():
     ap.add_argument("--no-value-check", action="store_true", help="skip the sampled wire-value comparison with the oracle")
     ap.add_argument("--verdicts-only", action="store_true",
                     help="do not keep the live wires readable: slot re-use + dead-store elimination (not the headline)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (float64): every witness's verdict and "
+                         "the values of a fixed, seeded sample of wires x witnesses, so that two builds can be compared")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    return args
 
 
 FIELD = {"bls381": 0x73eda753299d7d483339d80809a1d80553bda402fffe5bfeffffffff00000001,
@@ -129,6 +137,31 @@ def cpu_reference_run(circ_mod, flat, p, circuit, gates, n_counted, witnesses, n
     res = flat.eval_batch(gates, circuit.const_pool, p.to_bytes(eb, "little"), None, witnesses, n, n_threads=n_threads)
     dt = time.perf_counter() - t0
     return n_counted * n / dt, dt, res
+
+
+DUMP_WIRES = 4096          # wire-value sample of --dump-outputs: 4096 wires x 16 witnesses, 4 MB at 8 limbs
+DUMP_WITNESSES = 16
+
+
+def dump_outputs(out_dir, be, circuit, ff, w_np, corrupt_local, eb, wires_readable):
+    """--dump-outputs: the verdicts of the whole batch (first_fail_seq = -1 for a satisfied witness) and, when the wires are
+    kept readable, the values of a seeded sample of wires for a seeded sample of this rank's satisfied witnesses, as
+    little-endian u32 limbs [witness, wire, limb]; float64 holds every verdict and limb exactly"""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "verdict_ok.npy"), (ff >= (1 << 40)).astype(np.float64))
+    np.save(os.path.join(out_dir, "first_fail_seq.npy"), np.where(ff >= (1 << 40), -1, ff).astype(np.float64))
+    if not wires_readable:
+        return
+    rng = np.random.default_rng(SEED + 11)
+    nw = circuit.n_wires
+    wires = np.sort(rng.choice(nw, size=min(DUMP_WIRES, nw), replace=False))
+    good = np.array([j for j in range(len(w_np)) if j not in corrupt_local])
+    picks = np.sort(rng.choice(good, size=min(DUMP_WITNESSES, len(good)), replace=False))
+    handles = [be.scope_lookup(int(i)) for i in wires]
+    vals = np.zeros((len(picks), len(wires), eb), dtype=np.uint8)
+    for r, j in enumerate(picks):
+        vals[r] = [np.frombuffer(x.to_bytes(eb, "little"), np.uint8) for x in be.read_values(int(j), handles, eb)]
+    np.save(os.path.join(out_dir, "wire_values.npy"), vals.view("<u4").astype(np.float64))
 
 
 def workload_name(args):
@@ -312,12 +345,14 @@ def main():
     be.upload_inputs(None, w_host, n_local)
     st = be.stats()
     for _ in range(args.warmup):
-        v = run_resident()
-    check(first_fail_vector(v)[lo:hi])
+        run_resident()
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
     dev_ms, wall_ms, lv_ms, ff, v = timed(run_resident, args.steps)
+    check(ff[lo:hi])
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, be, circuit, ff, w_np, corrupt_local, eb, not args.verdicts_only)
     launches = be.timing()["kernel_launches"] * args.steps
     level_launches = be.timing()["level_launches"]
     ms_per_step = dev_ms / args.steps

@@ -109,14 +109,14 @@ def test_flatten_cuts_messages_every_100000(tmp_path):
     assert (k1 == k2).all() and (a1 == a2).all() and (bb1 == bb2).all() and len(k1) == n + 1
 
 
-def test_flatten_mode_refuses_evaluation():
+def test_flatten_mode_refuses_evaluation(tmp_path):
     z = zkb()
     msgs = STATEMENTS["example"]()
     e, _ = ours_flatten(msgs)
     with pytest.raises(z.ZkbError):
         e.get_violations()
     with pytest.raises(z.ZkbError):
-        e.flatten_to_dir("/tmp/x.sieve")
+        e.flatten_to_dir(str(tmp_path / "x.sieve"))
 
 
 @pytest.mark.parametrize("name", list(STATEMENTS))

@@ -103,3 +103,31 @@ def test_c4_2p20_rows_bn254_first_violated_row():
 def test_c5_2p22_leaf_gates_nested_for_probe_outputs():
     out = _bc().c5(10, 9, 64)                   # checks verdicts and probe wires against an independent numpy evaluation
     assert out["levels"] > 0
+
+
+def test_bench_dump_outputs_are_reproducible(tmp_path):
+    """bench.py --dump-outputs: the last timed step's verdicts and sampled wire values as float64 .npy files, consistent
+    with the JSON line, and identical across two runs with the same arguments (the inputs are seeded)"""
+    import json
+    import subprocess
+    dumps = []
+    for k in range(2):
+        d = tmp_path / f"run{k}"
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "2", "--warmup", str(k),
+                            "--log2-gates", "14", "--witnesses", "300", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr
+        line = json.loads(r.stdout.strip())
+        assert line["steps"] == 2 and line["warmup"] == k
+        files = {f.name: np.load(f) for f in d.iterdir()}
+        assert sorted(files) == ["first_fail_seq.npy", "verdict_ok.npy", "wire_values.npy"]
+        assert all(a.dtype == np.float64 for a in files.values()) and sum(a.nbytes for a in files.values()) <= 64 << 20
+        ok, ff = files["verdict_ok.npy"], files["first_fail_seq.npy"]
+        assert ok.shape == ff.shape == (300,)
+        assert int(ok.sum()) == line["verdicts"]["true"] and int((ok == 0).sum()) == line["verdicts"]["false"] > 0
+        assert ((ok == 1) == (ff == -1)).all()
+        wv = files["wire_values.npy"]
+        assert wv.shape[0] == 16 and wv.shape[2] == 8 and (wv >= 0).all() and (wv < 2 ** 32).all() and wv.any()
+        dumps.append(files)
+    for name in dumps[0]:
+        assert np.array_equal(dumps[0][name], dumps[1][name]), name
