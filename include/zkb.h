@@ -195,6 +195,8 @@ typedef struct {
                                     * arithmetic progression over the calls) */
     int64_t group_jit_state;       /* the groups' run-time specialised kernel: -2 none, -1 unavailable (the interpreter kernel
                                     * runs), 0 compiling in the background, 2 compiled, 3 loaded and in use */
+    uint64_t n_sink_ops;           /* after finalize: stored results that no gate reads (only a read-back needs them; tiles
+                                    * other than the last one run skip their stores) */
 } zkb_stats;
 int zkb_get_stats(zkb_ctx* ctx, zkb_stats* out);
 
@@ -344,6 +346,9 @@ int zkb_debug_barrier_cost(zkb_ctx* ctx, int kind, uint32_t blocks, uint32_t n_b
 /* hash of the finalized device plan (ops, assertion table, input loads, slot map): the levelizer's threaded passes must
  * give the plan its sequential form gives (ZKB_PLAN_THREADS) */
 int zkb_debug_plan_hash(zkb_ctx* ctx, uint64_t* out);
+/* device ops [first, first + n) of the finalized plan: ops4 = 4 x uint32 per op {a, b, out, meta}; values (NULL: skipped) = the
+ * SSA value each op computes (0xFFFFFFFF: not stored).  values needs a plan without slot re-use (zkb_finalize(ctx, 1)). */
+int zkb_debug_plan_ops(zkb_ctx* ctx, uint64_t first, uint64_t n, uint32_t* ops4, uint32_t* values);
 /* FlatBuffers reader -> owned structs -> writer on one size-prefixed message (round-trip tests); *out is valid until
  * the next call on this thread. */
 int zkb_debug_rewrite_message(zkb_ctx* ctx, const uint8_t* buf, size_t len, const uint8_t** out, size_t* out_len);

@@ -50,7 +50,8 @@ class ZkbStats(C.Structure):
                 ("n_device_ops", C.c_uint64), ("algo_bytes_per_witness", C.c_uint64), ("nlimb", C.c_uint32),
                 ("binary", C.c_uint32), ("tile_witnesses", C.c_uint32), ("n_tiles", C.c_uint32),
                 ("n_call_groups", C.c_uint64), ("n_group_calls", C.c_uint64),
-                ("n_group_launches", C.c_uint64), ("n_group_table_slots", C.c_uint64), ("group_jit_state", C.c_int64)]
+                ("n_group_launches", C.c_uint64), ("n_group_table_slots", C.c_uint64), ("group_jit_state", C.c_int64),
+                ("n_sink_ops", C.c_uint64)]
 
 
 class ZkbTiming(C.Structure):
@@ -78,7 +79,7 @@ EXPORTED = [
     "zkb_validator_ingest_buffer", "zkb_validator_ingest_paths", "zkb_validator_get_violations", "zkb_validator_violation",
     "zkb_validator_how_many_violations", "zkb_validator_live_wires", "zkb_validator_set_limits", "zkb_validator_last_error", "zkb_metrics_create", "zkb_metrics_destroy", "zkb_metrics_ingest_message",
     "zkb_metrics_ingest_buffer", "zkb_metrics_ingest_paths", "zkb_metrics_json", "zkb_metrics_last_error", "zkb_r1cs_load", "zkb_r1cs_check",
-    "zkb_r1cs_upload", "zkb_r1cs_run", "zkb_debug_field_ops", "zkb_debug_field_throughput", "zkb_debug_group_jit_wait", "zkb_debug_group_jit_source", "zkb_debug_gather_throughput", "zkb_debug_barrier_cost", "zkb_debug_r1cs_layout", "zkb_debug_rewrite_message", "zkb_debug_plan_hash", "zkb_debug_write_flat_relation",
+    "zkb_r1cs_upload", "zkb_r1cs_run", "zkb_debug_field_ops", "zkb_debug_field_throughput", "zkb_debug_group_jit_wait", "zkb_debug_group_jit_source", "zkb_debug_gather_throughput", "zkb_debug_barrier_cost", "zkb_debug_r1cs_layout", "zkb_debug_rewrite_message", "zkb_debug_plan_hash", "zkb_debug_plan_ops", "zkb_debug_write_flat_relation",
     "zkb_comm_unique_id", "zkb_comm_init_rank", "zkb_comm_init", "zkb_comm_info", "zkb_comm_broadcast_program", "zkb_comm_evaluate",
     "zkb_comm_run", "zkb_evaluate_sharded", "zkb_run_sharded",
 ]
@@ -171,6 +172,7 @@ _sig("zkb_debug_gather_throughput", _i, _vp, _u64, _u32, C.POINTER(C.c_double))
 _sig("zkb_debug_barrier_cost", _i, _vp, _i, _u32, _u32, C.POINTER(C.c_double))
 _sig("zkb_debug_r1cs_layout", _i, _vp, _i, _u64p, _vp, _vp, _vp)
 _sig("zkb_debug_plan_hash", _i, _vp, _u64p)
+_sig("zkb_debug_plan_ops", _i, _vp, _u64, _u64, _vp, _vp)
 _sig("zkb_debug_rewrite_message", _i, _vp, _u8p, _sz, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t))
 _sig("zkb_debug_write_flat_relation", _i, _vp, _u8p, _sz, _i, _vp, _u64, _u8p, _sz, _u64, C.POINTER(C.c_void_p),
      C.POINTER(C.c_size_t))
@@ -538,6 +540,16 @@ class GpuBackend:
         out = C.c_uint64()
         self._chk(_lib.zkb_debug_plan_hash(self._c, C.byref(out)))
         return out.value
+
+    def plan_ops(self, first: int = 0, n: int = -1, values: bool = False):
+        """device ops [first, first + n) as uint32 [n, 4] {a, b, out, meta}; with values=True also the SSA value each op
+        computes (0xFFFFFFFF: not stored; needs finalize(keep_all_values=True))"""
+        if n < 0:
+            n = self.stats()["n_device_ops"] - first
+        ops = np.zeros((n, 4), dtype=np.uint32)
+        vals = np.zeros(n, dtype=np.uint32) if values else None
+        self._chk(_lib.zkb_debug_plan_ops(self._c, first, n, ops.ctypes.data, vals.ctypes.data if values else None))
+        return (ops, vals) if values else ops
 
     def rewrite_message(self, buf: bytes) -> bytes:
         """C++ reader -> owned structs -> C++ writer (round-trip tests)"""

@@ -16,7 +16,9 @@ random_circuit  "random Add/Mul/AssertZero circuit" (configs C2, C3), SURVEY.md 
     witness-dependent assertion `Witness(k) = p - v(t); s = Add(t, k); AssertZero(s)` with k computed inside the circuit
     by the twin gates instead of being shipped as one extra witness value per assertion: at C3's size that would be
     1.5 M x 32 B = 48 MB per witness, 196 GB for the batch of 4096 -- more than a B200's HBM, let alone beside the
-    wire store.  No operand is shared between gates by construction and there are no constants.  Gate histogram:
+    wire store.  A gate and its twin share no operand, but operands are drawn independently, so the readers of one wire
+    do coincide: at 2^24, 37 % of the operand reads inside a wavefront repeat a wire another gate of that wavefront reads
+    (scripts/wavefront_reuse_model.py).  There are no constants.  Gate histogram:
     Add 50 %, Mul 41 %, AssertZero 9 % of `n_gates` (section 8(d)'s mix).
     Corrupting the mirror x'_k of a tracked input (k < n_tracked <= 64) makes every assertion whose t depends on x_k or
     x'_k fail (up to a 2^-250 coincidence): the first such assertion in program order is known from a taint pass

@@ -698,8 +698,10 @@ extern "C" int zkb_upload_inputs(zkb_ctx* c, const uint8_t* inst, uint64_t inst_
     return ZKB_OK;
 }
 
-// run one tile of witnesses through every wavefront
-static void run_tile(zkb_ctx* c, uint32_t tile, uint32_t* d_fail, uint64_t* launches, uint64_t* level_launches) {
+// run one tile of witnesses through every wavefront.  full = false: the next tile overwrites this one's wire store before
+// anything can read it back, so the level kernels skip the results no gate reads (F_SINK) and the tile is not left resident
+// (zkb_read_values re-runs it in full).  ZKB_SINK_STORES=1 stores them on every tile.
+static void run_tile(zkb_ctx* c, uint32_t tile, bool full, uint32_t* d_fail, uint64_t* launches, uint64_t* level_launches) {
     const Plan& pl = c->plan;
     const Program& p = c->prog;
     TileGeom g;
@@ -707,7 +709,9 @@ static void run_tile(zkb_ctx* c, uint32_t tile, uint32_t* d_fail, uint64_t* laun
     g.batch0 = tile << c->log2_wt;
     uint32_t wt = 1u << c->log2_wt;
     g.n_valid = std::min<uint32_t>(wt, c->n_batch - g.batch0);
-    g.pad = 0;
+    const char* ss = getenv("ZKB_SINK_STORES");
+    g.skip_mask = full || (ss && atoi(ss) != 0) ? 0u : F_SINK;
+    const int64_t resident = full ? (int64_t)tile : -1;
     uint8_t* rawflag = pl.n_raw_ops > 0 ? c->d_rawflag : nullptr;
     RawCtx rawctx;
     rawctx.rawflag = rawflag;
@@ -776,7 +780,7 @@ static void run_tile(zkb_ctx* c, uint32_t tile, uint32_t* d_fail, uint64_t* laun
                 (*launches)++;
                 if (level_launches) (*level_launches)++;
                 if (timed) cudaEventRecord(c->tile_ev[2 * tile + 1], c->stream);
-                c->resident_tile = tile;
+                c->resident_tile = resident;
                 return;
             }
             if (getenv("ZKB_DEBUG")) fprintf(stderr, "zkb: dataflow launch failed: %s\n", cudaGetErrorString(err));
@@ -797,7 +801,7 @@ static void run_tile(zkb_ctx* c, uint32_t tile, uint32_t* d_fail, uint64_t* laun
                 *launches += 2;  // marker fill + the launch
                 if (level_launches) (*level_launches)++;
                 if (timed) cudaEventRecord(c->tile_ev[2 * tile + 1], c->stream);
-                c->resident_tile = tile;
+                c->resident_tile = resident;
                 return;
             }
             if (getenv("ZKB_DEBUG")) fprintf(stderr, "zkb: dataflow launch failed: %s\n", cudaGetErrorString(err));
@@ -842,7 +846,7 @@ static void run_tile(zkb_ctx* c, uint32_t tile, uint32_t* d_fail, uint64_t* laun
         }
         if (first_level == pl.n_levels) {
             if (timed) cudaEventRecord(c->tile_ev[2 * tile + 1], c->stream);
-            c->resident_tile = tile;
+            c->resident_tile = resident;
             return;
         }
     }
@@ -882,7 +886,7 @@ static void run_tile(zkb_ctx* c, uint32_t tile, uint32_t* d_fail, uint64_t* laun
         }
     }
     if (timed) cudaEventRecord(c->tile_ev[2 * tile + 1], c->stream);
-    c->resident_tile = tile;
+    c->resident_tile = resident;
 }
 
 // SURVEY.md §8a trap 1: values >= p stay RAW in the reference.  The device works on residues, which is exact for add / mul
@@ -925,7 +929,7 @@ int ctx_run(zkb_ctx* c, zkb_verdict* out, uint32_t first, uint32_t n_total, bool
     launches++;
     {
         NvtxRange r_lv("zkb:levels");
-        for (uint32_t t = 0; t < n_tiles; t++) run_tile(c, t, c->d_first_fail + first, &launches, &level_launches);
+        for (uint32_t t = 0; t < n_tiles; t++) run_tile(c, t, t == n_tiles - 1, c->d_first_fail + first, &launches, &level_launches);
     }
     if (collective) {
         NvtxRange r_ar("zkb:verdict_allreduce");
@@ -1027,7 +1031,7 @@ extern "C" int zkb_read_values(zkb_ctx* c, uint32_t batch_idx, const zkb_wire* v
     if (c->resident_tile != (int64_t)tile) {
         uint64_t a = 0, b = 0;
         launch_fill_u32(c->d_scratch_fail, 0xFFFFFFFFu, c->n_batch, c->sm_count, c->stream);
-        run_tile(c, tile, c->d_scratch_fail, &a, &b);
+        run_tile(c, tile, true, c->d_scratch_fail, &a, &b);
     }
     // per requested value: its slot, kind and operand b (constant-pool index / stream position of an input)
     std::vector<uint32_t> slots(n), kinds(n), opbs(n);
@@ -1160,6 +1164,7 @@ extern "C" int zkb_get_stats(zkb_ctx* c, zkb_stats* s) {
         s->n_levels = c->plan.n_levels;
         s->n_device_ops = c->is_replica ? c->replica_n_ops : c->plan.ops.size();
         s->algo_bytes_per_witness = c->plan.algo_bytes_per_witness;
+        s->n_sink_ops = c->plan.n_sink_ops;
     }
     s->n_call_groups = c->plan.group_descs.empty() ? p.groups.size() : c->plan.group_descs.size();
     for (const auto& g : p.groups) s->n_group_calls += g.n_calls;
@@ -1207,6 +1212,29 @@ extern "C" int zkb_get_const(zkb_ctx* c, uint64_t idx, uint8_t* out, size_t cap,
 extern "C" int zkb_assert_value(zkb_ctx* c, uint64_t seq, zkb_wire* value) {
     if (seq >= c->prog.asserts.size()) return c->fail(ZKB_E_ARG, "assert index out of range");
     *value = c->prog.asserts[seq].value;
+    return ZKB_OK;
+}
+
+extern "C" int zkb_debug_plan_ops(zkb_ctx* c, uint64_t first, uint64_t n, uint32_t* ops4, uint32_t* values) {
+    if (!c->finalized) return c->fail(ZKB_E_ARG, "zkb_finalize must be called first");
+    if (c->is_replica) return c->fail(ZKB_E_ARG, "replica context: the host copy of the plan lives on the root rank");
+    const Plan& pl = c->plan;
+    if (first > pl.ops.size() || n > pl.ops.size() - first) return c->fail(ZKB_E_ARG, "op range out of bounds");
+    if (values && pl.n_reused_slots != 0) return c->fail(ZKB_E_ARG, "op values need a plan without slot re-use");
+    std::vector<uint32_t> value_of_slot;
+    if (values) {
+        value_of_slot.assign(pl.n_slots, kNoSlot);
+        for (uint32_t v = 0; v < (uint32_t)pl.slot_of_value.size(); v++)
+            if (pl.slot_of_value[v] != kNoSlot) value_of_slot[pl.slot_of_value[v]] = v;
+    }
+    for (uint64_t i = 0; i < n; i++) {
+        const GateOp& g = pl.ops[first + i];
+        ops4[4 * i] = g.a;
+        ops4[4 * i + 1] = g.b;
+        ops4[4 * i + 2] = g.out;
+        ops4[4 * i + 3] = g.meta;
+        if (values) values[i] = g.out < pl.n_slots ? value_of_slot[g.out] : kNoSlot;
+    }
     return ZKB_OK;
 }
 

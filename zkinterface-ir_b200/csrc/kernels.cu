@@ -217,7 +217,7 @@ k_level(const GateOp* __restrict__ ops, const uint32_t* __restrict__ aseq, uint6
             }
             rare_gate<N>(r, a, b, raw, lane, g, rc, fp);
         }
-        if (!(raw.w & F_NOSTORE)) store_elem<N>(store, raw.z, lane, g.log2_wt, r);
+        if (!(raw.w & (F_NOSTORE | g.skip_mask))) store_elem<N>(store, raw.z, lane, g.log2_wt, r);
         if (raw.w & F_ASSERT) {
             bool fail = !fe_is_zero<N>(r) && lane < g.n_valid;
             report_fail(fail, __ldg(aseq + gi), first_fail, g.batch0 + lane, single);
@@ -285,7 +285,7 @@ k_level_pipe(const GateOp* __restrict__ ops, const uint32_t* __restrict__ aseq, 
             if (opc == D_ADD || opc == D_ADDC) fe_add<N>(r + l * N, a0 + l * N, b0 + l * N, fp.p);
             else fe_mont_mul<N>(r + l * N, a0 + l * N, b0 + l * N, fp.p, fp.n0inv);
         }
-        if (!(d0.w & F_NOSTORE)) store_elem<PN>(store, d0.z, plane, log2_pwt, r);
+        if (!(d0.w & (F_NOSTORE | g.skip_mask))) store_elem<PN>(store, d0.z, plane, log2_pwt, r);
         if (d0.w & F_ASSERT) {
             const uint32_t seq = __ldg(aseq + (t0 >> log2_pwt));
 #pragma unroll
@@ -440,7 +440,7 @@ k_level_tma(const GateOp* __restrict__ ops, const uint32_t* __restrict__ aseq, u
         }
         if (opc == D_ADD || opc == D_ADDC) fe_add<N>(r, a, b, fp.p);
         else fe_mont_mul<N>(r, a, b, fp.p, fp.n0inv);
-        if (!(d0.w & F_NOSTORE)) store_elem<N>(store, d0.z, lane, g.log2_wt, r);
+        if (!(d0.w & (F_NOSTORE | g.skip_mask))) store_elem<N>(store, d0.z, lane, g.log2_wt, r);
         if (d0.w & F_ASSERT) {
             const uint32_t seq = __ldg(aseq + (gi >> log2_q));
             bool fail = !fe_is_zero<N>(r) && lane < g.n_valid;

@@ -17,7 +17,8 @@ struct TileGeom {
     uint32_t log2_wt;   // witnesses per tile (power of two)
     uint32_t n_valid;   // lanes of this tile that hold real witnesses
     uint32_t batch0;    // global index of lane 0
-    uint32_t pad;
+    uint32_t skip_mask; // op flags whose results the level kernels do not store (besides F_NOSTORE): F_SINK on a tile that
+                        // the next one overwrites before anything reads it back, else 0
 };
 
 struct InputDesc {

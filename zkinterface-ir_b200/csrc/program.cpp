@@ -420,12 +420,105 @@ void Plan::build(const Program& prog, bool keep_all, const std::vector<uint32_t>
         });
     }
     lap("placement");
+    // Inside each opcode group of a wavefront's hot range, gates that read the same wire run back to back: ordered by a key
+    // operand (the one more gates of the wavefront read; a on a tie; a for AddConstant / MulConstant), then by value.  Today's
+    // value order puts the readers of a wire hundreds of thousands of gates apart, by when its row has left L2; side by side,
+    // the repeat reads hit L2 (DESIGN.md section 4).  Slots are still handed out in position order, so every level keeps
+    // one ascending slot range.  ZKB_OPERAND_ORDER=0: value order.
+    const char* eo = getenv("ZKB_OPERAND_ORDER");
+    if ((!eo || atoi(eo) != 0) && n_levels + 1 < (1u << 24)) {
+        // readers of a wire in the current wavefront: (wavefront + 1) << 8 | count (saturating at 255) in the no longer needed
+        // level array, so no pass resets it between wavefronts
+        uint32_t* rd = level.data();
+        parallel_chunks(T, n, [&](unsigned, uint64_t b, uint64_t e) { memset(rd + b, 0, (e - b) * 4); });
+        std::vector<uint32_t> key_at(n_ops);
+        struct Group {
+            uint64_t lo, hi;
+        };
+        std::vector<Group> groups;
+        for (uint32_t l = 0; l < n_levels; l++) {
+            const uint64_t lo = level_off[l], hi = level_rare[l];
+            if (hi - lo < 2) continue;
+            for (uint32_t op = D_ADD; op <= D_MULC; op++) {
+                const uint64_t gl = cnt[(size_t)l * D_OPS + op], gh = cnt[(size_t)l * D_OPS + op + 1];
+                if (gh - gl >= 2) groups.push_back(Group{gl, gh});
+            }
+            const uint32_t st = (l + 1) << 8;
+            const unsigned Tl = (T > 1 && hi - lo >= (1u << 16)) ? T : 1;
+            auto two_input = [&](uint32_t v) { return kind[v] == V_ADD || kind[v] == V_MUL; };
+            parallel_chunks(Tl, hi - lo, [&](unsigned, uint64_t b, uint64_t e) {
+                auto bump = [&](uint32_t u) {
+                    if (is_callout(u)) return;
+                    uint32_t cur = __atomic_load_n(&rd[u], __ATOMIC_RELAXED);
+                    for (;;) {
+                        const uint32_t next = cur < st ? st + 1 : (cur & 255) == 255 ? cur : cur + 1;
+                        if (next == cur || __atomic_compare_exchange_n(&rd[u], &cur, next, true, __ATOMIC_RELAXED, __ATOMIC_RELAXED))
+                            break;
+                    }
+                };
+                for (uint64_t i = lo + b; i < lo + e; i++) {
+                    if (i + kAhead < lo + e) {
+                        const uint32_t w = value_at[i + kAhead];
+                        if (!is_callout(opa[w])) __builtin_prefetch(&rd[opa[w]], 1);
+                        if (two_input(w) && !is_callout(opb[w])) __builtin_prefetch(&rd[opb[w]], 1);
+                    }
+                    const uint32_t v = value_at[i];
+                    bump(opa[v]);
+                    if (two_input(v)) bump(opb[v]);
+                }
+            });
+            parallel_chunks(Tl, hi - lo, [&](unsigned, uint64_t b, uint64_t e) {
+                auto readers = [&](uint32_t u) { return is_callout(u) ? 0u : rd[u] & 255; };
+                for (uint64_t i = lo + b; i < lo + e; i++) {
+                    const uint32_t v = value_at[i];
+                    key_at[i] = two_input(v) && readers(opb[v]) > readers(opa[v]) ? opb[v] : opa[v];
+                }
+            });
+        }
+        // stable sort by key (value order inside a group is ascending already): LSD radix, 11-bit digits, largest group first
+        std::sort(groups.begin(), groups.end(), [](const Group& x, const Group& y) {
+            return x.hi - x.lo != y.hi - y.lo ? x.hi - x.lo > y.hi - y.lo : x.lo < y.lo;
+        });
+        std::atomic<size_t> next_group{0};
+        const unsigned Tg = (unsigned)std::min<size_t>(T, groups.size());
+        parallel_chunks(Tg, Tg, [&](unsigned, uint64_t, uint64_t) {  // one chunk per thread, groups from a shared queue
+            std::vector<uint32_t> tk, tv;
+            for (size_t gi; (gi = next_group.fetch_add(1, std::memory_order_relaxed)) < groups.size();) {
+                const uint64_t m = groups[gi].hi - groups[gi].lo;
+                uint32_t* key = key_at.data() + groups[gi].lo;
+                uint32_t* val = value_at.data() + groups[gi].lo;
+                uint32_t kmin = 0xFFFFFFFFu, kmax = 0;
+                for (uint64_t i = 0; i < m; i++) {
+                    kmin = std::min(kmin, key[i]);
+                    kmax = std::max(kmax, key[i]);
+                }
+                tk.resize(m);
+                tv.resize(m);
+                uint32_t *sk = key, *sv = val, *dk = tk.data(), *dv = tv.data();
+                for (uint32_t shift = 0; shift < 32 && ((kmax - kmin) >> shift) != 0; shift += 11) {
+                    uint64_t c[2049] = {0};
+                    for (uint64_t i = 0; i < m; i++) c[(((sk[i] - kmin) >> shift) & 2047) + 1]++;
+                    for (int d = 0; d < 2048; d++) c[d + 1] += c[d];
+                    for (uint64_t i = 0; i < m; i++) {
+                        const uint64_t j = c[((sk[i] - kmin) >> shift) & 2047]++;
+                        dk[j] = sk[i];
+                        dv[j] = sv[i];
+                    }
+                    std::swap(sk, dk);
+                    std::swap(sv, dv);
+                }
+                if (sv != val) memcpy(val, sv, m * 4);
+            }
+        });
+        lap("operand order");
+    }
     ops.assign(n_ops, GateOp{0, 0, 0, 0});
     op_assert_seq.assign(n_ops, kNoSeq);
     for (int i = 0; i < D_OPS; i++) n_dev_ops[i] = 0;
     std::vector<uint32_t> meta_of(n_ops, 0);
     n_reused_slots = 0;
     n_raw_ops = 0;
+    n_sink_ops = 0;
     double t_free = 0, t_dist = 0;
     for (uint32_t l = 0; l < n_levels; l++) {
         auto tf0 = std::chrono::steady_clock::now();
@@ -451,10 +544,10 @@ void Plan::build(const Program& prog, bool keep_all, const std::vector<uint32_t>
         // from a prefix sum over chunks of the wavefront, so the chunks can be processed by different threads.
         const uint64_t lo = level_off[l], hi = level_off[l + 1];
         const unsigned Tl = (T > 1 && hi - lo >= (1u << 16)) ? T : 1;
-        std::vector<uint64_t> stored(Tl + 1, 0);
+        std::vector<uint64_t> stored(Tl + 1, 0), sinks(Tl, 0);
         // pass A: the store decision and the flags of every op
         parallel_chunks(Tl, hi - lo, [&](unsigned t, uint64_t b, uint64_t e) {
-            uint64_t cnt_store = 0;
+            uint64_t cnt_store = 0, cnt_sink = 0;
             for (uint64_t i = lo + b; i < lo + e; i++) {
                 if (i + kAhead < lo + e) {  // values arrive in sorted, i.e. random, order: start their loads early
                     uint32_t va = value_at[i + kAhead];
@@ -473,13 +566,24 @@ void Plan::build(const Program& prog, bool keep_all, const std::vector<uint32_t>
                 // stored unless nothing will ever read it: a value only tested by its own fused assertion, or
                 // (with slot re-use on) a dead value — it is still computed
                 bool store = keep_all || used[v] || observable[v] || (!has_assert && !reuse);
-                if (!store) meta |= F_NOSTORE;
-                else cnt_store++;
+                if (!store) {
+                    meta |= F_NOSTORE;
+                } else {
+                    cnt_store++;
+                    if (!used[v]) {
+                        meta |= F_SINK;
+                        cnt_sink++;
+                    }
+                }
                 meta_of[i] = meta;
             }
             stored[t + 1] = cnt_store;
+            sinks[t] = cnt_sink;
         });
-        for (unsigned t = 0; t < Tl; t++) stored[t + 1] += stored[t];
+        for (unsigned t = 0; t < Tl; t++) {
+            stored[t + 1] += stored[t];
+            n_sink_ops += sinks[t];
+        }
         const uint64_t n_free = free_slots.size() - free_head, n_store = stored[Tl];
         // pass B: hand out the slots, collect what each stored value releases later
         std::vector<std::vector<std::pair<uint32_t, uint32_t>>> released(Tl);  // (wavefront after which it is free, slot)

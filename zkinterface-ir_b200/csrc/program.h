@@ -87,6 +87,9 @@ constexpr uint32_t F_ASSERT = 1u << 8;    // result must be zero; assert seq in 
 constexpr uint32_t F_NOSTORE = 1u << 9;   // value is consumed by nothing but the fused assert
 constexpr uint32_t F_RAW = 1u << 10;      // operand a is an input value: consult its "raw value >= p" flag (trap 1)
 constexpr uint32_t F_RAWB = 1u << 11;     // operand b (of And / Xor) is an input value: likewise
+// stored, but no gate reads it (a live wire nothing consumes, an observable assertion sum): only a read-back needs the
+// store, so a tile that is overwritten by the next one may skip it (TileGeom::skip_mask)
+constexpr uint32_t F_SINK = 1u << 12;
 constexpr uint32_t kNoSeq = 0xFFFFFFFFu;
 constexpr uint32_t kNoSlot = 0xFFFFFFFFu;
 
@@ -284,7 +287,10 @@ struct Plan {
     bool slot_reuse = true;               // liveness-based slot re-use (off: one slot per stored value)
     uint64_t n_reused_slots = 0;
     uint64_t n_raw_ops = 0;               // ops that need the raw-input flags (assert / not directly on an input)
-    std::vector<GateOp> ops;              // level-major, opcode-sorted inside a level
+    uint64_t n_sink_ops = 0;              // ops flagged F_SINK
+    // level-major, opcode-sorted inside a level; inside an opcode group of the hot range (Add, Mul, AddC, MulC) the gates
+    // are ordered by their shared operand (Plan::build), so the readers of one wire run back to back
+    std::vector<GateOp> ops;
     std::vector<uint32_t> op_assert_seq;  // parallel to ops
     std::vector<uint64_t> level_off;      // n_levels + 1 offsets into ops
     std::vector<uint64_t> level_rare;     // per level: where the rare opcodes (>= D_AND) start

@@ -642,7 +642,7 @@ extern "C" int zkb_r1cs_run(zkb_ctx* c, zkb_verdict* out) {
         g.log2_wt = r->log2_wt;
         g.batch0 = t << r->log2_wt;
         g.n_valid = std::min<uint32_t>(wt, r->n_batch - g.batch0);
-        g.pad = 0;
+        g.skip_mask = 0;
         unsigned grid = grid_for(r->n_vars << r->log2_wt, c->sm_count, 256);
         DISPATCH_N(N, (k_r1cs_load_z<N><<<grid, 256, 0, c->stream>>>(r->d_zraw, r->z_set_stride, r->stride, r->n_vars, r->d_z, g,
                                                                      c->d_unreduced, fp)));
