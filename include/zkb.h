@@ -186,15 +186,17 @@ typedef struct {
     uint32_t binary;        /* p == 2 */
     uint32_t tile_witnesses;/* witnesses resident per pass (after upload) */
     uint32_t n_tiles;
-    uint64_t n_call_groups; /* For loops over a plain function kept as ONE loop-structured descriptor each (Boolean
-                             * profile; evaluator.rs:495-559 + :441-471): the device expands them, only the calls'
-                             * outputs are SSA values (kind 11 in zkb_get_program) */
+    uint64_t n_call_groups; /* For loops over a plain function kept as ONE loop-structured descriptor each
+                             * (evaluator.rs:495-559 + :441-471; over a prime field: loops of >= 1024 calls whose body
+                             * holds Constant / Add / Mul / AddConstant / MulConstant and AssertZero on computed wires):
+                             * the device expands them, only the calls' outputs are SSA values (kind 11 in zkb_get_program) */
     uint64_t n_group_calls; /* function calls those groups stand for */
     uint64_t n_group_launches;     /* after finalize: kernel launches that expand them (one per dependency depth) */
     uint64_t n_group_table_slots;  /* after finalize: operand slots listed explicitly (inputs whose slots are not an
                                     * arithmetic progression over the calls) */
     int64_t group_jit_state;       /* the groups' run-time specialised kernel: -2 none, -1 unavailable (the interpreter kernel
-                                    * runs), 0 compiling in the background, 2 compiled, 3 loaded and in use */
+                                    * runs; always so over a prime field), 0 compiling in the background, 2 compiled, 3 loaded
+                                    * and in use */
     uint64_t n_sink_ops;           /* after finalize: stored results that no gate reads (only a read-back needs them; tiles
                                     * other than the last one run skip their stores) */
 } zkb_stats;
@@ -211,7 +213,8 @@ int zkb_get_const(zkb_ctx* ctx, uint64_t idx, uint8_t* out_le, size_t cap, size_
  * assertion, out[3] not stored, out[4] algorithmic bytes per witness (3E per two-operand gate, 2E per
  * one-operand gate, E per assertion; SURVEY.md section 8d) */
 int zkb_level_info(zkb_ctx* ctx, uint64_t level, uint64_t out[5]);
-/* asserted value handle of assertion seq */
+/* asserted value handle of assertion seq; ZKB_E_ARG for an assertion inside a call group (its value is a call-local wire
+ * without a handle; zkb_assert_info still gives its local wire id) */
 int zkb_assert_value(zkb_ctx* ctx, uint64_t seq, zkb_wire* value);
 
 typedef struct {

@@ -741,7 +741,10 @@ static void run_tile(zkb_ctx* c, uint32_t tile, bool full, uint32_t* d_fail, uin
         const uint32_t lo = pl.depth_off[d], hi = pl.depth_off[d + 1];
         if (hi == lo) continue;
         const uint64_t calls = (uint64_t)pl.group_descs[hi - 1].first_call + pl.group_descs[hi - 1].n_calls;
-        if (!group_jit_launch(c, c->d_group_descs + lo, hi - lo, calls, c->d_group_hints + pl.hint_off[d], g.log2_wt - 5, (void*)c->stream))
+        if (!p.binary)
+            launch_arith_groups(p.nlimb, c->d_group_descs + lo, hi - lo, calls, c->d_group_ops, c->d_group_tables, c->d_group_hints + pl.hint_off[d],
+                                c->d_store, c->d_consts, d_fail, g, p.fp, pl.group_regs, c->sm_count, c->stream);
+        else if (!group_jit_launch(c, c->d_group_descs + lo, hi - lo, calls, c->d_group_hints + pl.hint_off[d], g.log2_wt - 5, (void*)c->stream))
             launch_bool_groups(c->d_group_descs + lo, hi - lo, calls, c->d_group_ops, c->d_group_tables, c->d_group_hints + pl.hint_off[d],
                                c->d_store, g, pl.group_regs, c->sm_count, c->stream, pl.group_ops.data(), (uint32_t)pl.group_ops.size());
         (*launches)++;
@@ -1211,6 +1214,7 @@ extern "C" int zkb_get_const(zkb_ctx* c, uint64_t idx, uint8_t* out, size_t cap,
 
 extern "C" int zkb_assert_value(zkb_ctx* c, uint64_t seq, zkb_wire* value) {
     if (seq >= c->prog.asserts.size()) return c->fail(ZKB_E_ARG, "assert index out of range");
+    if (c->prog.asserts[seq].value == kGroupAssertValue) return c->fail(ZKB_E_ARG, "assertion inside a call group: its value is a call-local wire");
     *value = c->prog.asserts[seq].value;
     return ZKB_OK;
 }

@@ -358,14 +358,15 @@ struct zkb_evaluator {
         for (size_t idx = 0; idx < n_out; idx++) set(scope, outs[idx], p.copy(L[idx]));
     }
     // ---- loop-structured recording: a For loop over a plain function becomes ONE call group (program.h) -----------------
-    // The body qualifies when every gate is a value-defining simple gate the device interpreter runs on reduced values:
-    // no AssertZero (an assertion inside a call needs a sequence number per call), no Copy (an output that aliases a raw
+    // Over p = 2 the body qualifies when every gate is a value-defining simple gate the device interpreter runs on reduced values:
+    // no AssertZero, no Copy (an output that aliases a raw
     // input would carry its unreduced integer on), and no Not directly on a call input (Not tests the RAW integer of an
-    // input value, evaluator.rs:932-938; And / Xor / Add / Mul only see the low bit mod 2).  Boolean profile only.
+    // input value, evaluator.rs:932-938; And / Xor / Add / Mul only see the low bit mod 2).  Prime fields: arith_template_of.
     int template_of(const FunctionDecl& f) {
         if (f.tmpl != -1) return f.tmpl;
         f.tmpl = -2;
         Program& p = prog();
+        if (!p.binary) return f.tmpl = arith_template_of(f);
         if (!f.n_local || f.n_local > kMaxTemplateRegs || f.body->size() > kMaxTemplateOps || f.input_count > kMaxGroupInputs ||
             f.output_count == 0)
             return f.tmpl;
@@ -415,6 +416,108 @@ struct zkb_evaluator {
         p.templates.push_back(std::move(t));
         f.tmpl = (int)p.templates.size() - 1;
         return f.tmpl;
+    }
+
+    // Prime fields: Constant (< p), Add, Mul, AddConstant, MulConstant, and AssertZero on a register the body computed.  And /
+    // Xor / Not / Copy act on raw integers (evaluator.rs:924-938; a copy of an input would carry its unreduced integer on) and
+    // an AssertZero on an input tests the raw integer (trap 1): such bodies run gate by gate.  Registers are renamed by
+    // liveness in one linear scan (outputs pinned to 0 .. n_out-1, inputs start at n_out), so the device register file holds
+    // the values live at once rather than every wire of the body.
+    int arith_template_of(const FunctionDecl& f) {
+        Program& p = prog();
+        const uint64_t n_out = f.output_count, n_in = f.input_count;
+        if (!f.n_local || f.body->size() > kMaxTemplateOps || n_in > kMaxGroupInputs || n_out == 0 || n_out + n_in > kMaxTemplateRegs)
+            return -2;
+        auto is_input = [&](uint64_t w) { return w >= n_out && w < n_out + n_in; };
+        std::vector<int32_t> last(f.n_local, -1);  // index of the last gate reading each wire
+        for (size_t i = 0; i < f.body->size(); i++) {
+            const ir::Gate& g = (*f.body)[i];
+            switch (g.type) {
+                case ir::G_CONSTANT: break;
+                case ir::G_ASSERT_ZERO:
+                    if (is_input(g.w0)) return -2;
+                    last[g.w0] = (int32_t)i;
+                    break;
+                case ir::G_ADD: case ir::G_MUL: last[g.w1] = last[g.w2] = (int32_t)i; break;
+                case ir::G_ADD_CONSTANT: case ir::G_MUL_CONSTANT: last[g.w1] = (int32_t)i; break;
+                default: return -2;  // And, Xor, Not, Copy
+            }
+        }
+        Template t;
+        t.n_out = (uint32_t)n_out;
+        t.n_in = (uint32_t)n_in;
+        std::vector<int32_t> reg(f.n_local, -1);
+        for (uint64_t w = n_out; w < n_out + n_in; w++) reg[w] = (int32_t)w;
+        std::vector<uint32_t> free_regs;  // kept in descending order: back() is the lowest free register
+        uint32_t n_regs = (uint32_t)(n_out + n_in);
+        auto release = [&](uint64_t w, size_t i) {
+            if (w >= n_out && last[w] <= (int32_t)i && reg[w] >= 0) {
+                free_regs.insert(std::upper_bound(free_regs.begin(), free_regs.end(), (uint32_t)reg[w], std::greater<uint32_t>()),
+                                 (uint32_t)reg[w]);
+                reg[w] = -1;
+            }
+        };
+        for (size_t i = 0; i < f.body->size(); i++) {
+            const ir::Gate& g = (*f.body)[i];
+            TmplOp o{};
+            switch (g.type) {
+                case ir::G_CONSTANT: {
+                    const auto& v = (*f.consts)[g.const_idx];
+                    o.kind = V_CONST;
+                    o.b = p.intern_const(v.data(), v.size());
+                    if (p.const_unreduced[o.b]) return -2;  // a constant >= p stays a raw integer (trap 1)
+                    t.cb[CB_CONSTANT]++;
+                } break;
+                case ir::G_ADD: case ir::G_MUL:
+                    o.kind = g.type == ir::G_ADD ? V_ADD : V_MUL;
+                    o.a = (uint8_t)reg[g.w1];
+                    o.b = (uint32_t)reg[g.w2];
+                    t.cb[g.type == ir::G_ADD ? CB_ADD : CB_MUL]++;
+                    t.n_two++;
+                    break;
+                case ir::G_ADD_CONSTANT: case ir::G_MUL_CONSTANT: {  // reduced result: a constant >= p is fine here
+                    const auto& v = (*f.consts)[g.const_idx];
+                    o.kind = g.type == ir::G_ADD_CONSTANT ? V_ADDC : V_MULC;
+                    o.a = (uint8_t)reg[g.w1];
+                    o.b = p.intern_const(v.data(), v.size());
+                    t.cb[g.type == ir::G_ADD_CONSTANT ? CB_ADDC : CB_MULC]++;
+                    t.n_one++;
+                } break;
+                default:  // G_ASSERT_ZERO (the unrolled loop asserts a copy of the wire: one Copy callback each)
+                    o.kind = T_ASSERT;
+                    o.a = (uint8_t)reg[g.w0];
+                    o.b = (uint32_t)t.assert_wire.size();
+                    t.assert_wire.push_back(g.w0);
+                    t.cb[CB_ASSERT_ZERO]++;
+                    t.cb[CB_COPY]++;
+                    break;
+            }
+            if (g.type != ir::G_CONSTANT) t.ir_gates++;
+            if (g.type == ir::G_ASSERT_ZERO) {
+                release(g.w0, i);
+            } else {
+                if (g.type != ir::G_CONSTANT) release(g.w1, i);
+                if (g.type == ir::G_ADD || g.type == ir::G_MUL) release(g.w2, i);
+                uint32_t r;
+                if (g.w0 < n_out) {
+                    r = (uint32_t)g.w0;
+                } else if (!free_regs.empty()) {
+                    r = free_regs.back();
+                    free_regs.pop_back();
+                } else {
+                    r = n_regs++;
+                }
+                if (n_regs > kMaxTemplateRegs) return -2;
+                reg[g.w0] = (int32_t)r;
+                o.dst = (uint8_t)r;
+                release(g.w0, i);  // a value nothing reads: its register is free again at once
+            }
+            t.ops.push_back(o);
+        }
+        t.n_regs = n_regs;
+        t.cb[CB_COPY] += n_in + n_out;
+        p.templates.push_back(std::move(t));
+        return (int)p.templates.size() - 1;
     }
 
     struct AffineWire {
@@ -476,8 +579,9 @@ struct zkb_evaluator {
     // reports every error where the reference does.
     bool try_call_group(const ir::Complex& cx, const FunctionDecl& f, Scope& scope, Iters& iters, const uint32_t* weight) {
         Program& p = prog();
-        if (getenv("ZKB_NO_CALL_GROUPS") != nullptr || weight || p.keep_copies || p.expand_on || !p.field_set || !p.binary) return false;
+        if (getenv("ZKB_NO_CALL_GROUPS") != nullptr || weight || p.keep_copies || p.expand_on || !p.field_set) return false;
         if (cx.last < cx.first || cx.last - cx.first < 3 || cx.last - cx.first >= (1ull << 28)) return false;
+        if (!p.binary && cx.last - cx.first + 1 < kArithGroupMinCalls) return false;
         const int ti = template_of(f);
         if (ti < 0) return false;
         const uint64_t n = cx.last - cx.first + 1;
@@ -568,6 +672,8 @@ struct zkb_evaluator {
             cg.in_stride.push_back(st);
         }
         if (p.n_total_values() + n_new >= c->max_values || (uint64_t)p.n_callouts + n_new >= kMaxCallouts) return false;  // the gate-by-gate loop reports the limit
+        const uint64_t n_group_asserts = n * t.assert_wire.size();
+        if ((uint64_t)p.asserts.size() + n_group_asserts >= kNoSeq) return false;
         step(n * (1 + f.body->size()));
         // ---- commit: the outputs are implicit values (program.h), only the scope learns about them
         c->max_values = std::min<uint64_t>(c->max_values, kCalloutBit - 256);  // explicit handles stay below the callout space
@@ -585,6 +691,14 @@ struct zkb_evaluator {
                 for (uint32_t k = 0; k < t.n_out; k++) set(scope, wo[k].w0 + S * c, h_first + (uint32_t)(c * t.n_out + k));
         }
         p.n_callouts += (uint32_t)n_new;
+        // the calls' assertions, in the unrolled loop's order: call c's k-th is seq0 + c * A + k
+        cg.seq0 = (uint32_t)p.asserts.size();
+        if (n_group_asserts) {
+            std::vector<AssertRec> call(t.assert_wire.size());
+            for (size_t k = 0; k < call.size(); k++) call[k] = AssertRec{kGroupAssertValue, p.n_values(), t.assert_wire[k]};
+            p.asserts.reserve(p.asserts.size() + n_group_asserts);
+            for (uint64_t c = 0; c < n; c++) p.asserts.insert(p.asserts.end(), call.begin(), call.end());
+        }
         for (int k = 0; k < CB_KINDS; k++) p.cb_count[k] += n * t.cb[k];
         p.ir_gates += n * t.ir_gates;
         p.groups.push_back(std::move(cg));

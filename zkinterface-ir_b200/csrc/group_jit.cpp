@@ -231,7 +231,14 @@ void group_jit_start(zkb_ctx* c) {
     group_jit_free(c);
     const char* e = getenv("ZKB_GROUP_JIT");
     const bool sync = e && atoi(e) == 2;  // compile in the calling thread (tests; also without a device: NVRTC needs none)
-    if ((e && atoi(e) == 0) || c->plan.group_descs.empty() || (!c->has_gpu && !sync)) return;
+    if (c->plan.group_descs.empty()) return;
+    if (!c->prog.binary) {  // prime-field templates are left to the interpreter kernel (k_arith_groups): state -1
+        c->gjit = new GroupJit();
+        c->gjit->state = -1;
+        c->gjit->log = "call groups over a prime field run in the interpreter kernel";
+        return;
+    }
+    if ((e && atoi(e) == 0) || (!c->has_gpu && !sync)) return;
     GroupJit* j = new GroupJit();
     c->gjit = j;
     j->source = generate(c->plan);

@@ -992,6 +992,98 @@ k_bool_groups(const GroupDesc* __restrict__ descs, uint32_t n_groups, uint64_t t
     }
 }
 
+// Call groups over a prime field: thread <-> (call, witness lane), lane fastest, so for tiles of >= 32 lanes a warp loads
+// and stores one coalesced row per 16-byte chunk of the wire store, and for narrower tiles a warp spans calls.  A call's
+// inputs are read into a register file in dynamic shared memory, laid out like the wire store with the CTA's threads as
+// lanes (chunk c of register r of thread t at ((r * NC + c) * T + t) * CW limbs: a thread's 16-byte chunks are
+// conflict-free), the body runs over it op by op (Montgomery arithmetic of field_ptx.cuh, constants from the Montgomery
+// const table), the previous op's result stays in registers (GroupOp::fwd), an AssertZero tests its register in place and
+// reports seq0 + call * A + k, and only the outputs go back to the wire store (always stored: a group output is a level-0
+// value).  thread -> group as in k_bool_groups.
+template <int N>
+__global__ void __launch_bounds__(kGroupThreads)
+k_arith_groups(const GroupDesc* __restrict__ descs, uint32_t n_groups, uint64_t total_calls, const GroupOp* __restrict__ gops,
+               const uint32_t* __restrict__ tables, const uint32_t* __restrict__ hints, uint32_t* __restrict__ store,
+               const uint32_t* __restrict__ consts_mont, uint32_t* __restrict__ first_fail, TileGeom g, FieldParams fp) {
+    constexpr int CW = Elem<N>::CW, NC = Elem<N>::NC;
+    using V = typename Vec<CW>::T;
+    extern __shared__ __align__(16) uint8_t s_regs[];
+    const uint32_t T = blockDim.x;
+    V* R = reinterpret_cast<V*>(s_regs) + threadIdx.x;  // register r, chunk c: R[(r * NC + c) * T]
+    auto ld_reg = [&](uint32_t* x, uint32_t r) {
+#pragma unroll
+        for (int c = 0; c < NC; c++) unpack(R[(r * NC + c) * T], x + c * CW);
+    };
+    auto st_reg = [&](uint32_t r, const uint32_t* x) {
+#pragma unroll
+        for (int c = 0; c < NC; c++) {
+            V v;
+            pack(v, x + c * CW);
+            R[(r * NC + c) * T] = v;
+        }
+    };
+    const uint64_t total = total_calls << g.log2_wt;
+    const uint32_t wt_mask = (1u << g.log2_wt) - 1;
+    for (uint64_t tid = blockIdx.x * (uint64_t)T + threadIdx.x; tid < total; tid += (uint64_t)gridDim.x * T) {
+        const uint32_t lane = (uint32_t)tid & wt_mask;
+        const uint32_t call_g = (uint32_t)(tid >> g.log2_wt);
+        uint32_t gi = __ldg(hints + (call_g >> kGroupHintShift));
+        while (gi + 1 < n_groups && call_g >= __ldg(&descs[gi + 1].first_call)) gi++;
+        const GroupDesc* d = descs + gi;
+        const uint4 h0 = __ldg(reinterpret_cast<const uint4*>(d));      // tmpl_off, n_ops, n_out, n_in
+        const uint4 h1 = __ldg(reinterpret_cast<const uint4*>(d) + 1);  // n_calls, out_slot, first_call, seq0
+        const uint32_t call = call_g - h1.z;
+        uint32_t x[N], y[N], r[N];
+        for (uint32_t k = 0; k < h0.w; k++) {
+            const uint32_t base = __ldg(d->in_base + k), st = __ldg(d->in_stride + k);
+            const uint32_t slot = st == kTableStride ? __ldg(tables + base + call) : base + st * call;
+            load_elem<N>(x, store, slot, lane, g.log2_wt);
+            st_reg(h0.z + k, x);
+        }
+        const uint4* op = reinterpret_cast<const uint4*>(gops + h0.x);
+#pragma unroll
+        for (int k = 0; k < N; k++) r[k] = 0;
+        for (uint32_t i = 0; i < h0.y; i++) {
+            const uint4 o = __ldg(op + 2 * i);      // dst, a, b registers, fwd
+            const uint4 m = __ldg(op + 2 * i + 1);  // kind, const index, assertion ordinal, assertions per call
+            if (m.x == AG_CONST) {
+#pragma unroll
+                for (int k = 0; k < N; k++) r[k] = __ldg(consts_mont + (size_t)m.y * N + k);
+                st_reg(o.x, r);
+                continue;
+            }
+            if (o.w & 1) {
+#pragma unroll
+                for (int k = 0; k < N; k++) x[k] = r[k];
+            } else {
+                ld_reg(x, o.y);
+            }
+            if (m.x == AG_ASSERT) {
+                const bool fail = !fe_is_zero<N>(x) && lane < g.n_valid;
+                report_fail(fail, h1.w + call * m.w + m.z, first_fail, g.batch0 + lane, false);
+                continue;
+            }
+            if (m.x == AG_ADDC || m.x == AG_MULC) {
+#pragma unroll
+                for (int k = 0; k < N; k++) y[k] = __ldg(consts_mont + (size_t)m.y * N + k);
+            } else if (o.w & 2) {
+#pragma unroll
+                for (int k = 0; k < N; k++) y[k] = r[k];
+            } else {
+                ld_reg(y, o.z);
+            }
+            if (m.x == AG_ADD || m.x == AG_ADDC) fe_add<N>(r, x, y, fp.p);
+            else fe_mont_mul<N>(r, x, y, fp.p, fp.n0inv);
+            st_reg(o.x, r);
+        }
+        const uint32_t out0 = h1.y + call * h0.z;
+        for (uint32_t k = 0; k < h0.z; k++) {
+            ld_reg(x, k);
+            store_elem<N>(store, out0 + k, lane, g.log2_wt, x);
+        }
+    }
+}
+
 __global__ void k_bool_read_values(const uint32_t* __restrict__ slots, uint32_t n, const uint32_t* __restrict__ store, uint32_t lane,
                                    uint32_t log2_wt, uint32_t* __restrict__ out) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1343,6 +1435,34 @@ void launch_bool_groups(const GroupDesc* descs, uint32_t n_groups, uint64_t tota
         if (wide) k_bool_groups<4, false><<<grid, kGroupThreads, smem, s>>>(descs, n_groups, total_calls, gops, tables, hints, store, log2_words, none);
         else k_bool_groups<1, false><<<grid, kGroupThreads, smem, s>>>(descs, n_groups, total_calls, gops, tables, hints, store, log2_words, none);
     }
+}
+
+// CTA size: the largest power of two <= 256 threads whose register file (n_regs x 4N bytes a thread) leaves room for two
+// CTAs per SM
+static constexpr size_t kArithGroupSmemPerCta = 112 * 1024;
+uint32_t arith_group_threads(int nlimb, uint32_t n_regs) {
+    uint32_t t = kGroupThreads;
+    while (t > 32 && (size_t)n_regs * nlimb * 4 * t > kArithGroupSmemPerCta) t >>= 1;
+    return t;
+}
+template <int N>
+static void launch_arith_groups_n(const GroupDesc* descs, uint32_t n_groups, uint64_t total_calls, const GroupOp* gops, const uint32_t* tables,
+                                  const uint32_t* hints, uint32_t* store, const uint32_t* consts_mont, uint32_t* first_fail, TileGeom g,
+                                  const FieldParams& fp, uint32_t n_regs, int sm_count, cudaStream_t s) {
+    static std::atomic<uint64_t> attr_seen{0};
+    if (first_on_device(attr_seen)) cudaFuncSetAttribute(k_arith_groups<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kArithGroupSmemPerCta);
+    const uint32_t T = arith_group_threads(N, n_regs);
+    const size_t smem = (size_t)std::max<uint32_t>(n_regs, 1) * N * 4 * T;
+    const uint64_t blocks = ((total_calls << g.log2_wt) + T - 1) / T;
+    const unsigned grid = (unsigned)std::min<uint64_t>(blocks, (uint64_t)sm_count * (2048 / T));
+    k_arith_groups<N><<<grid, T, smem, s>>>(descs, n_groups, total_calls, gops, tables, hints, store, consts_mont, first_fail, g, fp);
+}
+void launch_arith_groups(int nlimb, const GroupDesc* descs, uint32_t n_groups, uint64_t total_calls, const GroupOp* gops, const uint32_t* tables,
+                         const uint32_t* hints, uint32_t* store, const uint32_t* consts_mont, uint32_t* first_fail, TileGeom g,
+                         const FieldParams& fp, uint32_t n_regs, int sm_count, cudaStream_t s) {
+    if (n_groups == 0 || total_calls == 0) return;
+    ZKB_DISPATCH_N(nlimb, (launch_arith_groups_n<N>(descs, n_groups, total_calls, gops, tables, hints, store, consts_mont, first_fail, g, fp,
+                                                    n_regs, sm_count, s)));
 }
 
 void launch_bool_read_values(const uint32_t* slots, uint32_t n, const uint32_t* store, uint32_t lane, uint32_t log2_wt,

@@ -69,6 +69,12 @@ cudaError_t launch_levels_flow_wide(int nlimb, const GateOp* ops, const uint32_t
 // k_levels_coop, 2: the hardware barrier of one 8-CTA cluster)
 cudaError_t measure_barrier_cost(int kind, unsigned blocks, unsigned n_barriers, uint32_t* barrier_ctr, uint32_t* barrier_epoch,
                                  cudaStream_t s, cudaEvent_t ev0, cudaEvent_t ev1, float* us_per_barrier);
+// call groups of one depth over a prime field (k_arith_groups): n_regs = the widest template's register count; first_fail gets
+// the calls' failing assertions
+void launch_arith_groups(int nlimb, const GroupDesc* descs, uint32_t n_groups, uint64_t total_calls, const GroupOp* gops, const uint32_t* tables,
+                         const uint32_t* hints, uint32_t* store, const uint32_t* consts_mont, uint32_t* first_fail, TileGeom g,
+                         const FieldParams& fp, uint32_t n_regs, int sm_count, cudaStream_t s);
+uint32_t arith_group_threads(int nlimb, uint32_t n_regs);  // its CTA size
 void launch_read_values(int nlimb, const uint32_t* slots, uint32_t n, const uint32_t* store, uint32_t lane, uint32_t log2_wt,
                         uint32_t* out, const FieldParams& fp, cudaStream_t s);
 

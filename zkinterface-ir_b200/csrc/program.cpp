@@ -289,6 +289,7 @@ void Plan::build(const Program& prog, bool keep_all, const std::vector<uint32_t>
     callout_assert_value.clear();
     for (size_t s = 0; s < prog.asserts.size(); s++) {
         uint32_t v = prog.asserts[s].value;
+        if (v == kGroupAssertValue) continue;  // inside a call group: tested by the group kernel
         if (is_callout(v)) {  // AssertZero directly on a group output: a standalone test in wavefront 1
             callout_assert_seq.push_back((uint32_t)s);
             callout_assert_value.push_back(v);
@@ -713,8 +714,30 @@ void Plan::build(const Program& prog, bool keep_all, const std::vector<uint32_t>
             group_regs = std::max(group_regs, prog.templates[t].n_regs);
             tmpl_off[t] = (uint32_t)group_ops.size();
             uint32_t prev_dst = 0xFFFFFFFFu;
+            const uint32_t n_asserts = (uint32_t)prog.templates[t].assert_wire.size();
             for (const TmplOp& o : prog.templates[t].ops) {
                 GroupOp g{};
+                if (!prog.binary) {  // register numbers and the op (program.h, GroupOp over a prime field)
+                    const bool two = o.kind == V_ADD || o.kind == V_MUL;
+                    switch (o.kind) {
+                        case V_ADD: g.m_and = AG_ADD; break;
+                        case V_MUL: g.m_and = AG_MUL; break;
+                        case V_ADDC: g.m_and = AG_ADDC; g.m_xor = o.b; break;
+                        case V_MULC: g.m_and = AG_MULC; g.m_xor = o.b; break;
+                        case V_CONST: g.m_and = AG_CONST; g.m_xor = o.b; break;
+                        default: g.m_and = AG_ASSERT; g.m_a = o.b; g.m_c = n_asserts; break;  // T_ASSERT
+                    }
+                    g.dst_off = o.kind == T_ASSERT ? 0 : o.dst;
+                    g.a_off = o.kind == V_CONST ? 0 : o.a;
+                    g.b_off = two ? o.b : g.a_off;
+                    if (o.kind != V_CONST && prev_dst != 0xFFFFFFFFu) {
+                        if (o.a == prev_dst) g.fwd |= 1;
+                        if (two && o.b == prev_dst) g.fwd |= 2;
+                    }
+                    if (o.kind != T_ASSERT) prev_dst = o.dst;  // an assertion writes nothing: the held result stays
+                    group_ops.push_back(g);
+                    continue;
+                }
                 const uint32_t all = 0xFFFFFFFFu;
                 const bool two = o.kind == V_ADD || o.kind == V_MUL || o.kind == V_AND || o.kind == V_XOR;
                 const uint32_t cmask = (o.kind == V_CONST || o.kind == V_ADDC || o.kind == V_MULC)
@@ -755,6 +778,7 @@ void Plan::build(const Program& prog, bool keep_all, const std::vector<uint32_t>
             gd.n_calls = cg.n_calls;
             gd.out_slot = callout_slot0 + cg.first_callout;
             gd.first_call = calls_before[cg.depth];
+            gd.pad = prog.binary ? 0 : cg.seq0;
             calls_before[cg.depth] += cg.n_calls;
             for (uint32_t k = 0; k < tp.n_in; k++) {
                 const uint32_t b = cg.in_base[k], st = cg.in_stride[k];

@@ -54,8 +54,16 @@ constexpr uint32_t kCalloutBit = 0x80000000u;
 constexpr uint32_t kMaxCallouts = 0x7FFFFF00u;
 inline bool is_callout(uint32_t h) { return (h & kCalloutBit) != 0; }  // (Scope::kNone has the bit too: test it first)
 inline uint32_t callout_index(uint32_t h) { return h & ~kCalloutBit; }
+// Over a prime field a loop qualifies only with at least kArithGroupMinCalls calls: below that the gate-by-gate recording
+// is small and one launch per depth costs more than it saves.  Its body may hold AssertZero (TmplOp kind T_ASSERT); a call's
+// k-th assertion has the sequence number seq0 + call * n_asserts + k, which is the unrolled loop's program order.
+constexpr uint64_t kArithGroupMinCalls = 1024;
+constexpr uint8_t T_ASSERT = 0xF0;  // template-only op kind: AssertZero on register a, b = its ordinal k inside the body
+// AssertRec::value of an assertion inside a call group: the asserted value is a call-local wire that has no handle
+constexpr uint32_t kGroupAssertValue = 0xFFFFFFFFu;
 struct TmplOp {       // 8 bytes
-    uint8_t kind;     // ValKind: V_CONST (b = const-pool index), V_ADD, V_MUL, V_ADDC / V_MULC (b = const-pool index), V_AND, V_XOR, V_NOT
+    uint8_t kind;     // ValKind: V_CONST (b = const-pool index), V_ADD, V_MUL, V_ADDC / V_MULC (b = const-pool index), V_AND, V_XOR, V_NOT;
+                      // T_ASSERT (prime fields)
     uint8_t dst;      // register written
     uint8_t a;        // register read
     uint8_t pad;
@@ -67,6 +75,7 @@ struct Template {
     uint64_t cb[12] = {0};   // callbacks one call makes, by CbKind (copies of the inputs and outputs included)
     uint64_t ir_gates = 0;
     uint64_t n_two = 0, n_one = 0;  // two-input / one-input value gates (algorithmic bytes, SURVEY.md section 8d)
+    std::vector<uint64_t> assert_wire;  // per AssertZero of the body, in order: its local wire id (what a violation names)
 };
 struct CallGroup {
     uint32_t tmpl = 0;
@@ -75,6 +84,7 @@ struct CallGroup {
     uint32_t depth = 0;        // 0: reads input values only; d: reads outputs of groups of depth < d as well
     std::vector<uint32_t> in_base, in_stride;  // per input position: handle of call c's input = base + stride * c
     uint32_t n_out = 0;
+    uint32_t seq0 = 0;  // assertion sequence number of call 0's first AssertZero (templates with assertions)
 };
 
 // callback counters (one per ZKBackend method that the Evaluator drives)
@@ -119,7 +129,7 @@ struct GroupDesc {  // 16-byte aligned
     uint32_t n_calls;
     uint32_t out_slot;   // slot of output 0 of call 0; outputs are consecutive slots
     uint32_t first_call; // calls of the groups before this one in the same launch (prefix sum: thread -> group search)
-    uint32_t pad;
+    uint32_t pad;        // prime fields: CallGroup::seq0 (0 for p = 2)
     uint32_t in_base[kMaxGroupInputs];
     uint32_t in_stride[kMaxGroupInputs];
 };
@@ -131,10 +141,16 @@ struct GroupDesc {  // 16-byte aligned
 constexpr uint32_t kGroupThreads = 256;
 // fwd: bit 0 / bit 1 = operand a / b is the result of the previous op, which the interpreter still holds in registers (5 of the
 // 16 operand reads of C5's body): no shared-memory load for it
+//
+// Over a prime field (kernels.cu: k_arith_groups) the same 32 bytes carry register NUMBERS (the kernel picks the CTA size,
+// hence the layout of the register file, at launch) and the op itself:
+//   dst_off, a_off, b_off = registers, fwd as above, m_and = AG_* kind, m_xor = const-pool index (AG_CONST / AG_ADDC /
+//   AG_MULC), m_a = the assertion's ordinal k in the body (AG_ASSERT), m_c = assertions per call (AG_ASSERT)
 struct GroupOp {
     uint32_t dst_off, a_off, b_off, fwd;
     uint32_t m_and, m_xor, m_a, m_c;
 };
+enum ArithGroupKind : uint32_t { AG_ADD = 0, AG_MUL, AG_ADDC, AG_MULC, AG_CONST, AG_ASSERT };
 constexpr uint32_t kGroupHintShift = 7;  // Plan::group_hints: one entry per 128 calls of a launch
 
 struct InputLoad {  // level-0 values: filled by the input kernel on every pass
