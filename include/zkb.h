@@ -167,6 +167,17 @@ const char* zkb_pending_error(zkb_ctx* ctx);
  * witness batch_idx of the last evaluation — what Evaluator::get (evaluator.rs:750-752) returns
  * for wires bound to those values.  Requires zkb_finalize(ctx, 1). */
 int zkb_read_values(zkb_ctx* ctx, uint32_t batch_idx, const zkb_wire* values, uint64_t n, uint8_t* out_le, size_t stride);
+/* Values to capture on every following run (zkb_evaluate / zkb_run / zkb_comm_* / *_sharded), for every witness of the
+ * batch: the device writes them out tile by tile while the batch is evaluated, so no tile is run again to read them.
+ * After zkb_finalize; n = 0 clears the list.  Same readability rule and errors as zkb_read_values.  A new zkb_finalize
+ * (or a program broadcast to this rank) clears the list.  A captured value that no gate reads is stored on every tile. */
+int zkb_capture_values(zkb_ctx* ctx, const zkb_wire* values, uint64_t n);
+/* What the last run captured for this context's witnesses [first, first + n_witnesses):
+ * out_le[(j - first) * n * stride + i * stride] = value i of witness j, in the bytes zkb_read_values(ctx, j, ...) returns
+ * (canonical residue; the raw bytes of an instance / witness value or of a constant >= p; 0/1 over p = 2).  Needs a run
+ * since the last zkb_capture_values, zkb_finalize or input upload.  On a rank of a communicator, j indexes the rank's own
+ * block of the batch. */
+int zkb_read_captured(zkb_ctx* ctx, uint32_t first, uint32_t n_witnesses, uint8_t* out_le, size_t stride);
 /* value currently bound to IR wire id `wire` in the flat scope of zkb_push_gates */
 int zkb_scope_lookup(zkb_ctx* ctx, uint64_t wire, zkb_wire* out);
 

@@ -112,6 +112,19 @@ public:
         check(zkb_evaluate(ctx_, instances, instance_set_stride, witnesses, witness_set_stride, value_stride, n_batch, out.data()));
         return out;
     }
+    // values of every witness of each following run (zkb_capture_values); empty clears the list
+    void capture(const std::vector<Wire>& values) { check(zkb_capture_values(ctx_, values.data(), values.size())); }
+    // witnesses [first, first + n_witnesses) of the last run, value-minor: n_witnesses x n_values x stride bytes
+    std::vector<uint8_t> read_captured(uint32_t first, uint32_t n_witnesses, uint64_t n_values, size_t stride = 32) {
+        std::vector<uint8_t> out((size_t)n_witnesses * n_values * stride);
+        check(zkb_read_captured(ctx_, first, n_witnesses, out.data(), stride));
+        return out;
+    }
+    std::vector<uint8_t> read_values(uint32_t batch_idx, const std::vector<Wire>& values, size_t stride = 32) {
+        std::vector<uint8_t> out(values.size() * stride);
+        check(zkb_read_values(ctx_, batch_idx, values.data(), values.size(), out.data(), stride));
+        return out;
+    }
     zkb_stats stats() { zkb_stats s; check(zkb_get_stats(ctx_, &s)); return s; }
     const char* pending_error() { return zkb_pending_error(ctx_); }
     zkb_ctx* raw() { return ctx_; }

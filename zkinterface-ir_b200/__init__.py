@@ -20,6 +20,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import threading
 from typing import Iterable, List, Optional, Sequence
 
 import numpy as np
@@ -71,7 +72,8 @@ EXPORTED = [
     "zkb_create", "zkb_destroy", "zkb_last_error", "zkb_set_limits", "zkb_set_field", "zkb_one", "zkb_minus_one", "zkb_zero", "zkb_copy",
     "zkb_constant", "zkb_assert_zero", "zkb_add", "zkb_multiply", "zkb_add_constant", "zkb_mul_constant", "zkb_and",
     "zkb_xor", "zkb_not", "zkb_instance", "zkb_witness", "zkb_push_gates", "zkb_finalize", "zkb_evaluate",
-    "zkb_upload_inputs", "zkb_run", "zkb_assert_info", "zkb_pending_error", "zkb_read_values", "zkb_scope_lookup",
+    "zkb_upload_inputs", "zkb_run", "zkb_assert_info", "zkb_pending_error", "zkb_read_values", "zkb_capture_values",
+    "zkb_read_captured", "zkb_scope_lookup",
     "zkb_get_stats", "zkb_get_timing", "zkb_get_program", "zkb_get_const", "zkb_assert_value", "zkb_level_info", "zkb_evaluator_create", "zkb_evaluator_destroy", "zkb_evaluator_ingest_message",
     "zkb_evaluator_ingest_buffer", "zkb_evaluator_ingest_paths", "zkb_evaluator_get_violations",
     "zkb_evaluator_violation", "zkb_evaluator_get_wire", "zkb_evaluator_lookup", "zkb_evaluator_last_error", "zkb_evaluator_set_flatten", "zkb_evaluator_set_expand_definable", "zkb_evaluator_flatten",
@@ -120,6 +122,8 @@ _sig("zkb_upload_inputs", _i, _vp, _u8p, _u64, _u8p, _u64, _u32, _u32)
 _sig("zkb_run", _i, _vp, _vp)
 _sig("zkb_assert_info", _i, _vp, _u64, _u64p)
 _sig("zkb_read_values", _i, _vp, _u32, _vp, _u64, _u8p, _sz)
+_sig("zkb_capture_values", _i, _vp, _vp, _u64)
+_sig("zkb_read_captured", _i, _vp, _u32, _u32, _u8p, _sz)
 _sig("zkb_scope_lookup", _i, _vp, _u64, _u64p)
 _sig("zkb_get_stats", _i, _vp, C.POINTER(ZkbStats))
 _sig("zkb_get_timing", _i, _vp, C.POINTER(ZkbTiming))
@@ -398,6 +402,26 @@ class GpuBackend:
         self._chk(_lib.zkb_read_values(self._c, batch_idx, _buf(vals), len(vals), _buf(out), stride))
         return [int.from_bytes(out[i].tobytes(), "little") for i in range(len(vals))]
 
+    def capture(self, values: Sequence[int]):
+        """values (handles) whose canonical values every following run writes out for every witness of the batch (read them
+        with read_captured); an empty list clears it"""
+        vals = np.ascontiguousarray(values, dtype=np.uint64)
+        self._chk(_lib.zkb_capture_values(self._c, _buf(vals), len(vals)))
+        self._n_capture = len(vals)
+
+    def read_captured(self, first: int = 0, n: Optional[int] = None, stride: Optional[int] = None) -> np.ndarray:
+        """what the last run captured for witnesses [first, first + n): uint8 [n, n_values, stride], little-endian, the bytes
+        read_values returns (n: to the end of the batch, one witness after a run the Evaluator made itself; stride: the
+        field's element bytes)"""
+        if n is None:
+            n = getattr(self, "_n_batch", 1) - first
+        if stride is None:
+            st = self.stats()
+            stride = 4 if st["binary"] else 4 * st["nlimb"]
+        out = np.zeros((n, getattr(self, "_n_capture", 0), stride), dtype=np.uint8)
+        self._chk(_lib.zkb_read_captured(self._c, first, n, _buf(out), stride))
+        return out
+
     def scope_lookup(self, wire: int) -> int:
         out = C.c_uint64()
         self._chk(_lib.zkb_scope_lookup(self._c, wire, C.byref(out)))
@@ -608,6 +632,7 @@ class ShardedBackend:
             raise ZkbError(rc, msg)
         self.root = self.backends[0]
         self._n_batch = 0
+        self._replicated = False  # the other ranks hold the root's program (the root finalizes once)
 
     def close(self):
         for b in getattr(self, "backends", []):
@@ -631,12 +656,47 @@ class ShardedBackend:
         self.root._chk(_lib.zkb_evaluate_sharded(self._arr, len(self.backends), _buf(inst), iss, _buf(wit), wss, stride, n_batch,
                                                  _buf(out)))
         self._n_batch = n_batch
+        self._replicated = True
         return out
 
     def run(self) -> np.ndarray:
         out = np.zeros(self._n_batch, dtype=VERDICT_DTYPE)
         self.root._chk(_lib.zkb_run_sharded(self._arr, len(self.backends), self._n_batch, _buf(out)))
         return out
+
+    def _fan_out(self, fn):
+        """fn(backend) on every rank at once (a collective blocks until every rank has joined it)"""
+        errs = [None] * len(self.backends)
+
+        def one(i):
+            try:
+                fn(self.backends[i])
+            except ZkbError as e:
+                errs[i] = e
+
+        th = [threading.Thread(target=one, args=(i,)) for i in range(1, len(self.backends))]
+        for t in th:
+            t.start()
+        one(0)
+        for t in th:
+            t.join()
+        for e in errs:
+            if e is not None:
+                raise e
+
+    def capture(self, values: Sequence[int]):
+        """the same capture list on every rank (handles of the root's program); the ranks that have not received the
+        program yet get it first"""
+        if len(self.backends) > 1 and not self._replicated:
+            self._fan_out(lambda b: b.comm_broadcast_program(0))
+            self._replicated = True
+        for b in self.backends:
+            b.capture(values)
+
+    def read_captured(self, stride: Optional[int] = None) -> np.ndarray:
+        """what the last run captured for the whole batch, in batch order: uint8 [n_batch, n_values, stride]"""
+        return np.concatenate([b.read_captured(0, hi - lo, stride)
+                               for b, (lo, hi) in zip(self.backends, (self.shard_of(r, self._n_batch) for r in range(len(self.backends))))])
 
 
 class Source:
@@ -728,6 +788,11 @@ class Evaluator:
         out = C.c_uint64()
         self._chk(_lib.zkb_evaluator_lookup(self._e, wire_id, C.byref(out)))
         return out.value
+
+    def capture_wires(self, wire_ids: Sequence[int]):
+        """capture the live top-scope wires wire_ids on every following run of the backend (GpuBackend.capture); their
+        values come back from backend.read_captured() in this order"""
+        self.backend.capture([self.value_handle(w) for w in wire_ids])
 
     def get(self, wire_id: int) -> int:
         out = C.create_string_buffer(64)

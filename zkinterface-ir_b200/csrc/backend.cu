@@ -89,6 +89,7 @@ int ctx_finalize(zkb_ctx* c, int keep_values) {
         NvtxRange r("zkb:levelize");
         c->plan.build(c->prog, keep_all, &live);
     }
+    capture_reset(c, false);  // the device ops are about to be replaced
     c->keep_all = keep_all;
     c->finalized = true;
     c->resident_tile = -1;
@@ -197,6 +198,10 @@ extern "C" void zkb_destroy(zkb_ctx* c) {
         cudaFree(c->d_tab_opb);
         cudaFree(c->d_tab_readable);
         cudaFree(c->d_tab_kind);
+        cudaFree(c->d_cap_desc);
+        cudaFree(c->d_cap_raw);
+        cudaFree(c->d_cap_unsunk);
+        cudaFree(c->d_cap_out);
         r1cs_free(c);
         comm_free(c);
         group_jit_free(c);
@@ -695,6 +700,7 @@ extern "C" int zkb_upload_inputs(zkb_ctx* c, const uint8_t* inst, uint64_t inst_
     if ((rc = ensure_fail_vectors(c, n_batch)) != ZKB_OK) return rc;
     c->inputs_uploaded = true;
     c->resident_tile = -1;
+    c->cap_valid = false;
     return ZKB_OK;
 }
 
@@ -925,6 +931,26 @@ int ctx_run(zkb_ctx* c, zkb_verdict* out, uint32_t first, uint32_t n_total, bool
     if (rc != ZKB_OK) return rc;
     const uint32_t wt = 1u << c->log2_wt;
     const uint32_t n_tiles = (c->n_batch + wt - 1) / wt;
+    c->cap_valid = false;
+    uint32_t cap_E = 0;
+    if (c->cap_n) {  // every captured value takes E bytes: the widest of an element, an input value and a listed raw constant
+        const size_t eb = c->prog.binary ? 4 : elem_bytes(c);
+        cap_E = (uint32_t)((std::max<size_t>({eb, c->in.stride, c->cap_raw_stride}) + 3) / 4 * 4);
+        const size_t need = (size_t)c->n_batch * c->cap_n * cap_E;
+        if (need > c->cap_out_bytes) {
+            cudaFree(c->d_cap_out);
+            c->d_cap_out = nullptr;
+            c->cap_out_bytes = 0;
+            if (cudaMalloc((void**)&c->d_cap_out, need) != cudaSuccess) {
+                cudaGetLastError();  // not sticky: the context stays usable
+                char buf[160];
+                snprintf(buf, sizeof buf, "capture buffer of %zu bytes (%u witnesses x %llu values x %u) does not fit in device memory",
+                         need, c->n_batch, (unsigned long long)c->cap_n, cap_E);
+                return c->fail(ZKB_E_CUDA, buf);
+            }
+            c->cap_out_bytes = need;
+        }
+    }
     uint64_t launches = 0, level_launches = 0;
     CUDA_TRY(c, cudaEventRecord(c->ev[2], c->stream));
     launch_fill_u32(c->d_first_fail, 0xFFFFFFFFu, n_total, c->sm_count, c->stream);
@@ -932,7 +958,15 @@ int ctx_run(zkb_ctx* c, zkb_verdict* out, uint32_t first, uint32_t n_total, bool
     launches++;
     {
         NvtxRange r_lv("zkb:levels");
-        for (uint32_t t = 0; t < n_tiles; t++) run_tile(c, t, t == n_tiles - 1, c->d_first_fail + first, &launches, &level_launches);
+        for (uint32_t t = 0; t < n_tiles; t++) {
+            run_tile(c, t, t == n_tiles - 1, c->d_first_fail + first, &launches, &level_launches);
+            if (!c->cap_n) continue;
+            // after the tile's last wavefront, before the next tile overwrites the store; outside the tile's level events
+            TileGeom g{c->log2_wt, std::min<uint32_t>(1u << c->log2_wt, c->n_batch - (t << c->log2_wt)), t << c->log2_wt, 0};
+            CUDA_TRY(c, launch_capture(c->prog.binary ? 0 : c->prog.nlimb, c->d_cap_desc, (uint32_t)c->cap_n, c->d_store, c->in, c->d_cap_raw,
+                                       c->cap_raw_stride, g, cap_E, c->d_cap_out, c->prog.fp, c->stream));
+            launches++;
+        }
     }
     if (collective) {
         NvtxRange r_ar("zkb:verdict_allreduce");
@@ -960,6 +994,8 @@ int ctx_run(zkb_ctx* c, zkb_verdict* out, uint32_t first, uint32_t n_total, bool
     c->timing.level_launches = level_launches;
     c->timing.kernel_launches = launches;
     c->n_unreduced_inputs = c->h_res[n_total];
+    c->cap_E = cap_E;
+    c->cap_valid = c->cap_n > 0;
     if (out)
         for (uint32_t j = 0; j < n_total; j++) {
             uint32_t f = c->h_res[j];
@@ -1023,21 +1059,15 @@ __global__ void k_gather_value_tables(const uint64_t* __restrict__ handles, uint
     out[4 * i + 3] = t_kind[v];
 }
 
-extern "C" int zkb_read_values(zkb_ctx* c, uint32_t batch_idx, const zkb_wire* values, uint64_t n, uint8_t* out, size_t stride) {
-    if (!c->finalized || !c->inputs_uploaded) return c->fail(ZKB_E_ARG, "nothing has been evaluated yet");
-    if (!c->has_gpu) return c->fail(ZKB_E_CUDA, "no CUDA device in this context (there is no CPU fallback)");
-    if (batch_idx >= c->n_batch) return c->fail(ZKB_E_ARG, "batch index out of range");
+// Per requested value: its slot, kind and operand b (constant-pool index / stream position of an input), from the host
+// tables or, on a replica, from the device tables (k_gather_value_tables).  Fails on an unknown handle or a value that
+// was not kept on the device.
+static int resolve_values(zkb_ctx* c, const zkb_wire* values, uint64_t n, std::vector<uint32_t>& slots, std::vector<uint32_t>& kinds,
+                          std::vector<uint32_t>& opbs) {
     const Program& p = c->prog;
-    const size_t eb = p.binary ? 4 : elem_bytes(c);
-    CUDA_TRY(c, cudaSetDevice(c->device));
-    uint32_t tile = batch_idx >> c->log2_wt;
-    if (c->resident_tile != (int64_t)tile) {
-        uint64_t a = 0, b = 0;
-        launch_fill_u32(c->d_scratch_fail, 0xFFFFFFFFu, c->n_batch, c->sm_count, c->stream);
-        run_tile(c, tile, true, c->d_scratch_fail, &a, &b);
-    }
-    // per requested value: its slot, kind and operand b (constant-pool index / stream position of an input)
-    std::vector<uint32_t> slots(n), kinds(n), opbs(n);
+    slots.resize(n);
+    kinds.resize(n);
+    opbs.resize(n);
     if (c->is_replica) {
         uint64_t* d_h = nullptr;
         uint32_t* d_t = nullptr;
@@ -1070,6 +1100,25 @@ extern "C" int zkb_read_values(zkb_ctx* c, uint32_t batch_idx, const zkb_wire* v
     for (uint64_t i = 0; i < n; i++)
         if (slots[i] == kNoSlot)
             return c->fail(ZKB_E_ARG, "value was not kept on device (finalize with keep_all_values = 1 to read every value)");
+    return ZKB_OK;
+}
+
+extern "C" int zkb_read_values(zkb_ctx* c, uint32_t batch_idx, const zkb_wire* values, uint64_t n, uint8_t* out, size_t stride) {
+    if (!c->finalized || !c->inputs_uploaded) return c->fail(ZKB_E_ARG, "nothing has been evaluated yet");
+    if (!c->has_gpu) return c->fail(ZKB_E_CUDA, "no CUDA device in this context (there is no CPU fallback)");
+    if (batch_idx >= c->n_batch) return c->fail(ZKB_E_ARG, "batch index out of range");
+    const Program& p = c->prog;
+    const size_t eb = p.binary ? 4 : elem_bytes(c);
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    uint32_t tile = batch_idx >> c->log2_wt;
+    if (c->resident_tile != (int64_t)tile) {
+        uint64_t a = 0, b = 0;
+        launch_fill_u32(c->d_scratch_fail, 0xFFFFFFFFu, c->n_batch, c->sm_count, c->stream);
+        run_tile(c, tile, true, c->d_scratch_fail, &a, &b);
+    }
+    std::vector<uint32_t> slots, kinds, opbs;
+    int rc = resolve_values(c, values, n, slots, kinds, opbs);
+    if (rc != ZKB_OK) return rc;
     uint32_t *d_slots = nullptr, *d_out = nullptr;
     CUDA_TRY(c, cudaMalloc((void**)&d_slots, std::max<size_t>(n, 1) * 4));
     CUDA_TRY(c, cudaMalloc((void**)&d_out, std::max<size_t>(n, 1) * eb));
@@ -1105,6 +1154,135 @@ extern "C" int zkb_read_values(zkb_ctx* c, uint32_t batch_idx, const zkb_wire* v
         while (nb > 0 && src[nb - 1] == 0) nb--;
         if (nb > stride) return c->fail(ZKB_E_ARG, "output stride too small for the value");
         memcpy(dst, src, nb);
+    }
+    return ZKB_OK;
+}
+
+namespace zkb {
+
+void capture_mark_sinks(zkb_ctx* c, bool set) {
+    if (c->cap_n_unsunk) launch_set_sink(c->d_ops, c->d_cap_unsunk, c->cap_n_unsunk, set, c->stream);
+}
+
+void capture_reset(zkb_ctx* c, bool restore_sinks) {
+    if (c->has_gpu) {
+        if (restore_sinks && c->cap_n_unsunk) {
+            capture_mark_sinks(c, true);
+            cudaStreamSynchronize(c->stream);  // the op list is freed below
+        }
+        cudaFree(c->d_cap_desc);
+        cudaFree(c->d_cap_raw);
+        cudaFree(c->d_cap_unsunk);
+    }
+    c->d_cap_desc = nullptr;
+    c->d_cap_raw = nullptr;
+    c->d_cap_unsunk = nullptr;
+    c->cap_n_unsunk = 0;
+    c->cap_raw_stride = 0;
+    c->cap_n = 0;
+    c->cap_valid = false;
+}
+
+}  // namespace zkb
+
+extern "C" int zkb_capture_values(zkb_ctx* c, const zkb_wire* values, uint64_t n) {
+    if (!c->finalized) return c->fail(ZKB_E_ARG, "zkb_finalize must be called first");
+    if (n >= 0xFFFFFFFFull) return c->fail(ZKB_E_ARG, "too many values to capture");
+    if (c->has_gpu) CUDA_TRY(c, cudaSetDevice(c->device));
+    std::vector<uint32_t> slots, kinds, opbs;
+    int rc = resolve_values(c, values, n, slots, kinds, opbs);
+    if (rc != ZKB_OK) return rc;  // the previous list stays
+    const Program& p = c->prog;
+    auto raw_const = [&](uint64_t i) { return kinds[i] == V_CONST && p.const_unreduced[opbs[i]]; };
+    size_t widest = 0;
+    for (uint64_t i = 0; i < n; i++)
+        if (raw_const(i)) widest = std::max(widest, p.const_raw[opbs[i]].size());
+    const uint32_t raw_stride = (uint32_t)((widest + 3) / 4 * 4);
+    std::vector<CaptureDesc> desc(n);
+    std::vector<uint8_t> raw;
+    std::vector<uint32_t> slot_bits(c->plan.n_slots / 32 + 1, 0);  // slots whose producer must store on every tile
+    for (uint64_t i = 0; i < n; i++) {
+        if (kinds[i] == V_INSTANCE || kinds[i] == V_WITNESS) {
+            desc[i] = CaptureDesc{slots[i], kinds[i] == V_INSTANCE ? (uint32_t)CAP_INSTANCE : (uint32_t)CAP_WITNESS, opbs[i], 0};
+        } else if (raw_const(i)) {
+            desc[i] = CaptureDesc{slots[i], CAP_RAW_CONST, (uint32_t)(raw.size() / raw_stride), 0};
+            const auto& r = p.const_raw[opbs[i]];
+            raw.insert(raw.end(), r.begin(), r.end());
+            raw.resize(raw.size() + raw_stride - r.size(), 0);
+        } else {
+            desc[i] = CaptureDesc{slots[i], CAP_STORE, 0, 0};
+            slot_bits[slots[i] >> 5] |= 1u << (slots[i] & 31);
+        }
+    }
+    capture_reset(c, true);
+    if (!c->has_gpu || n == 0) {  // a host-only context only validates the list
+        c->cap_n = n;
+        return ZKB_OK;
+    }
+    // descriptors, raw rows and the sink search; the bitmap and the found-op count live in one scratch allocation
+    uint32_t* d_scratch = nullptr;
+    const size_t scratch_words = slot_bits.size() + 1;
+    cudaError_t e = cudaMalloc((void**)&c->d_cap_desc, n * sizeof(CaptureDesc));
+    if (e == cudaSuccess && !raw.empty()) e = cudaMalloc((void**)&c->d_cap_raw, raw.size());
+    if (e == cudaSuccess) e = cudaMalloc((void**)&c->d_cap_unsunk, n * 4);
+    if (e == cudaSuccess) e = cudaMalloc((void**)&d_scratch, scratch_words * 4);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(c->d_cap_desc, desc.data(), n * sizeof(CaptureDesc), cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess && !raw.empty()) e = cudaMemcpyAsync(c->d_cap_raw, raw.data(), raw.size(), cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(d_scratch, slot_bits.data(), slot_bits.size() * 4, cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(d_scratch + slot_bits.size(), 0, 4, c->stream);
+    uint32_t n_found = 0;
+    if (e == cudaSuccess) {
+        const uint64_t n_ops = c->is_replica ? c->replica_n_ops : c->plan.ops.size();
+        launch_unsink(c->d_ops, n_ops, d_scratch, c->d_cap_unsunk, (uint32_t)n, d_scratch + slot_bits.size(), c->sm_count, c->stream);
+        e = cudaMemcpyAsync(&n_found, d_scratch + slot_bits.size(), 4, cudaMemcpyDeviceToHost, c->stream);
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);  // (also: the pageable sources above are copied)
+    cudaFree(d_scratch);
+    // a written value has one producer and a captured slot is not re-used, so at most n ops are found
+    c->cap_n_unsunk = std::min<uint32_t>(n_found, (uint32_t)n);
+    c->cap_raw_stride = raw_stride;
+    c->cap_n = n;
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        capture_reset(c, true);
+        return c->fail(ZKB_E_CUDA, std::string("zkb_capture_values: ") + cudaGetErrorString(e));
+    }
+    return ZKB_OK;
+}
+
+extern "C" int zkb_read_captured(zkb_ctx* c, uint32_t first, uint32_t n_witnesses, uint8_t* out, size_t stride) {
+    if (!c->finalized) return c->fail(ZKB_E_ARG, "zkb_finalize must be called first");
+    if (!c->has_gpu) return c->fail(ZKB_E_CUDA, "no CUDA device in this context (there is no CPU fallback)");
+    if (!c->cap_valid) return c->fail(ZKB_E_ARG, "nothing has been captured yet (zkb_capture_values, then a run)");
+    if ((uint64_t)first + n_witnesses > c->n_batch) return c->fail(ZKB_E_ARG, "batch index out of range");
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    const size_t E = c->cap_E, n = c->cap_n;
+    const uint8_t* src = c->d_cap_out + (size_t)first * n * E;
+    if (stride == E) {  // the device layout: one copy
+        CUDA_TRY(c, cudaMemcpyAsync(out, src, (size_t)n_witnesses * n * E, cudaMemcpyDeviceToHost, c->stream));
+        CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+        return ZKB_OK;
+    }
+    // other strides: through a host buffer, a block of witnesses at a time
+    const size_t per_w = n * E;
+    const uint32_t chunk = (uint32_t)std::max<size_t>(1, ((size_t)64 << 20) / std::max<size_t>(per_w, 1));
+    std::vector<uint8_t> host(std::min<size_t>(chunk, n_witnesses) * per_w);
+    for (uint32_t w0 = 0; w0 < n_witnesses; w0 += chunk) {
+        const uint32_t nw = std::min(chunk, n_witnesses - w0);
+        CUDA_TRY(c, cudaMemcpyAsync(host.data(), src + (size_t)w0 * per_w, nw * per_w, cudaMemcpyDeviceToHost, c->stream));
+        CUDA_TRY(c, cudaStreamSynchronize(c->stream));
+        for (size_t k = 0; k < (size_t)nw * n; k++) {
+            const uint8_t* v = host.data() + k * E;
+            uint8_t* dst = out + ((size_t)w0 * n + k) * stride;
+            if (stride > E) {
+                memcpy(dst, v, E);
+                memset(dst + E, 0, stride - E);
+            } else {
+                for (size_t b = stride; b < E; b++)
+                    if (v[b]) return c->fail(ZKB_E_ARG, "output stride too small for the value");
+                memcpy(dst, v, stride);
+            }
+        }
     }
     return ZKB_OK;
 }

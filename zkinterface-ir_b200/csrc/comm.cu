@@ -426,10 +426,14 @@ static int broadcast_program(zkb_ctx* c, int root) {
         c->inputs_uploaded = false;
         c->resident_tile = -1;
         c->flat_scope.clear();
+        capture_reset(c, false);  // the device ops are about to be replaced
     }
     lap("unpack");
-    // 3. the device plan, device to device
-    if ((rc = bcast_array(c, c->d_ops, h.n_ops, root, is_root)) != ZKB_OK) return rc;
+    // 3. the device plan, device to device; the root sends its ops as the plan made them, without its capture list's changes
+    if (is_root) capture_mark_sinks(c, true);
+    rc = bcast_array(c, c->d_ops, h.n_ops, root, is_root);
+    if (is_root) capture_mark_sinks(c, false);
+    if (rc != ZKB_OK) return rc;
     if ((rc = bcast_array(c, c->d_aseq, h.n_ops, root, is_root)) != ZKB_OK) return rc;
     if ((rc = bcast_array(c, c->d_loads, h.n_loads, root, is_root)) != ZKB_OK) return rc;
     if ((rc = bcast_array(c, c->d_consts, h.n_consts * h.nlimb, root, is_root)) != ZKB_OK) return rc;  // already in Montgomery form

@@ -197,6 +197,18 @@ struct zkb_ctx {
     std::vector<cudaEvent_t> tile_ev;
     zkb_timing timing{};
 
+    // capture list (zkb_capture_values): written out for every witness after each tile of a run (k_capture)
+    uint64_t cap_n = 0;                      // values in the list (a host-only context validates and counts them)
+    zkb::CaptureDesc* d_cap_desc = nullptr;
+    uint8_t* d_cap_raw = nullptr;            // raw bytes of the listed constants >= p, cap_raw_stride each
+    uint32_t cap_raw_stride = 0;
+    uint32_t* d_cap_unsunk = nullptr;        // device ops whose F_SINK the list cleared (restored when the list goes)
+    uint32_t cap_n_unsunk = 0;
+    uint8_t* d_cap_out = nullptr;            // n_batch x cap_n x cap_E bytes, witness-major
+    size_t cap_out_bytes = 0;
+    uint32_t cap_E = 0;
+    bool cap_valid = false;                  // d_cap_out holds a run over the current list and inputs
+
     zkb::R1csDev* r1cs = nullptr;
     zkb::GroupJit* gjit = nullptr;   // run-time specialisation of the call-group kernel (group_jit.cpp), if any
 
@@ -234,6 +246,10 @@ void ctx_latch(zkb_ctx* c, const std::string& msg);
 void r1cs_free(zkb_ctx* c);
 int ctx_run(zkb_ctx* c, zkb_verdict* out, uint32_t first, uint32_t n_total, bool collective);
 void ctx_finish_e2e_timing(zkb_ctx* c);
+// the capture list's cleared F_SINK flags: back on (set = true) or off again, in the device ops
+void capture_mark_sinks(zkb_ctx* c, bool set);
+// forget the capture list; restore_sinks = false when the device ops it changed are being replaced
+void capture_reset(zkb_ctx* c, bool restore_sinks);
 // comm.cu
 int comm_allreduce_min_u32(zkb_ctx* c, uint32_t* d_buf, size_t n);  // in place, on c->stream
 void comm_free(zkb_ctx* c);

@@ -1092,6 +1092,110 @@ __global__ void k_bool_read_values(const uint32_t* __restrict__ slots, uint32_t 
     out[i] = (word >> (lane & 31)) & 1;
 }
 
+// ---------------------------------------------------------------------------------------------
+// capture list (zkb_capture_values): after a tile's last wavefront, the chosen values of every lane -> a witness-major buffer,
+// in the bytes zkb_read_values returns.  A CTA holds 32 lanes x VB values (blockDim = 32 x VB): the reads are coalesced over
+// lanes (the store is witness-minor), the tile is transposed through shared memory, and the writes are coalesced over values
+// (witness j's VB values are VB * E consecutive bytes of the output).
+// ---------------------------------------------------------------------------------------------
+constexpr uint32_t kCaptureLanes = 32;
+
+template <int N>  // N = 0: p = 2, one bit per lane
+__device__ __forceinline__ void capture_tile(const CaptureDesc* __restrict__ descs, uint32_t n, const uint32_t* __restrict__ store,
+                                             const InputDesc& in, const uint8_t* __restrict__ raw_consts, uint32_t raw_stride,
+                                             const TileGeom& g, uint32_t ew, uint32_t* __restrict__ out, const FieldParams& fp) {
+    extern __shared__ uint32_t cap_sm[];
+    const uint32_t vb = blockDim.y;
+    const uint32_t row = vb * ew + 1;  // words per lane; the odd pitch puts the lanes of a warp in different banks
+    const uint32_t l = threadIdx.x, v = threadIdx.y;
+    const uint32_t i0 = blockIdx.x * vb, i = i0 + v;
+    const uint32_t nv = min(vb, n - i0);
+    const uint32_t n_lane_blocks = (g.n_valid + kCaptureLanes - 1) / kCaptureLanes;
+    CaptureDesc d{0, 0, 0, 0};
+    if (i < n) d = descs[i];
+    for (uint32_t lb = blockIdx.y; lb < n_lane_blocks; lb += gridDim.y) {
+        const uint32_t j = lb * kCaptureLanes + l;  // lane of the tile
+        uint32_t* dst = cap_sm + l * row + v * ew;
+        if (i < n && j < g.n_valid) {
+            uint32_t w = 0;  // words written
+            if (d.kind == CAP_STORE) {
+                if constexpr (N == 0) {
+                    dst[0] = (store[((size_t)d.slot << (g.log2_wt - 5)) + (j >> 5)] >> (j & 31)) & 1;
+                    w = 1;
+                } else {
+                    uint32_t a[N], one[N], r[N];
+                    load_elem<N>(a, store, d.slot, j, g.log2_wt);
+#pragma unroll
+                    for (int k = 0; k < N; k++) one[k] = (k == 0);
+                    fe_mont_mul<N>(r, a, one, fp.p, fp.n0inv);  // leave Montgomery form, as k_read_values does
+#pragma unroll
+                    for (int k = 0; k < N; k++) dst[k] = r[k];
+                    w = N;
+                }
+            } else {  // raw bytes: an input value as the reference holds it, or a constant >= p
+                const uint8_t* src;
+                uint32_t len;
+                if (d.kind == CAP_RAW_CONST) {
+                    src = raw_consts + (size_t)d.opb * raw_stride;
+                    len = raw_stride;
+                } else {
+                    const uint64_t widx = g.batch0 + j;
+                    src = (d.kind == CAP_INSTANCE ? in.inst + widx * in.inst_set_stride : in.wit + widx * in.wit_set_stride) +
+                          (uint64_t)d.opb * in.stride;
+                    len = in.stride;
+                }
+                for (; 4 * w < len; w++) {
+                    uint32_t x = 0;
+                    for (uint32_t b = 0; b < 4 && 4 * w + b < len; b++) x |= (uint32_t)src[4 * w + b] << (8 * b);
+                    dst[w] = x;
+                }
+            }
+            for (; w < ew; w++) dst[w] = 0;
+        }
+        __syncthreads();
+        const uint32_t nl = min(kCaptureLanes, g.n_valid - lb * kCaptureLanes);
+        const uint32_t per_lane = nv * ew;
+        for (uint32_t q = v * kCaptureLanes + l; q < nl * per_lane; q += vb * kCaptureLanes) {
+            const uint32_t ll = q / per_lane, r = q - ll * per_lane;
+            out[((size_t)(g.batch0 + lb * kCaptureLanes + ll) * n + i0) * ew + r] = cap_sm[ll * row + r];
+        }
+        __syncthreads();
+    }
+}
+
+template <int N>
+__global__ void __launch_bounds__(256)
+k_capture(const CaptureDesc* __restrict__ descs, uint32_t n, const uint32_t* __restrict__ store, InputDesc in,
+          const uint8_t* __restrict__ raw_consts, uint32_t raw_stride, TileGeom g, uint32_t ew, uint32_t* __restrict__ out, FieldParams fp) {
+    capture_tile<N>(descs, n, store, in, raw_consts, raw_stride, g, ew, out, fp);
+}
+
+__global__ void __launch_bounds__(256)
+k_bool_capture(const CaptureDesc* __restrict__ descs, uint32_t n, const uint32_t* __restrict__ store, InputDesc in,
+               const uint8_t* __restrict__ raw_consts, uint32_t raw_stride, TileGeom g, uint32_t ew, uint32_t* __restrict__ out, FieldParams fp) {
+    capture_tile<0>(descs, n, store, in, raw_consts, raw_stride, g, ew, out, fp);
+}
+
+// a captured value that no gate reads (F_SINK) must be stored on every tile: clear the flag of the op producing it
+__global__ void k_unsink(GateOp* ops, uint64_t n_ops, const uint32_t* __restrict__ slot_bits, uint32_t* found, uint32_t cap, uint32_t* n_found) {
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n_ops; i += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t m = ops[i].meta;
+        if (!(m & F_SINK)) continue;
+        const uint32_t s = ops[i].out;
+        if (!((slot_bits[s >> 5] >> (s & 31)) & 1)) continue;
+        ops[i].meta = m & ~F_SINK;
+        const uint32_t k = atomicAdd(n_found, 1u);
+        if (k < cap) found[k] = (uint32_t)i;
+    }
+}
+
+__global__ void k_set_sink(GateOp* ops, const uint32_t* __restrict__ idx, uint32_t n, uint32_t set) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    GateOp& op = ops[idx[i]];
+    op.meta = set ? (op.meta | F_SINK) : (op.meta & ~F_SINK);
+}
+
 __global__ void k_fill_u32(uint32_t* p, uint32_t v, uint64_t n) {
     for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x) p[i] = v;
 }
@@ -1469,6 +1573,46 @@ void launch_bool_read_values(const uint32_t* slots, uint32_t n, const uint32_t* 
                              uint32_t* out, cudaStream_t s) {
     if (n == 0) return;
     k_bool_read_values<<<(n + 127) / 128, 128, 0, s>>>(slots, n, store, lane, log2_wt, out);
+}
+
+template <class K>
+static cudaError_t launch_capture_k(K kernel, const CaptureDesc* descs, uint32_t n, const uint32_t* store, const InputDesc& in,
+                                   const uint8_t* raw_consts, uint32_t raw_stride, const TileGeom& g, uint32_t ew, uint8_t* out,
+                                   const FieldParams& fp, cudaStream_t s) {
+    // 8 values a CTA (256 threads) while the transpose buffer fits the default 48 KB, fewer for wide raw inputs
+    auto smem_for = [&](uint32_t vb) { return (size_t)kCaptureLanes * (vb * ew + 1) * 4; };
+    uint32_t vb = 8;
+    while (vb > 1 && smem_for(vb) > 48 * 1024) vb >>= 1;
+    const size_t smem = smem_for(vb);
+    if (smem > 48 * 1024) {
+        if (smem > 227 * 1024) return cudaErrorInvalidValue;
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return e;
+    }
+    const uint32_t lane_blocks = (g.n_valid + kCaptureLanes - 1) / kCaptureLanes;
+    const dim3 grid((n + vb - 1) / vb, std::min<uint32_t>(lane_blocks, 65535));
+    kernel<<<grid, dim3(kCaptureLanes, vb), smem, s>>>(descs, n, store, in, raw_consts, raw_stride, g, ew, (uint32_t*)out, fp);
+    return cudaPeekAtLastError();
+}
+
+cudaError_t launch_capture(int nlimb, const CaptureDesc* descs, uint32_t n, const uint32_t* store, InputDesc in, const uint8_t* raw_consts,
+                           uint32_t raw_stride, TileGeom g, uint32_t E, uint8_t* out, const FieldParams& fp, cudaStream_t s) {
+    if (n == 0 || g.n_valid == 0) return cudaSuccess;
+    cudaError_t e = cudaSuccess;
+    if (nlimb == 0) return launch_capture_k(k_bool_capture, descs, n, store, in, raw_consts, raw_stride, g, E / 4, out, fp, s);
+    ZKB_DISPATCH_N(nlimb, (e = launch_capture_k(k_capture<N>, descs, n, store, in, raw_consts, raw_stride, g, E / 4, out, fp, s)));
+    return e;
+}
+
+void launch_unsink(GateOp* ops, uint64_t n_ops, const uint32_t* slot_bits, uint32_t* found, uint32_t cap, uint32_t* n_found, int sm_count,
+                   cudaStream_t s) {
+    if (n_ops == 0) return;
+    k_unsink<<<grid_for(n_ops, sm_count, 8), 256, 0, s>>>(ops, n_ops, slot_bits, found, cap, n_found);
+}
+
+void launch_set_sink(GateOp* ops, const uint32_t* idx, uint32_t n, bool set, cudaStream_t s) {
+    if (n == 0) return;
+    k_set_sink<<<(n + 255) / 256, 256, 0, s>>>(ops, idx, n, set ? 1u : 0u);
 }
 
 void launch_fill_u32(uint32_t* p, uint32_t v, uint64_t n, int sm_count, cudaStream_t s) {

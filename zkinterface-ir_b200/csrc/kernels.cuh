@@ -94,6 +94,26 @@ void launch_bool_groups(const GroupDesc* descs, uint32_t n_groups, uint64_t tota
 void launch_bool_read_values(const uint32_t* slots, uint32_t n, const uint32_t* store, uint32_t lane, uint32_t log2_wt,
                              uint32_t* out, cudaStream_t s);
 
+// capture list (zkb_capture_values): what one captured value is read from
+enum CaptureKind : uint32_t {
+    CAP_STORE = 0,  // the wire store at `slot` (canonical residue; 0/1 over p = 2)
+    CAP_INSTANCE,   // raw bytes of instance value `opb` (d_inst)
+    CAP_WITNESS,    // raw bytes of witness value `opb` (d_wit)
+    CAP_RAW_CONST,  // row `opb` of the capture list's table of constants >= p
+};
+struct CaptureDesc {
+    uint32_t slot, kind, opb, pad;
+};
+// one tile's captured values -> out, witness-major: value i of tile lane j at out + ((g.batch0 + j) * n + i) * E bytes
+// (E a multiple of 4, the value zero padded to E).  nlimb = 0: p = 2 (k_bool_capture), else k_capture<nlimb>.
+cudaError_t launch_capture(int nlimb, const CaptureDesc* descs, uint32_t n, const uint32_t* store, InputDesc in, const uint8_t* raw_consts,
+                           uint32_t raw_stride, TileGeom g, uint32_t E, uint8_t* out, const FieldParams& fp, cudaStream_t s);
+// ops whose result lands in a slot marked in slot_bits and that carry F_SINK: clear the flag and list the op (up to cap of
+// them; *n_found counts all).  launch_set_sink: F_SINK on (set) or off the listed ops.
+void launch_unsink(GateOp* ops, uint64_t n_ops, const uint32_t* slot_bits, uint32_t* found, uint32_t cap, uint32_t* n_found, int sm_count,
+                   cudaStream_t s);
+void launch_set_sink(GateOp* ops, const uint32_t* idx, uint32_t n, bool set, cudaStream_t s);
+
 void launch_fill_u32(uint32_t* p, uint32_t v, uint64_t n, int sm_count, cudaStream_t s);
 
 }  // namespace zkb
