@@ -262,6 +262,35 @@ int zkb_evaluator_get_wire(zkb_evaluator* ev, uint64_t wire_id, uint8_t* out_le,
 int zkb_evaluator_lookup(zkb_evaluator* ev, uint64_t wire_id, zkb_wire* out);
 const char* zkb_evaluator_last_error(zkb_evaluator* ev);
 
+/* Value sets: one relation checked against many instance / witness sets in one device batch.  A value set is a group of
+ * Instance / Witness messages; values ingested with the calls above are COMMON to every set.  Set j's statement is: the
+ * common instance messages, then set j's; the common witness messages, then set j's; the relation message(s).  Its result
+ * is what zkb_evaluator_get_violations returns for that statement on its own (evaluator.rs:199-208).
+ * Batch mode begins with the first set; every set must be added before the first relation message, and so must the common
+ * values.  The relation is recorded once, against the longest streams; while recording, a panic no longer fails the ingest
+ * call: like a recording error, it ends the recording and is decided per set.  Refused with ZKB_E_ARG: a set after a
+ * relation message, a Relation message inside a set, a set on a flatten / expand-definable evaluator, get_violations /
+ * get_wire once a set is added, a set index out of range.  A host-only backend records; its batch results are ZKB_E_CUDA. */
+/* One set from a concatenation of size-prefixed Instance / Witness messages. */
+int zkb_evaluator_add_value_set_buffer(zkb_evaluator* ev, const uint8_t* buf, size_t len);
+/* One set from files / directories of *.sieve, in Source order (source.rs:69-89); errors name the file. */
+int zkb_evaluator_add_value_set_paths(zkb_evaluator* ev, const char* const* paths, size_t n_paths);
+/* number of value sets added */
+size_t zkb_evaluator_value_sets(zkb_evaluator* ev);
+/* Split the batch over the contexts of one communicator (zkb_comm_init, same order; ctxs[0] is the evaluator's backend)
+ * with zkb_evaluate_sharded.  With fewer sets than contexts the batch runs on ctxs[0] alone. */
+int zkb_evaluator_use_devices(zkb_evaluator* ev, zkb_ctx** ctxs, int n);
+/* Result of set `set`; the first call evaluates the whole batch (once).  *status ZKB_OK: the set's violation strings
+ * follow (none: the statement is TRUE); ZKB_E_FATAL: the reference panics on this statement, the one string is the
+ * panic text.  The call itself fails only for the whole batch (argument, CUDA). */
+int zkb_evaluator_batch_result(zkb_evaluator* ev, uint64_t set, int* status, size_t* n_violations);
+const char* zkb_evaluator_batch_violation(zkb_evaluator* ev, uint64_t set, size_t i);
+/* Evaluator::get(id) for one set: read back on the context that evaluated it, from the top scope the whole recording left.
+ * ZKB_E_FATAL for a set whose statement panics.  ZKB_E_ARG for a set whose recording stops early (a stream of its own runs
+ * out, or the relation's own error is reached: its violations end with that error), since its statement's scope at that
+ * point can differ from the final one. */
+int zkb_evaluator_get_wire_of(zkb_evaluator* ev, uint64_t set, uint64_t wire_id, uint8_t* out_le, size_t cap, size_t* len);
+
 /* `zki_sieve flatten` (cli.rs:442-472): the Evaluator driving the reference's IRFlattener backend
  * (consumers/flattening.rs:42-191) instead of an evaluating one.  Call set_flatten(ev, 1) BEFORE ingesting; the
  * statement is then recorded gate for gate as the IRFlattener's GateBuilder would emit it (one SIMPLE gate per
@@ -372,6 +401,10 @@ int zkb_debug_write_flat_relation(zkb_ctx* ctx, const uint8_t* modulus_le, size_
                                   const zkb_gate* gates, uint64_t n_gates, const uint8_t* const_pool_le, size_t const_stride,
                                   uint64_t n_consts, const uint8_t** out, size_t* out_len);
 int zkb_debug_r1cs_layout(zkb_ctx* ctx, int kind, uint64_t counts[3], uint32_t* slices, uint32_t* terms, uint32_t* row_ids);
+/* Cut point of value set `set`, from the recording alone (host-only contexts too): *what 0 none, 1 its instance stream is
+ * found empty, 2 its witness stream is found empty, 3 the recording's own error / panic; *seq = assertions recorded before
+ * that point (UINT64_MAX: none).  A failing assertion with a smaller seq is the set's violation; else the cut decides. */
+int zkb_debug_value_set_cut(zkb_evaluator* ev, uint64_t set, uint64_t* seq, int* what);
 
 /* ------------------------------------------------------------------ 7. multi-GPU (witness-batch sharding)
  * The reference is single-threaded (evaluator.rs:191-230 checks one witness at a time); the path shards over independent

@@ -184,6 +184,44 @@ public:
     }
     GpuBackend& backend() { return backend_; }
 
+    // value sets (zkb.h section 4): one relation, one statement per set; every set before the first relation message
+    void add_value_set(const Source& src) {
+        if (src.in_memory()) {
+            std::vector<uint8_t> all;
+            for (const auto& b : src.buffers()) all.insert(all.end(), b.begin(), b.end());
+            check(zkb_evaluator_add_value_set_buffer(ev_, all.data(), all.size()));
+        } else {
+            std::vector<const char*> ptrs;
+            for (const auto& p : src.paths()) ptrs.push_back(p.c_str());
+            check(zkb_evaluator_add_value_set_paths(ev_, ptrs.data(), ptrs.size()));
+        }
+    }
+    // the contexts of one communicator (zkb_comm_init order), ctxs[0] = backend().raw()
+    void use_devices(std::vector<zkb_ctx*> ctxs) { check(zkb_evaluator_use_devices(ev_, ctxs.data(), (int)ctxs.size())); }
+    struct SetResult {
+        int status;                           // ZKB_OK, or ZKB_E_FATAL: the statement panics, violations[0] is the panic text
+        std::vector<std::string> violations;  // what get_violations returns for the set's statement
+    };
+    std::vector<SetResult> get_batch_violations() {
+        std::vector<SetResult> out;
+        const size_t n_sets = zkb_evaluator_value_sets(ev_);
+        if (n_sets == 0) check(zkb_evaluator_batch_result(ev_, 0, nullptr, nullptr));
+        for (size_t j = 0; j < n_sets; j++) {
+            SetResult r;
+            size_t n = 0;
+            check(zkb_evaluator_batch_result(ev_, j, &r.status, &n));
+            for (size_t i = 0; i < n; i++) r.violations.emplace_back(zkb_evaluator_batch_violation(ev_, j, i));
+            out.push_back(std::move(r));
+        }
+        return out;
+    }
+    Value get(uint64_t set, uint64_t wire_id) {  // Evaluator::get for one set
+        uint8_t buf[64];
+        size_t n = 0;
+        check(zkb_evaluator_get_wire_of(ev_, set, wire_id, buf, sizeof buf, &n));
+        return Value(buf, buf + n);
+    }
+
 private:
     void check(int rc) {
         if (rc != ZKB_OK) throw Error(rc, zkb_evaluator_last_error(ev_));

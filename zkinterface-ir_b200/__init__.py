@@ -77,7 +77,9 @@ EXPORTED = [
     "zkb_get_stats", "zkb_get_timing", "zkb_get_program", "zkb_get_const", "zkb_assert_value", "zkb_level_info", "zkb_evaluator_create", "zkb_evaluator_destroy", "zkb_evaluator_ingest_message",
     "zkb_evaluator_ingest_buffer", "zkb_evaluator_ingest_paths", "zkb_evaluator_get_violations",
     "zkb_evaluator_violation", "zkb_evaluator_get_wire", "zkb_evaluator_lookup", "zkb_evaluator_last_error", "zkb_evaluator_set_flatten", "zkb_evaluator_set_expand_definable", "zkb_evaluator_flatten",
-    "zkb_evaluator_flatten_to_dir", "zkb_validator_create", "zkb_validator_destroy", "zkb_validator_ingest_message",
+    "zkb_evaluator_flatten_to_dir", "zkb_evaluator_add_value_set_buffer", "zkb_evaluator_add_value_set_paths",
+    "zkb_evaluator_value_sets", "zkb_evaluator_use_devices", "zkb_evaluator_batch_result", "zkb_evaluator_batch_violation",
+    "zkb_evaluator_get_wire_of", "zkb_debug_value_set_cut", "zkb_validator_create", "zkb_validator_destroy", "zkb_validator_ingest_message",
     "zkb_validator_ingest_buffer", "zkb_validator_ingest_paths", "zkb_validator_get_violations", "zkb_validator_violation",
     "zkb_validator_how_many_violations", "zkb_validator_live_wires", "zkb_validator_set_limits", "zkb_validator_last_error", "zkb_metrics_create", "zkb_metrics_destroy", "zkb_metrics_ingest_message",
     "zkb_metrics_ingest_buffer", "zkb_metrics_ingest_paths", "zkb_metrics_json", "zkb_metrics_last_error", "zkb_r1cs_load", "zkb_r1cs_check",
@@ -146,6 +148,14 @@ _sig("zkb_evaluator_set_expand_definable", _i, _vp, C.c_char_p)
 _sig("zkb_evaluator_flatten", _i, _vp, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.POINTER(C.c_void_p),
      C.POINTER(C.c_size_t), C.POINTER(C.c_void_p), C.POINTER(C.c_size_t))
 _sig("zkb_evaluator_flatten_to_dir", _i, _vp, C.c_char_p)
+_sig("zkb_evaluator_add_value_set_buffer", _i, _vp, _u8p, _sz)
+_sig("zkb_evaluator_add_value_set_paths", _i, _vp, C.POINTER(C.c_char_p), _sz)
+_sig("zkb_evaluator_value_sets", _sz, _vp)
+_sig("zkb_evaluator_use_devices", _i, _vp, C.POINTER(C.c_void_p), _i)
+_sig("zkb_evaluator_batch_result", _i, _vp, _u64, C.POINTER(C.c_int), C.POINTER(C.c_size_t))
+_sig("zkb_evaluator_batch_violation", C.c_char_p, _vp, _u64, _sz)
+_sig("zkb_evaluator_get_wire_of", _i, _vp, _u64, _u64, _u8p, _sz, C.POINTER(C.c_size_t))
+_sig("zkb_debug_value_set_cut", _i, _vp, _u64, _u64p, C.POINTER(C.c_int))
 _sig("zkb_validator_create", _vp, _i)
 _sig("zkb_validator_destroy", None, _vp)
 _sig("zkb_validator_ingest_message", _i, _vp, _u8p, _sz)
@@ -378,6 +388,11 @@ class GpuBackend:
     def upload_inputs(self, instances, witnesses, n_batch: int):
         inst, iss, wit, wss, stride = self._strides(instances, witnesses, n_batch)
         self._chk(_lib.zkb_upload_inputs(self._c, _buf(inst), iss, _buf(wit), wss, stride, n_batch))
+        self._n_batch = n_batch
+
+    def resident_batch(self, n_batch: int):
+        """the library itself uploaded the inputs of a batch of n_batch (an Evaluator's value sets): run() and
+        read_captured() use them"""
         self._n_batch = n_batch
 
     def run(self) -> np.ndarray:
@@ -659,6 +674,12 @@ class ShardedBackend:
         self._replicated = True
         return out
 
+    def resident_batch(self, n_batch: int):
+        """the library itself evaluated a batch of n_batch over these contexts (zkb_evaluate_sharded, e.g. an Evaluator's
+        value sets): every rank holds the program and its block of the inputs; run() and read_captured() use them"""
+        self._n_batch = n_batch
+        self._replicated = True
+
     def run(self) -> np.ndarray:
         out = np.zeros(self._n_batch, dtype=VERDICT_DTYPE)
         self.root._chk(_lib.zkb_run_sharded(self._arr, len(self.backends), self._n_batch, _buf(out)))
@@ -729,6 +750,8 @@ class Evaluator:
         flatten = flatten or expand_gate_set is not None
         self.backend = backend or GpuBackend(-1 if flatten else device)
         self._e = _lib.zkb_evaluator_create(self.backend._c)
+        self._n_sets = 0
+        self._sharded = None
         if expand_gate_set is not None:   # ExpandDefinable in front of the flattener (consumers/exp_definable.rs)
             self._chk(_lib.zkb_evaluator_set_expand_definable(self._e, expand_gate_set.encode()))
         elif flatten:
@@ -791,8 +814,68 @@ class Evaluator:
 
     def capture_wires(self, wire_ids: Sequence[int]):
         """capture the live top-scope wires wire_ids on every following run of the backend (GpuBackend.capture); their
-        values come back from backend.read_captured() in this order"""
-        self.backend.capture([self.value_handle(w) for w in wire_ids])
+        values come back from backend.read_captured() in this order.  With value sets: a capture list can only be set on a
+        finalized program, so the batch is evaluated (once, if get_batch_violations has not done it) and then run once more
+        with the list; read_captured() of the backend that ran it (the ShardedBackend given to use_devices when the batch was
+        split, else `backend`) returns [set, wire, bytes] for every set.  The values are those of the relation recorded in
+        full: for a set whose recording stops early (value_set_cut(set)[0] != 0), values defined after its cut are computed
+        from zero-padded inputs and are not part of its statement."""
+        handles = [self.value_handle(w) for w in wire_ids]
+        if not self._n_sets:
+            self.backend.capture(handles)
+            return
+        self.get_batch_violations()
+        runner = self._batch_runner()
+        runner.resident_batch(self._n_sets)
+        runner.capture(handles)
+        runner.run()
+
+    # ---- value sets: one relation, many instance / witness sets (zkb.h section 4) ----------------------------------
+    def add_value_set(self, source: Source):
+        """one value set (Instance / Witness messages); every set comes before the first relation message"""
+        if source.buffers is not None:
+            b = b"".join(source.buffers)
+            self._chk(_lib.zkb_evaluator_add_value_set_buffer(self._e, _buf(b), len(b)))
+        else:
+            arr = (C.c_char_p * len(source.paths))(*[p.encode() for p in source.paths])
+            self._chk(_lib.zkb_evaluator_add_value_set_paths(self._e, arr, len(source.paths)))
+        self._n_sets = int(_lib.zkb_evaluator_value_sets(self._e))
+
+    def use_devices(self, sharded: ShardedBackend):
+        """split the batch over sharded's contexts; sharded.root must be this evaluator's backend"""
+        self._chk(_lib.zkb_evaluator_use_devices(self._e, sharded._arr, len(sharded.backends)))
+        self._sharded = sharded
+
+    def get_batch_violations(self) -> List[tuple]:
+        """[(status, violations)] per set: (ZKB_OK, what get_violations returns for the set's statement) or
+        (ZKB_E_FATAL, [panic text]) where that statement makes the reference panic"""
+        out = []
+        st, n = C.c_int(), C.c_size_t()
+        for j in range(self._n_sets):
+            self._chk(_lib.zkb_evaluator_batch_result(self._e, j, C.byref(st), C.byref(n)))
+            out.append((st.value, [_lib.zkb_evaluator_batch_violation(self._e, j, i).decode("utf-8", "replace")
+                                   for i in range(n.value)]))
+        if not self._n_sets:   # the library's refusal
+            self._chk(_lib.zkb_evaluator_batch_result(self._e, 0, C.byref(st), C.byref(n)))
+        return out
+
+    def get_of(self, set_index: int, wire_id: int) -> int:
+        """Evaluator.get for one value set (ZKB_E_ARG for a set whose recording stops early: value_set_cut)"""
+        out = C.create_string_buffer(64)
+        n = C.c_size_t()
+        self._chk(_lib.zkb_evaluator_get_wire_of(self._e, set_index, wire_id, C.cast(out, C.c_void_p), 64, C.byref(n)))
+        return int.from_bytes(out.raw[:n.value], "little")
+
+    def value_set_cut(self, set_index: int):
+        """(what, seq) of a set's cut point, from the recording alone: what 0 none, 1 instance stream empty, 2 witness
+        stream empty, 3 the recording's own error / panic; seq = assertions recorded before it (None: no cut)"""
+        seq, what = C.c_uint64(), C.c_int()
+        self._chk(_lib.zkb_debug_value_set_cut(self._e, set_index, C.byref(seq), C.byref(what)))
+        return what.value, (None if what.value == 0 else seq.value)
+
+    def _batch_runner(self):
+        sh = self._sharded
+        return sh if sh is not None and len(sh.backends) > 1 and self._n_sets >= len(sh.backends) else self.backend
 
     def get(self, wire_id: int) -> int:
         out = C.create_string_buffer(64)

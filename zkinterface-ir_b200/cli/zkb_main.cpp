@@ -1,5 +1,7 @@
 // zkb — verbs of zki_sieve (rust/src/cli.rs) on the GPU backend.
 //   zkb evaluate [--device N] <workspace dir | *.sieve ... | ->       cli.rs:130, 315-320, 557-571
+//   zkb evaluate [--device N | --devices a,b,...] --sets DIR <paths...>
+//                                                                     one statement per subdirectory of DIR (its value set)
 //   zkb flatten --out <dir | -> <workspace dir | *.sieve ... | ->     cli.rs:442-472 (host only)
 //   zkb expand-definable --gate-set <s> --out <dir | -> <paths...>    cli.rs:513-553 (host only)
 //   zkb validate <workspace dir | *.sieve ... | ->                    cli.rs:297-313 (host only)
@@ -8,10 +10,13 @@
 // `evaluate` / `validate` print exactly what the reference prints on stderr ("The statement is TRUE!" /
 // "The statement is COMPLIANT with the specification!" / the violation lists) and exit non-zero with
 // "Found N violations." when there are any.
+#include <dirent.h>
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <sys/stat.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -19,13 +24,17 @@
 
 static int usage(const char* argv0) {
     fprintf(stderr,
-            "usage: %s evaluate [--device N] <paths...>\n"
+            "usage: %s evaluate [--device N | --devices a,b,...] [--sets DIR] <paths...>\n"
             "       %s flatten --out <dir|-> <paths...>\n"
             "       %s expand-definable --gate-set <gateset> --out <dir|-> <paths...>\n"
             "       %s validate <paths...>\n"
             "       %s metrics <paths...>\n"
             "       %s valid-eval-metrics [--device N] <paths...>\n",
             argv0, argv0, argv0, argv0, argv0, argv0);
+    fprintf(stderr,
+            "  --sets DIR      every subdirectory of DIR is one value set (instance / witness .sieve files); <paths> hold the\n"
+            "                  relation and the values common to all sets\n"
+            "  --devices LIST  split the sets over these device ordinals (repeats share one device)\n");
     return 2;
 }
 
@@ -43,18 +52,112 @@ static int print_violations(size_t n, const std::vector<std::string>& v, const c
     return 0;
 }
 
+// "0,1,1": device ordinals, at least one
+static bool parse_devices(const char* list, std::vector<int>& out) {
+    std::string s = list;
+    size_t pos = 0;
+    while (true) {
+        size_t comma = s.find(',', pos);
+        std::string item = s.substr(pos, comma == std::string::npos ? std::string::npos : comma - pos);
+        char* end = nullptr;
+        long d = strtol(item.c_str(), &end, 10);
+        if (item.empty() || *end != '\0' || d < 0 || d > 1024) return false;
+        out.push_back((int)d);
+        if (comma == std::string::npos) return true;
+        pos = comma + 1;
+    }
+}
+
+static int fail_with(const char* msg) {
+    fprintf(stderr, "Error: %s\n", msg);
+    return 1;
+}
+
+// zkb evaluate --sets DIR <paths...>: one statement per subdirectory of DIR, each printed as `zkb evaluate <paths...>
+// DIR/<name>` prints it, after a "== <name> ==" line
+static int evaluate_sets(const char* sets_dir, const std::vector<int>& devs, bool comm, const std::vector<const char*>& paths) {
+    std::vector<std::string> names;
+    DIR* d = opendir(sets_dir);
+    if (!d) {
+        fprintf(stderr, "Error: cannot read directory %s\n", sets_dir);
+        return 1;
+    }
+    while (dirent* e = readdir(d)) {
+        std::string name = e->d_name;
+        struct stat st;
+        if (name == "." || name == ".." || stat((std::string(sets_dir) + "/" + name).c_str(), &st) != 0 || !S_ISDIR(st.st_mode)) continue;
+        names.push_back(name);
+    }
+    closedir(d);
+    std::sort(names.begin(), names.end());
+    if (names.empty()) {
+        fprintf(stderr, "Error: no value set (subdirectory) in %s\n", sets_dir);
+        return 1;
+    }
+    std::vector<zkb_ctx*> ctxs;
+    for (int dev : devs) {
+        ctxs.push_back(zkb_create(dev));
+        if (zkb_last_error(ctxs.back())[0]) return fail_with(zkb_last_error(ctxs.back()));
+    }
+    zkb_evaluator* ev = zkb_evaluator_create(ctxs[0]);
+    if (comm) {  // --devices: the contexts form one communicator, the sets are split over them
+        if (zkb_comm_init(ctxs.data(), (int)ctxs.size()) != ZKB_OK) return fail_with(zkb_last_error(ctxs[0]));
+        if (zkb_evaluator_use_devices(ev, ctxs.data(), (int)ctxs.size()) != ZKB_OK) return fail_with(zkb_evaluator_last_error(ev));
+    }
+    for (const auto& name : names) {
+        const std::string dir = std::string(sets_dir) + "/" + name;
+        const char* p = dir.c_str();
+        if (zkb_evaluator_add_value_set_paths(ev, &p, 1) != ZKB_OK) return fail_with(zkb_evaluator_last_error(ev));
+    }
+    if (zkb_evaluator_ingest_paths(ev, paths.data(), paths.size()) != ZKB_OK) return fail_with(zkb_evaluator_last_error(ev));
+    size_t not_true = 0;
+    for (size_t j = 0; j < names.size(); j++) {
+        int status = ZKB_OK;
+        size_t n = 0;
+        if (zkb_evaluator_batch_result(ev, j, &status, &n) != ZKB_OK) return fail_with(zkb_evaluator_last_error(ev));
+        fprintf(stderr, "== %s ==\n", names[j].c_str());
+        if (status != ZKB_OK) {
+            fprintf(stderr, "Error: %s\n", zkb_evaluator_batch_violation(ev, j, 0));
+            not_true++;
+            continue;
+        }
+        std::vector<std::string> v;
+        for (size_t i = 0; i < n; i++) v.push_back(zkb_evaluator_batch_violation(ev, j, i));
+        not_true += print_violations(n, v, "TRUE") != 0;
+    }
+    zkb_evaluator_destroy(ev);
+    for (auto c : ctxs) zkb_destroy(c);
+    if (not_true) {
+        fprintf(stderr, "Error: %zu of %zu statements are NOT TRUE.\n", not_true, names.size());
+        return 1;
+    }
+    return 0;
+}
+
 int main(int argc, char** argv) {
     if (argc < 3) return usage(argv[0]);
     const std::string verb = argv[1];
     int device = 0;
+    bool device_given = false;
     const char* out = nullptr;
     const char* gate_set = nullptr;
+    const char* sets_dir = nullptr;
+    const char* devices_list = nullptr;
     std::vector<const char*> paths;
     for (int i = 2; i < argc; i++) {
-        if (strcmp(argv[i], "--device") == 0 && i + 1 < argc) device = atoi(argv[++i]);
+        if (strcmp(argv[i], "--device") == 0 && i + 1 < argc) device = atoi(argv[++i]), device_given = true;
         else if (strcmp(argv[i], "--out") == 0 && i + 1 < argc) out = argv[++i];
         else if (strcmp(argv[i], "--gate-set") == 0 && i + 1 < argc) gate_set = argv[++i];
+        else if (verb == "evaluate" && strcmp(argv[i], "--sets") == 0 && i + 1 < argc) sets_dir = argv[++i];
+        else if (verb == "evaluate" && strcmp(argv[i], "--devices") == 0 && i + 1 < argc) devices_list = argv[++i];
         else paths.push_back(argv[i]);
+    }
+    if (verb == "evaluate" && (sets_dir || devices_list)) {
+        if (!sets_dir || device_given) return usage(argv[0]);  // --devices needs --sets, and excludes --device
+        std::vector<int> devs;
+        if (devices_list && !parse_devices(devices_list, devs)) return usage(argv[0]);
+        if (devs.empty()) devs.push_back(device);
+        return evaluate_sets(sets_dir, devs, devices_list != nullptr, paths);
     }
     if (verb == "evaluate") {
         zkb_ctx* ctx = zkb_create(device);

@@ -86,6 +86,8 @@ std::string u64s(uint64_t v) { return std::to_string((unsigned long long)v); }
 
 }  // namespace
 
+static unsigned parse_threads();
+
 struct zkb_evaluator {
     zkb_ctx* c;
     std::string err;
@@ -106,6 +108,44 @@ struct zkb_evaluator {
     std::vector<std::string> violations;
     std::vector<uint8_t> flat_out[3];  // flatten output (instance, witness, relation), owned here
     std::vector<Scope*> scope_pool;
+
+    // ---- value sets (batch mode, zkb.h section 4) -------------------------------------------------------------------
+    // Set j's statement is: the common instance values, set j's; the common witness values, set j's; the relation.  The
+    // relation is recorded once, against the longest streams: stream positions past the common values stand for the sets'
+    // values.  Values of all sets are kept packed, trimmed of trailing zero bytes, one arena per stream.
+    struct Arena {
+        std::vector<uint8_t> bytes;
+        std::vector<uint64_t> end{0};  // value k is bytes[end[k], end[k + 1])
+        size_t widest = 0;
+        uint64_t size() const { return end.size() - 1; }
+        void push(const std::vector<uint8_t>& v) {
+            size_t n = v.size();
+            while (n > 0 && v[n - 1] == 0) n--;
+            bytes.insert(bytes.end(), v.data(), v.data() + n);
+            end.push_back(bytes.size());
+            widest = std::max(widest, n);
+        }
+    };
+    struct ValueSet {
+        uint64_t inst0, n_inst, wit0, n_wit;  // ranges in the arenas
+    };
+    Arena set_inst, set_wit;
+    std::vector<ValueSet> sets;
+    uint64_t max_set_inst = 0, max_set_wit = 0;
+    bool relation_seen = false;
+    uint32_t n_common_inst = 0, n_common_wit = 0;  // stream positions of the common values, fixed at the first relation
+    // the first recording error or panic in batch mode (it ends the recording, as in a single statement): value handles
+    // recorded before it, its text, and whether it is a panic
+    uint32_t global_cut = UINT32_MAX;
+    std::string global_cut_msg;
+    bool global_cut_fatal = false;
+    std::vector<zkb_ctx*> devices;  // zkb_evaluator_use_devices: the batch is split over these contexts
+    bool batch_evaluated = false, batch_sharded = false;
+    std::vector<int> set_status;
+    std::vector<std::vector<std::string>> set_violations;
+    std::vector<uint32_t> set_cut;  // value handles recorded before each set's cut (UINT32_MAX: none)
+
+    bool batch() const { return !sets.empty(); }
 
     explicit zkb_evaluator(zkb_ctx* ctx) : c(ctx) {}
     ~zkb_evaluator() {
@@ -1134,7 +1174,7 @@ struct zkb_evaluator {
                               size_t* serial_n) {
         Program& p = prog();
         *serial_n = w1 - w0;
-        if (fatal || evaluated || has_error || p.keep_copies || p.expand_on || !values.sparse.empty() || getenv("ZKB_NO_FLAT_INGEST")) return 0;
+        if (fatal || evaluated || batch_evaluated || has_error || p.keep_copies || p.expand_on || !values.sparse.empty() || getenv("ZKB_NO_FLAT_INGEST")) return 0;
         size_t nm = w1 - w0;
         static const bool timing = getenv("ZKB_TIMING") != nullptr;
         auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
@@ -1164,6 +1204,7 @@ struct zkb_evaluator {
             w1 = w0 + nm;
             cnt.resize(nm);
         }
+        begin_relation();
         uint64_t tv = 0, ta = 0, ti = 0, tw = 0, tg = 0, max_w0 = 0;
         for (auto& k : cnt) {
             tv += k.n_values; ta += k.n_asserts; ti += k.n_inst; tw += k.n_wit; tg += k.n_gates;
@@ -1327,10 +1368,25 @@ struct zkb_evaluator {
         return nm;
     }
 
+    // The first relation message fixes the streams: in batch mode, positions n_common .. n_common + (longest set) - 1 follow
+    // the common values in both queues.
+    void begin_relation() {
+        if (relation_seen) return;
+        relation_seen = true;
+        if (!batch()) return;
+        n_common_inst = (uint32_t)instance_values.size();
+        n_common_wit = (uint32_t)witness_values.size();
+        for (uint64_t k = 0; k < max_set_inst; k++) instance_queue.push_back(n_common_inst + (uint32_t)k);
+        for (uint64_t k = 0; k < max_set_wit; k++) witness_queue.push_back(n_common_wit + (uint32_t)k);
+    }
+
     // Evaluator::ingest_message, :213-230: errors latch, later messages are skipped
     int ingest_parsed(ir::Message& m) {
         if (fatal) return fail(ZKB_E_FATAL, err);
-        if (evaluated) return fail(ZKB_E_ARG, "evaluator already finished (get_violations was called)");
+        if (evaluated || batch_evaluated) return fail(ZKB_E_ARG, "evaluator already finished (get_violations was called)");
+        if (batch() && relation_seen && m.type != ir::MSG_RELATION)
+            return fail(ZKB_E_ARG, "with value sets, common instance / witness values must come before the first relation message");
+        if (m.type == ir::MSG_RELATION) begin_relation();
         if (has_error) return ZKB_OK;
         try {
             if (m.type == ir::MSG_RELATION) ingest_relation(m);
@@ -1339,7 +1395,18 @@ struct zkb_evaluator {
             has_error = true;
             found_error = e.msg;
             ctx_latch(c, e.msg);
+            if (batch()) {
+                global_cut = prog().n_values();
+                global_cut_msg = e.msg;
+            }
         } catch (const Fatal& f) {
+            if (batch()) {  // not an error of the call: a cut point of every set that gets this far (decided per set)
+                has_error = true;
+                global_cut = prog().n_values();
+                global_cut_msg = f.msg;
+                global_cut_fatal = true;
+                return ZKB_OK;
+            }
             if (assertion_fails_before(f)) return ZKB_OK;
             fatal = true;
             return fail(ZKB_E_FATAL, f.msg);
@@ -1366,6 +1433,68 @@ struct zkb_evaluator {
         return code;
     }
 
+    // The deferred evaluation shared by one statement and by value sets: levelize + upload the recorded program (once),
+    // pack the streams (common values, then each set's; one set of the common values alone without sets) and run them as
+    // one batch, split over the communicator of zkb_evaluator_use_devices when there are at least as many sets as contexts.
+    // t_begin >= 0: ZKB_TIMING report of the phases.
+    int run_recorded(std::vector<zkb_verdict>& v, double t_begin) {
+        Program& p = prog();
+        auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+        if (!c->finalized) {
+            c->live_values.clear();
+            values.for_each([&](uint64_t, uint32_t h) {
+                if (!is_callout(h)) c->live_values.push_back(h);  // group outputs (implicit values) are always kept
+            });
+            int rc = ctx_finalize(c, 0);
+            if (rc != ZKB_OK) return fail(rc, c->err);
+        }
+        if (t_begin >= 0) fprintf(stderr, "finish: live wires + levelize + program upload %.3f s\n", now() - t_begin);
+        const size_t S = std::max<size_t>(sets.size(), 1);
+        // one stride for every set: the widest value over all of them (raw values >= p keep their bytes, trap 1)
+        size_t stride = (size_t)p.nlimb * 4;
+        for (const auto* vals : {&instance_values, &witness_values})
+            for (const auto& x : *vals) {
+                size_t n = x.size();
+                while (n > 0 && x[n - 1] == 0) n--;
+                stride = std::max(stride, n);
+            }
+        stride = std::max(stride, std::max(set_inst.widest, set_wit.widest));
+        stride = (stride + 3) / 4 * 4;
+        // [set][position][stride]; one shared vector (set stride 0) when no set brings values of that stream
+        auto pack = [&](const std::vector<std::vector<uint8_t>>& common, const Arena& a, uint32_t need, uint64_t ValueSet::*first,
+                        uint64_t ValueSet::*count, uint64_t& set_stride) {
+            const bool per_set = a.size() > 0;
+            const size_t per = (size_t)std::max<uint32_t>(need, 1) * stride;
+            set_stride = per_set ? per : 0;
+            std::vector<uint8_t> out(per_set ? per * S : per, 0);
+            parallel_for(per_set ? S : 1, parse_threads(), [&](size_t j) {
+                uint8_t* o = out.data() + j * set_stride;
+                uint32_t k = 0;
+                for (; k < need && k < common.size(); k++) {
+                    size_t n = common[k].size();
+                    while (n > 0 && common[k][n - 1] == 0) n--;
+                    memcpy(o + (size_t)k * stride, common[k].data(), n);
+                }
+                if (!per_set) return;
+                const uint64_t v0 = sets[j].*first, nv = sets[j].*count;
+                for (uint64_t i = 0; i < nv && k < need; i++, k++)
+                    memcpy(o + (size_t)k * stride, a.bytes.data() + a.end[v0 + i], a.end[v0 + i + 1] - a.end[v0 + i]);
+            });
+            return out;
+        };
+        uint64_t iss = 0, wss = 0;
+        const std::vector<uint8_t> ib = pack(instance_values, set_inst, p.n_instance, &ValueSet::inst0, &ValueSet::n_inst, iss);
+        const std::vector<uint8_t> wb = pack(witness_values, set_wit, p.n_witness, &ValueSet::wit0, &ValueSet::n_wit, wss);
+        v.assign(S, zkb_verdict{});
+        const double t_eval = now();
+        batch_sharded = batch() && devices.size() > 1 && S >= devices.size();
+        int rc = batch_sharded ? zkb_evaluate_sharded(devices.data(), (int)devices.size(), ib.data(), iss, wb.data(), wss, (uint32_t)stride, (uint32_t)S, v.data())
+                               : zkb_evaluate(c, ib.data(), iss, wb.data(), wss, (uint32_t)stride, (uint32_t)S, v.data());
+        if (rc != ZKB_OK) return fail(rc, c->err);
+        if (t_begin >= 0) fprintf(stderr, "finish: zkb_evaluate (allocations, input upload, kernels, verdict) %.3f s\n", now() - t_eval);
+        return ZKB_OK;
+    }
+
     // The deferred evaluation: levelize + upload the recorded program (once), run it for the queued instance / witness
     // values (a batch of one), and rebuild the reference's text for the first failing assertion (:357-362).
     int evaluate_recorded(bool& have_error, std::string& first_error) {
@@ -1375,41 +1504,10 @@ struct zkb_evaluator {
         auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
         const double t_begin = now();
         if (!p.field_set || p.n_values() == 0) return ZKB_OK;
-        if (!c->finalized) {
-            c->live_values.clear();
-            values.for_each([&](uint64_t, uint32_t v) {
-                if (!is_callout(v)) c->live_values.push_back(v);  // group outputs (implicit values) are always kept
-            });
-            int rc = ctx_finalize(c, 0);
-            if (rc != ZKB_OK) return fail(rc, c->err);
-        }
-        if (timing) fprintf(stderr, "finish: live wires + levelize + program upload %.3f s\n", now() - t_begin);
-        // pack the queued streams: one statement = batch of 1
-        size_t stride = (size_t)p.nlimb * 4;
-        auto widen = [&](const std::vector<std::vector<uint8_t>>& vals) {
-            for (const auto& v : vals) {
-                size_t n = v.size();
-                while (n > 0 && v[n - 1] == 0) n--;
-                stride = std::max(stride, (n + 3) / 4 * 4);
-            }
-        };
-        widen(instance_values);
-        widen(witness_values);
-        auto pack = [&](const std::vector<std::vector<uint8_t>>& vals, uint32_t need) {
-            std::vector<uint8_t> out((size_t)std::max<uint32_t>(need, 1) * stride, 0);
-            for (uint32_t i = 0; i < need && i < vals.size(); i++) {
-                size_t n = vals[i].size();
-                while (n > 0 && vals[i][n - 1] == 0) n--;
-                memcpy(out.data() + (size_t)i * stride, vals[i].data(), n);
-            }
-            return out;
-        };
-        std::vector<uint8_t> ib = pack(instance_values, p.n_instance), wb = pack(witness_values, p.n_witness);
-        zkb_verdict v;
-        const double t_eval = now();
-        int rc = zkb_evaluate(c, ib.data(), 0, wb.data(), 0, (uint32_t)stride, 1, &v);
-        if (rc != ZKB_OK) return fail(rc, c->err);
-        if (timing) fprintf(stderr, "finish: zkb_evaluate (allocations, input upload, kernels, verdict) %.3f s\n", now() - t_eval);
+        std::vector<zkb_verdict> vs;
+        int rc = run_recorded(vs, timing ? t_begin : -1.0);
+        if (rc != ZKB_OK) return rc;
+        const zkb_verdict& v = vs[0];
         if (v.first_fail_seq != UINT64_MAX) {
             uint64_t w = p.asserts[v.first_fail_seq].src_wire;
             first_error = "Wire_" + u64s(w) + " (may be weighted) should be 0, while it is not";  // :357-362
@@ -1450,6 +1548,143 @@ struct zkb_evaluator {
         if (have_error) violations.push_back(first_error);
         evaluated = true;
         return ZKB_OK;
+    }
+
+    // ---- value sets ------------------------------------------------------------------------------------------------------
+    // One set from a concatenation of size-prefixed Instance / Witness messages (`where` names the source in errors).  The
+    // set is committed by add_value_set_end once all of its buffers have been read.
+    int add_value_set_bytes(const uint8_t* buf, size_t len, const std::string& where) {
+        std::vector<std::pair<size_t, size_t>> msgs;
+        ir::split_messages(buf, len, msgs);
+        for (size_t i = 0; i < msgs.size(); i++) {
+            ir::Message m;
+            std::string e;
+            if (!ir::read_message(buf + msgs[i].first, msgs[i].second, m, e)) return fail(ZKB_E_FORMAT, where + ": " + e);
+            if (m.type == ir::MSG_RELATION)
+                return fail(ZKB_E_ARG, where + ": a value set holds Instance and Witness messages only (message " + u64s(i) + " is a Relation)");
+            Arena& a = m.type == ir::MSG_INSTANCE ? set_inst : set_wit;
+            for (const auto& v : m.values) a.push(v);
+        }
+        return ZKB_OK;
+    }
+    int add_value_set_begin() {
+        if (fatal) return fail(ZKB_E_FATAL, err);
+        if (prog().keep_copies) return fail(ZKB_E_ARG, "value sets need an evaluating backend (not flatten / expand-definable)");
+        if (relation_seen) return fail(ZKB_E_ARG, "every value set must be added before the first relation message");
+        if (batch_evaluated || evaluated) return fail(ZKB_E_ARG, "evaluator already finished");
+        sets.push_back(ValueSet{set_inst.size(), 0, set_wit.size(), 0});
+        return ZKB_OK;
+    }
+    int add_value_set_end(int rc) {
+        ValueSet& s = sets.back();
+        if (rc == ZKB_OK) {
+            s.n_inst = set_inst.size() - s.inst0;
+            s.n_wit = set_wit.size() - s.wit0;
+            if (instance_values.size() + s.n_inst >= 0xFFFFFFF0u || witness_values.size() + s.n_wit >= 0xFFFFFFF0u)
+                rc = fail(ZKB_E_ARG, "zkb: too many input values");
+        }
+        if (rc != ZKB_OK) {  // the set is not added
+            set_inst.bytes.resize(set_inst.end[s.inst0]);
+            set_inst.end.resize(s.inst0 + 1);
+            set_wit.bytes.resize(set_wit.end[s.wit0]);
+            set_wit.end.resize(s.wit0 + 1);
+            sets.pop_back();
+            return rc;
+        }
+        max_set_inst = std::max(max_set_inst, s.n_inst);
+        max_set_wit = std::max(max_set_wit, s.n_wit);
+        return ZKB_OK;
+    }
+
+    // Handle of the first value that consumed each stream position, then the minimum over every later position: entry L is
+    // where a stream of L values is first found empty (a Switch hands its branches copies of a prefix of the queue, so a
+    // position can be skipped; any later one consumed first marks the same point).
+    std::vector<uint32_t> first_use_after(uint8_t kind, uint64_t n_pos) {
+        const Program& p = prog();
+        std::vector<uint32_t> f(n_pos + 1, UINT32_MAX);
+        for (uint32_t v = 0, n = p.n_values(); v < n; v++)
+            if (p.kind[v] == kind && p.opb[v] < n_pos && f[p.opb[v]] == UINT32_MAX) f[p.opb[v]] = v;
+        for (uint64_t k = n_pos; k-- > 0;) f[k] = std::min(f[k], f[k + 1]);
+        return f;
+    }
+    // assertions recorded before value handle h was pushed (an assertion's pos is the number of values recorded before it)
+    uint64_t seq_before(uint32_t h) {
+        const auto& a = prog().asserts;
+        return (uint64_t)(std::upper_bound(a.begin(), a.end(), h, [](uint32_t x, const AssertRec& r) { return x < r.pos; }) - a.begin());
+    }
+
+    // Cut of each set: the earliest of its instance stream found empty, its witness stream found empty, the global cut.
+    // 0 none, 1 instance, 2 witness, 3 global; the handle in set_cut.
+    std::vector<uint8_t> compute_cuts() {
+        const uint64_t ni = n_common_inst + max_set_inst, nw = n_common_wit + max_set_wit;
+        const std::vector<uint32_t> fi = first_use_after(V_INSTANCE, ni), fw = first_use_after(V_WITNESS, nw);
+        std::vector<uint8_t> what(sets.size(), 0);
+        set_cut.assign(sets.size(), UINT32_MAX);
+        for (size_t j = 0; j < sets.size(); j++) {
+            const uint32_t ci = relation_seen ? fi[n_common_inst + sets[j].n_inst] : UINT32_MAX;
+            const uint32_t cw = relation_seen ? fw[n_common_wit + sets[j].n_wit] : UINT32_MAX;
+            uint32_t cut = global_cut;
+            uint8_t w = global_cut != UINT32_MAX ? 3 : 0;
+            if (cw < cut) cut = cw, w = 2;
+            if (ci < cut) cut = ci, w = 1;
+            set_cut[j] = cut;
+            what[j] = w;
+        }
+        return what;
+    }
+
+    // Evaluates every set in one batch (once) and decides each one as finish() decides a single statement: the first failing
+    // assertion if it comes before the set's cut, else the cut's error (status OK) or panic (ZKB_E_FATAL).
+    int evaluate_batch() {
+        if (batch_evaluated) return ZKB_OK;
+        if (fatal) return fail(ZKB_E_FATAL, err);
+        Program& p = prog();
+        const size_t S = sets.size();
+        const std::vector<uint8_t> what = compute_cuts();
+        std::vector<uint64_t> first_fail(S, UINT64_MAX);
+        if (p.field_set && p.n_values() > 0) {
+            std::vector<zkb_verdict> v;
+            int rc = run_recorded(v, -1.0);
+            if (rc != ZKB_OK) return rc;
+            for (size_t j = 0; j < S; j++) first_fail[j] = v[j].first_fail_seq;
+        }
+        set_status.assign(S, ZKB_OK);
+        set_violations.assign(S, {});
+        for (size_t j = 0; j < S; j++) {
+            auto& out = set_violations[j];
+            if (!verified_at_least_one_gate) out.push_back("Did not receive any gate to verify.");
+            const uint64_t cut_seq = what[j] ? seq_before(set_cut[j]) : UINT64_MAX;
+            if (first_fail[j] != UINT64_MAX && first_fail[j] < cut_seq) {
+                out.push_back("Wire_" + u64s(p.asserts[first_fail[j]].src_wire) + " (may be weighted) should be 0, while it is not");
+            } else if (what[j] == 1) {
+                out.push_back("Not enough instance to consume");
+            } else if (what[j] == 2 || (what[j] == 3 && global_cut_fatal)) {
+                set_status[j] = ZKB_E_FATAL;
+                out.assign(1, what[j] == 2 ? std::string("Missing witness value for PlaintextBackend") : global_cut_msg);
+            } else if (what[j] == 3) {
+                out.push_back(global_cut_msg);
+            }
+        }
+        batch_evaluated = true;
+        return ZKB_OK;
+    }
+
+    // the context that evaluated set j, and j's index in its block of the batch
+    zkb_ctx* owner_of(size_t j, uint32_t& idx) {
+        if (!batch_sharded) {
+            idx = (uint32_t)j;
+            return c;
+        }
+        const uint64_t S = sets.size(), n = devices.size();
+        for (uint64_t r = 0; r < n; r++) {
+            const uint64_t lo = S * r / n, hi = S * (r + 1) / n;
+            if (j >= lo && j < hi) {
+                idx = (uint32_t)(j - lo);
+                return devices[r];
+            }
+        }
+        idx = 0;
+        return c;
     }
 };
 
@@ -1638,6 +1873,7 @@ extern "C" int zkb_debug_write_flat_relation(zkb_ctx* c, const uint8_t* modulus_
 }
 
 extern "C" int zkb_evaluator_set_flatten(zkb_evaluator* ev, int on) {
+    if (ev->batch()) return ev->fail(ZKB_E_ARG, "value sets need an evaluating backend (not flatten / expand-definable)");
     if (ev->prog().n_values() > 0) return ev->fail(ZKB_E_ARG, "flatten mode must be chosen before anything is recorded");
     ev->prog().keep_copies = on != 0;
     return ZKB_OK;
@@ -1645,6 +1881,7 @@ extern "C" int zkb_evaluator_set_flatten(zkb_evaluator* ev, int on) {
 
 // `zki_sieve expand-definable --gate-set <s>` (cli.rs:513-553): ExpandDefinable wraps the flattener
 extern "C" int zkb_evaluator_set_expand_definable(zkb_evaluator* ev, const char* gate_set) {
+    if (ev->batch()) return ev->fail(ZKB_E_ARG, "value sets need an evaluating backend (not flatten / expand-definable)");
     if (ev->prog().n_values() > 0) return ev->fail(ZKB_E_ARG, "expand-definable must be chosen before anything is recorded");
     uint16_t mask = 0;
     std::string e;
@@ -1857,6 +2094,7 @@ extern "C" int zkb_evaluator_ingest_paths(zkb_evaluator* ev, const char* const* 
 }
 
 extern "C" int zkb_evaluator_get_violations(zkb_evaluator* ev, size_t* n) {
+    if (ev->batch()) return ev->fail(ZKB_E_ARG, "the evaluator holds value sets: use zkb_evaluator_batch_result");
     int rc = ev->finish();
     if (rc != ZKB_OK) return rc;
     *n = ev->violations.size();
@@ -1868,6 +2106,7 @@ extern "C" const char* zkb_evaluator_violation(zkb_evaluator* ev, size_t i) {
 }
 
 extern "C" int zkb_evaluator_get_wire(zkb_evaluator* ev, uint64_t wire_id, uint8_t* out, size_t cap, size_t* len) {
+    if (ev->batch()) return ev->fail(ZKB_E_ARG, "the evaluator holds value sets: use zkb_evaluator_get_wire_of");
     int rc = ev->finish();
     if (rc != ZKB_OK) return rc;
     uint32_t v = ev->values.get(wire_id);
@@ -1886,5 +2125,94 @@ extern "C" int zkb_evaluator_lookup(zkb_evaluator* ev, uint64_t wire_id, zkb_wir
     uint32_t v = ev->values.get(wire_id);
     if (v == Scope::kNone) return ev->fail(ZKB_E_SEMANTIC, "No value given for wire_" + u64s(wire_id));
     *out = v;
+    return ZKB_OK;
+}
+
+// ---- value sets (batch mode) ------------------------------------------------------------------------------------------
+extern "C" int zkb_evaluator_add_value_set_buffer(zkb_evaluator* ev, const uint8_t* buf, size_t len) {
+    int rc = ev->add_value_set_begin();
+    if (rc != ZKB_OK) return rc;
+    return ev->add_value_set_end(ev->add_value_set_bytes(buf, len, "value set " + u64s(ev->sets.size() - 1)));
+}
+
+extern "C" int zkb_evaluator_add_value_set_paths(zkb_evaluator* ev, const char* const* paths, size_t n_paths) {
+    std::vector<std::string> files;
+    std::string e;
+    int rc = zkb::list_workspace_files(paths, n_paths, files, e);
+    if (rc != ZKB_OK) return ev->fail(rc, e);
+    if ((rc = ev->add_value_set_begin()) != ZKB_OK) return rc;
+    for (const auto& f : files) {
+        zkb::FileBytes data;
+        if (!data.open(f)) {
+            rc = ev->fail(ZKB_E_ARG, "cannot read " + f);
+            break;
+        }
+        if ((rc = ev->add_value_set_bytes(data.data, data.size, f)) != ZKB_OK) break;
+    }
+    return ev->add_value_set_end(rc);
+}
+
+extern "C" size_t zkb_evaluator_value_sets(zkb_evaluator* ev) { return ev->sets.size(); }
+
+extern "C" int zkb_evaluator_use_devices(zkb_evaluator* ev, zkb_ctx** ctxs, int n) {
+    if (!ctxs || n < 1 || ctxs[0] != ev->c) return ev->fail(ZKB_E_ARG, "zkb_evaluator_use_devices: ctxs[0] must be the evaluator's backend");
+    if (ev->batch_evaluated) return ev->fail(ZKB_E_ARG, "the batch has already been evaluated");
+    for (int i = 0; i < n; i++) {
+        int rank = -1, size = 0;
+        if (!ctxs[i] || zkb_comm_info(ctxs[i], &rank, &size, nullptr, nullptr) != ZKB_OK || rank != i || size != n)
+            return ev->fail(ZKB_E_ARG, "zkb_evaluator_use_devices: pass the contexts of one communicator in the order given to zkb_comm_init");
+    }
+    ev->devices.assign(ctxs, ctxs + n);
+    return ZKB_OK;
+}
+
+static int batch_ready(zkb_evaluator* ev, uint64_t set) {
+    if (!ev->batch()) return ev->fail(ZKB_E_ARG, "no value set has been added");
+    if (set >= ev->sets.size()) return ev->fail(ZKB_E_ARG, "value set index " + u64s(set) + " out of range (" + u64s(ev->sets.size()) + " sets)");
+    return ev->evaluate_batch();
+}
+
+extern "C" int zkb_evaluator_batch_result(zkb_evaluator* ev, uint64_t set, int* status, size_t* n_violations) {
+    int rc = batch_ready(ev, set);
+    if (rc != ZKB_OK) return rc;
+    if (status) *status = ev->set_status[set];
+    if (n_violations) *n_violations = ev->set_violations[set].size();
+    return ZKB_OK;
+}
+
+extern "C" const char* zkb_evaluator_batch_violation(zkb_evaluator* ev, uint64_t set, size_t i) {
+    if (!ev->batch_evaluated || set >= ev->set_violations.size() || i >= ev->set_violations[set].size()) return nullptr;
+    return ev->set_violations[set][i].c_str();
+}
+
+extern "C" int zkb_evaluator_get_wire_of(zkb_evaluator* ev, uint64_t set, uint64_t wire_id, uint8_t* out, size_t cap, size_t* len) {
+    int rc = batch_ready(ev, set);
+    if (rc != ZKB_OK) return rc;
+    if (ev->set_status[set] != ZKB_OK) return ev->fail(ev->set_status[set], ev->set_violations[set][0]);
+    // The top scope is the one the whole recording left.  A set whose streams run out earlier stops at its cut, where its
+    // own statement's scope can differ (wires freed or bound after the cut): its wires are not answered from this scope.
+    if (ev->set_cut[set] != UINT32_MAX)
+        return ev->fail(ZKB_E_ARG, "value set " + u64s(set) + " stops recording before the relation ends: wire values are read for sets recorded in full");
+    uint32_t v = ev->values.get(wire_id);
+    if (v == Scope::kNone) return ev->fail(ZKB_E_SEMANTIC, "No value given for wire_" + u64s(wire_id));
+    uint32_t idx = 0;
+    zkb_ctx* owner = ev->owner_of(set, idx);
+    zkb_wire w = v;
+    memset(out, 0, cap);
+    rc = zkb_read_values(owner, idx, &w, 1, out, cap);
+    if (rc != ZKB_OK) return ev->fail(rc, owner->err);
+    size_t n = cap;
+    while (n > 1 && out[n - 1] == 0) n--;
+    if (len) *len = n;
+    return ZKB_OK;
+}
+
+// stream cut of a value set, from the recording alone (no device): *what 0 none, 1 its instance stream runs out, 2 its witness
+// stream runs out, 3 the recording's own error or panic; *seq the assertions recorded before that point
+extern "C" int zkb_debug_value_set_cut(zkb_evaluator* ev, uint64_t set, uint64_t* seq, int* what) {
+    if (set >= ev->sets.size()) return ev->fail(ZKB_E_ARG, "value set index " + u64s(set) + " out of range (" + u64s(ev->sets.size()) + " sets)");
+    const std::vector<uint8_t> w = ev->compute_cuts();
+    *what = w[set];
+    *seq = w[set] ? ev->seq_before(ev->set_cut[set]) : UINT64_MAX;
     return ZKB_OK;
 }
