@@ -10,7 +10,10 @@ from collections import Counter
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BUILD = os.path.join(ROOT, "zkinterface-ir_b200", "build")
-KERNELS = [("kernels.cu.o", "k_level_tmaILi8"), ("kernels.cu.o", "k_level_pipeILi8ELi1"), ("kernels.cu.o", "k_level_pipeILi2ELi2"),
+# Lj0 / Lj1: the generic Montgomery product / the one for moduli whose low 64 bits are 2^64 - 2^32 + 1 (FieldParams::mul_form)
+KERNELS = [("kernels.cu.o", "k_level_tmaILi8ELj0"), ("kernels.cu.o", "k_level_tmaILi8ELj1"), ("kernels.cu.o", "k_level_pipeILi8ELi1ELj0"),
+           ("kernels.cu.o", "k_level_pipeILi8ELi1ELj1"), ("kernels.cu.o", "k_arith_groupsILi8ELj0"), ("kernels.cu.o", "k_arith_groupsILi8ELj1"),
+           ("kernels.cu.o", "k_level_pipeILi2ELi2"),
            ("kernels.cu.o", "k_levels_coopILi8ELb0"), ("kernels.cu.o", "k_levels_coopILi2ELb1"), ("kernels.cu.o", "k_levels_flowILi2"),
            ("kernels.cu.o", "k_levels_flow_wideILi8"), ("kernels.cu.o", "k_bool_levelILi4"), ("kernels.cu.o", "k_bool_groupsILi1"),
            ("kernels.cu.o", "k_bool_groupsILi4"), ("kernels.cu.o", "k_load_inputsILi8"), ("r1cs.cu.o", "k_r1cs_checkILi8"),

@@ -22,9 +22,9 @@ using namespace zkb;
 
 namespace {
 
-// op: 0 add, 1 mont_mul (product path of the kernels), 2 mont_mul portable,
+// op: 0 add, 1 mont_mul (the product of the level kernels, FORM = the field's mul_form), 2 mont_mul portable,
 //     3 lazy reduction: REDC(a b + a b + a b + b R) = 3 mont_mul(a, b) + b,  4: REDC(a R + b R) = a + b  (N = 4, 8 only)
-template <int N>
+template <int N, uint32_t FORM>
 __global__ void k_field_ops(int op, const uint32_t* a, const uint32_t* b, uint32_t* r, uint64_t n, FieldParams fp) {
     uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -35,7 +35,7 @@ __global__ void k_field_ops(int op, const uint32_t* a, const uint32_t* b, uint32
         y[k] = b[i * N + k];
     }
     if (op == 0) fe_add<N>(z, x, y, fp.p);
-    else if (op == 1) fe_mont_mul<N>(z, x, y, fp.p, fp.n0inv);
+    else if (op == 1) fe_mont_mul_form<N, FORM>(z, x, y, fp.p, fp.n0inv);
     else if (op == 2) fe_mont_mul_portable<N>(z, x, y, fp.p, fp.n0inv);
     else if constexpr (N == 4 || N == 8) {
         uint32_t T[2 * N + 1];
@@ -75,7 +75,7 @@ __global__ void k_field_ops(int op, const uint32_t* a, const uint32_t* b, uint32
 }
 
 // a chain of dependent products per thread (x <- x*y), operands in registers: no memory traffic
-template <int N>
+template <int N, uint32_t FORM>
 __global__ void __launch_bounds__(256) k_field_throughput(int op, uint32_t iters, uint32_t* sink, FieldParams fp) {
     uint32_t x[N], y[N];
 #pragma unroll
@@ -86,7 +86,7 @@ __global__ void __launch_bounds__(256) k_field_throughput(int op, uint32_t iters
     for (uint32_t i = 0; i < iters; i++) {
         uint32_t z[N];
         if (op == 0) fe_add<N>(z, x, y, fp.p);
-        else fe_mont_mul<N>(z, x, y, fp.p, fp.n0inv);
+        else fe_mont_mul_form<N, FORM>(z, x, y, fp.p, fp.n0inv);
 #pragma unroll
         for (int k = 0; k < N; k++) x[k] = z[k];
     }
@@ -123,12 +123,20 @@ __global__ void __launch_bounds__(256) k_gather_throughput(const uint4* __restri
 
 }  // namespace
 
-#define DISPATCH_N(nlimb, CALL)                        \
-    switch (nlimb) {                                   \
-        case 1: { constexpr int N = 1; CALL; } break;  \
-        case 2: { constexpr int N = 2; CALL; } break;  \
-        case 4: { constexpr int N = 4; CALL; } break;  \
-        default: { constexpr int N = 8; CALL; } break; \
+// N and the product's form (FieldParams::mul_form), as launch_level chooses them
+#define DISPATCH_N(fp, CALL)                                                                                   \
+    if ((fp).nlimb == 8 && (fp).mul_form == kMulFormLow64) {                                                   \
+        constexpr int N = 8;                                                                                   \
+        constexpr uint32_t FORM = kMulFormLow64;                                                               \
+        CALL;                                                                                                  \
+    } else {                                                                                                   \
+        constexpr uint32_t FORM = kMulFormGeneric;                                                             \
+        switch ((fp).nlimb) {                                                                                  \
+            case 1: { constexpr int N = 1; CALL; } break;                                                      \
+            case 2: { constexpr int N = 2; CALL; } break;                                                      \
+            case 4: { constexpr int N = 4; CALL; } break;                                                      \
+            default: { constexpr int N = 8; CALL; } break;                                                     \
+        }                                                                                                      \
     }
 
 extern "C" int zkb_debug_field_ops(zkb_ctx* c, int op, const uint32_t* a, const uint32_t* b, uint32_t* r, uint64_t n) {
@@ -144,7 +152,7 @@ extern "C" int zkb_debug_field_ops(zkb_ctx* c, int op, const uint32_t* a, const 
     CUDA_TRY(c, cudaMemcpyAsync(da, a, bytes, cudaMemcpyHostToDevice, c->stream));
     CUDA_TRY(c, cudaMemcpyAsync(db, b, bytes, cudaMemcpyHostToDevice, c->stream));
     const FieldParams fp = c->prog.fp;
-    DISPATCH_N(N, (k_field_ops<N><<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(op, da, db, dr, n, fp)));
+    DISPATCH_N(fp, (k_field_ops<N, FORM><<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(op, da, db, dr, n, fp)));
     CUDA_TRY(c, cudaMemcpyAsync(r, dr, bytes, cudaMemcpyDeviceToHost, c->stream));
     CUDA_TRY(c, cudaStreamSynchronize(c->stream));
     cudaFree(da);
@@ -157,7 +165,6 @@ extern "C" int zkb_debug_field_throughput(zkb_ctx* c, int op, uint32_t iters, do
     if (!c->prog.field_set || c->prog.binary) return c->fail(ZKB_E_ARG, "set an odd field first");
     if (!c->has_gpu) return c->fail(ZKB_E_CUDA, "no CUDA device in this context (there is no CPU fallback)");
     CUDA_TRY(c, cudaSetDevice(c->device));
-    const int N = c->prog.nlimb;
     const FieldParams fp = c->prog.fp;
     uint32_t* sink = nullptr;
     CUDA_TRY(c, cudaMalloc((void**)&sink, 4));
@@ -165,7 +172,7 @@ extern "C" int zkb_debug_field_throughput(zkb_ctx* c, int op, uint32_t iters, do
     float best = 1e30f;
     for (int rep = 0; rep < 4; rep++) {
         CUDA_TRY(c, cudaEventRecord(c->ev[0], c->stream));
-        DISPATCH_N(N, (k_field_throughput<N><<<grid, 256, 0, c->stream>>>(op, iters, sink, fp)));
+        DISPATCH_N(fp, (k_field_throughput<N, FORM><<<grid, 256, 0, c->stream>>>(op, iters, sink, fp)));
         CUDA_TRY(c, cudaEventRecord(c->ev[1], c->stream));
         CUDA_TRY(c, cudaStreamSynchronize(c->stream));
         float ms = 0;

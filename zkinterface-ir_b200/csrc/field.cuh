@@ -32,7 +32,13 @@ struct FieldParams {
     uint32_t n0inv;            // -p^{-1} mod 2^32
     uint32_t nlimb;            // 1, 2, 4 or 8
     uint32_t top_mask;         // mask of the bits of limb N-1 that can be set in a value < 2^bitlen(p)
-    uint32_t reserved;
+    uint32_t mul_form;         // kMulForm*: which Montgomery product the hot kernels may run for this modulus
+};
+
+// FieldParams::mul_form (Program::set_field)
+enum : uint32_t {
+    kMulFormGeneric = 0,  // any odd p
+    kMulFormLow64 = 1,    // 8 limbs and p = 2^64 - 2^32 + 1 mod 2^64 (BLS12-381 Fr): field_ptx.cuh fe_mont_mul_low64
 };
 
 template <int N>
@@ -114,6 +120,10 @@ ZKB_HD void fe_mont_mul_portable(uint32_t* r, const uint32_t* a, const uint32_t*
 #if !(defined(__CUDA_ARCH__) && !defined(ZKB_NO_PTX_FIELD))
 template <int N>
 ZKB_HD void fe_mont_mul(uint32_t* r, const uint32_t* a, const uint32_t* b, const uint32_t* p, uint32_t n0inv) {
+    fe_mont_mul_portable<N>(r, a, b, p, n0inv);
+}
+template <int N, uint32_t FORM>
+ZKB_HD void fe_mont_mul_form(uint32_t* r, const uint32_t* a, const uint32_t* b, const uint32_t* p, uint32_t n0inv) {
     fe_mont_mul_portable<N>(r, a, b, p, n0inv);
 }
 template <int N>

@@ -104,6 +104,52 @@ __device__ __forceinline__ uint32_t mad_chain4_cbot(uint32_t* acc, uint32_t x0, 
     return c;
 }
 
+// The reduction chains of fe_mont_mul_low64 (p mod 2^64 = 2^64 - 2^32 + 1, m = -acc[0] mod 2^32): the bottom pair's product
+// is not multiplied.
+// even: acc pairs += (0 : m) + x1 * y << 64 + x2 * y << 128 + x3 * y << 192 with p0 = 1, i.e. the bottom pair gets m.  acc[0] + m
+// = 0 mod 2^32 carries exactly when acc[0] != 0; acc[0] itself (which would become 0) is left as it is: the shift drops it.
+// Returns cin + the carry out of the top pair.
+__device__ __forceinline__ uint32_t mad_chain4_low_even(uint32_t* acc, uint32_t x1, uint32_t x2, uint32_t x3, uint32_t y, uint32_t cin) {
+    uint32_t c, t;
+    asm("add.cc.u32 %8, %9, 0xFFFFFFFF;\n\t"
+        "addc.cc.u32 %0, %0, 0;\n\t"
+        "madc.lo.cc.u32 %1, %10, %13, %1;\n\t"
+        "madc.hi.cc.u32 %2, %10, %13, %2;\n\t"
+        "madc.lo.cc.u32 %3, %11, %13, %3;\n\t"
+        "madc.hi.cc.u32 %4, %11, %13, %4;\n\t"
+        "madc.lo.cc.u32 %5, %12, %13, %5;\n\t"
+        "madc.hi.cc.u32 %6, %12, %13, %6;\n\t"
+        "addc.u32 %7, %14, 0;"
+        : ZKB_ACC(acc[1]), ZKB_ACC(acc[2]), ZKB_ACC(acc[3]), ZKB_ACC(acc[4]), ZKB_ACC(acc[5]), ZKB_ACC(acc[6]), ZKB_ACC(acc[7]), "=r"(c), "=r"(t)
+        : "r"(acc[0]), "r"(x1), "r"(x2), "r"(x3), "r"(y), "r"(cin));
+    return c;
+}
+// odd: acc pairs += (hi : lo) + x1 * y << 64 + x2 * y << 128 + x3 * y << 192, where (hi : lo) = p1 * m = m 2^32 - m as a
+// 64-bit pair (p1 = 2^32 - 1): lo = -m = the row's T0, hi = m - [m != 0].  Returns cin + the carry out of the top pair.
+__device__ __forceinline__ uint32_t mad_chain4_low_odd(uint32_t* acc, uint32_t lo, uint32_t hi, uint32_t x1, uint32_t x2, uint32_t x3,
+                                                       uint32_t y, uint32_t cin) {
+    uint32_t c;
+    asm("add.cc.u32 %0, %0, %9;\n\t"
+        "addc.cc.u32 %1, %1, %10;\n\t"
+        "madc.lo.cc.u32 %2, %11, %14, %2;\n\t"
+        "madc.hi.cc.u32 %3, %11, %14, %3;\n\t"
+        "madc.lo.cc.u32 %4, %12, %14, %4;\n\t"
+        "madc.hi.cc.u32 %5, %12, %14, %5;\n\t"
+        "madc.lo.cc.u32 %6, %13, %14, %6;\n\t"
+        "madc.hi.cc.u32 %7, %13, %14, %7;\n\t"
+        "addc.u32 %8, %15, 0;"
+        : ZKB_ACC(acc[0]), ZKB_ACC(acc[1]), ZKB_ACC(acc[2]), ZKB_ACC(acc[3]), ZKB_ACC(acc[4]), ZKB_ACC(acc[5]), ZKB_ACC(acc[6]), ZKB_ACC(acc[7]), "=r"(c)
+        : "r"(lo), "r"(hi), "r"(x1), "r"(x2), "r"(x3), "r"(y), "r"(cin));
+    return c;
+}
+// m = -t0 mod 2^32 (the row's multiplier when n0inv = 2^32 - 1) and mh = m - [m != 0]: sub.cc borrows exactly when t0 != 0
+__device__ __forceinline__ void low64_m(uint32_t& m, uint32_t& mh, uint32_t t0) {
+    asm("sub.cc.u32 %0, 0, %2;\n\t"
+        "subc.u32 %1, %0, 0;"
+        : "=r"(m), "=r"(mh)
+        : "r"(t0));
+}
+
 // ---- N = 4: two pairs per chain --------------------------------------------------------------
 __device__ __forceinline__ uint32_t mad_chain2_cbot(uint32_t* acc, uint32_t x0, uint32_t x1, uint32_t y, uint32_t cbot) {
     uint32_t c, t;
@@ -340,6 +386,47 @@ __device__ __forceinline__ void fe_mont_mul_chain(uint32_t* r, const uint32_t* a
     fe_cond_sub_p<N>(r, t, top, p);
 }
 
+// fe_mont_mul_chain<8> for a modulus whose low 64 bits are 2^64 - 2^32 + 1 (p0 = 1, p1 = 2^32 - 1: BLS12-381 Fr), so that
+// n0inv = 2^32 - 1.  A row's multiplier is m = -T0 mod 2^32 (no multiply), p0 * m = m and p1 * m = (m - [m != 0] : T0): the
+// reduction of a row takes 6 wide products instead of 8, a product 112 multiplies instead of 136.  Every chain adds the
+// same integers as in fe_mont_mul_chain<8>, so T + m p, the carries and the result are bit for bit the same for every input
+// that product accepts (a b < p R).
+__device__ __forceinline__ void fe_mont_mul_low64(uint32_t* r, const uint32_t* a, const uint32_t* b, const uint32_t* p) {
+    using Ch = PtxChains<8>;
+    uint32_t E[8], O[8], m, mh;
+    Ch::mul_even(E, a, b[0]);
+    Ch::mul_odd(O, a, b[0]);
+    low64_m(m, mh, E[0]);
+    uint32_t cO = mad_chain4_low_odd(O, E[0], mh, p[3], p[5], p[7], m, 0);
+    uint32_t cE = mad_chain4_low_even(E, p[2], p[4], p[6], m, 0);
+#pragma unroll
+    for (int i = 1; i < 8; i++) {
+        uint32_t nE[8], nO[8];
+#pragma unroll
+        for (int j = 1; j < 8; j++) nE[j] = O[j];
+#pragma unroll
+        for (int j = 0; j < 6; j++) nO[j] = E[j + 2];
+        nO[6] = cE;
+        nO[7] = cO;
+        cO = Ch::mad_odd_fold(nE[0], O[0], E[1], nO, a, b[i]);
+        cE = Ch::mad_even(nE, a, b[i]);
+        low64_m(m, mh, nE[0]);
+        cO = mad_chain4_low_odd(nO, nE[0], mh, p[3], p[5], p[7], m, cO);
+        cE = mad_chain4_low_even(nE, p[2], p[4], p[6], m, cE);
+#pragma unroll
+        for (int j = 0; j < 8; j++) {
+            E[j] = nE[j];
+            O[j] = nO[j];
+        }
+    }
+    uint32_t t[8], up[8];
+#pragma unroll
+    for (int j = 0; j < 7; j++) up[j] = E[j + 1];
+    up[7] = cE;
+    const uint32_t top = add_chain8(t, up, O) + cO;
+    cond_sub_chain8(r, t, top, p);
+}
+
 // ---- lazy reduction (the R1CS check: one Montgomery reduction per linear combination instead of one per term) --------
 // A linear combination sum_k coef_k * z_k of Montgomery residues is accumulated as the plain integer
 //     T = sum_k (z_k R)(coef_k R)  +  sum over coefficient-one terms of (z_k R) * R            (R = 2^(32N)),
@@ -515,6 +602,14 @@ __device__ __forceinline__ void fe_mont_mul(uint32_t* r, const uint32_t* a, cons
     else if constexpr (N == 2) fe_mont_mul_u64(r, a, b, p, n0inv);
 #endif
     else fe_mont_mul_portable<N>(r, a, b, p, n0inv);
+}
+
+// the hot kernels' product: FORM is the modulus's FieldParams::mul_form, a template parameter chosen at launch (a branch on
+// it inside the kernel would hold both products' registers)
+template <int N, uint32_t FORM>
+__device__ __forceinline__ void fe_mont_mul_form(uint32_t* r, const uint32_t* a, const uint32_t* b, const uint32_t* p, uint32_t n0inv) {
+    if constexpr (N == 8 && FORM == kMulFormLow64) fe_mont_mul_low64(r, a, b, p);
+    else fe_mont_mul<N>(r, a, b, p, n0inv);
 }
 
 }  // namespace zkb

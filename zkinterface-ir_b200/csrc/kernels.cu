@@ -252,7 +252,7 @@ __device__ __forceinline__ void load_operands(uint32_t* a, uint32_t* b, const ui
 #ifndef ZKB_LEVEL_PIPE_MIN_CTAS
 #define ZKB_LEVEL_PIPE_MIN_CTAS 4  // 64 registers: 4 resident CTAs per SM measured 6 % faster than 3 (scripts/ab_min_ctas.sh)
 #endif
-template <int N, int LPT>
+template <int N, int LPT, uint32_t FORM = kMulFormGeneric>
 __global__ void __launch_bounds__(256, ZKB_LEVEL_PIPE_MIN_CTAS)
 k_level_pipe(const GateOp* __restrict__ ops, const uint32_t* __restrict__ aseq, uint64_t n_ops, uint32_t* __restrict__ store,
              const uint32_t* __restrict__ consts_mont, uint32_t* __restrict__ first_fail, TileGeom g, FieldParams fp) {
@@ -283,7 +283,7 @@ k_level_pipe(const GateOp* __restrict__ ops, const uint32_t* __restrict__ aseq, 
 #pragma unroll
         for (int l = 0; l < LPT; l++) {
             if (opc == D_ADD || opc == D_ADDC) fe_add<N>(r + l * N, a0 + l * N, b0 + l * N, fp.p);
-            else fe_mont_mul<N>(r + l * N, a0 + l * N, b0 + l * N, fp.p, fp.n0inv);
+            else fe_mont_mul_form<N, FORM>(r + l * N, a0 + l * N, b0 + l * N, fp.p, fp.n0inv);
         }
         if (!(d0.w & (F_NOSTORE | g.skip_mask))) store_elem<PN>(store, d0.z, plane, log2_pwt, r);
         if (d0.w & F_ASSERT) {
@@ -359,7 +359,7 @@ __device__ __forceinline__ uint4 lds128(uint32_t a) {
 
 constexpr size_t kTmaSmemBytes = (size_t)ZKB_TMA_STAGES * 16384;
 
-template <int N>
+template <int N, uint32_t FORM>
 __global__ void __launch_bounds__(256, ZKB_TMA_MIN_CTAS)
 k_level_tma(const GateOp* __restrict__ ops, const uint32_t* __restrict__ aseq, uint64_t n_ops, uint32_t* __restrict__ store,
             const uint32_t* __restrict__ consts_mont, uint32_t* __restrict__ first_fail, TileGeom g, FieldParams fp) {
@@ -439,7 +439,7 @@ k_level_tma(const GateOp* __restrict__ ops, const uint32_t* __restrict__ aseq, u
             }
         }
         if (opc == D_ADD || opc == D_ADDC) fe_add<N>(r, a, b, fp.p);
-        else fe_mont_mul<N>(r, a, b, fp.p, fp.n0inv);
+        else fe_mont_mul_form<N, FORM>(r, a, b, fp.p, fp.n0inv);
         if (!(d0.w & (F_NOSTORE | g.skip_mask))) store_elem<N>(store, d0.z, lane, g.log2_wt, r);
         if (d0.w & F_ASSERT) {
             const uint32_t seq = __ldg(aseq + (gi >> log2_q));
@@ -1000,7 +1000,7 @@ k_bool_groups(const GroupDesc* __restrict__ descs, uint32_t n_groups, uint64_t t
 // const table), the previous op's result stays in registers (GroupOp::fwd), an AssertZero tests its register in place and
 // reports seq0 + call * A + k, and only the outputs go back to the wire store (always stored: a group output is a level-0
 // value).  thread -> group as in k_bool_groups.
-template <int N>
+template <int N, uint32_t FORM>
 __global__ void __launch_bounds__(kGroupThreads)
 k_arith_groups(const GroupDesc* __restrict__ descs, uint32_t n_groups, uint64_t total_calls, const GroupOp* __restrict__ gops,
                const uint32_t* __restrict__ tables, const uint32_t* __restrict__ hints, uint32_t* __restrict__ store,
@@ -1073,7 +1073,7 @@ k_arith_groups(const GroupDesc* __restrict__ descs, uint32_t n_groups, uint64_t 
                 ld_reg(y, o.z);
             }
             if (m.x == AG_ADD || m.x == AG_ADDC) fe_add<N>(r, x, y, fp.p);
-            else fe_mont_mul<N>(r, x, y, fp.p, fp.n0inv);
+            else fe_mont_mul_form<N, FORM>(r, x, y, fp.p, fp.n0inv);
             st_reg(o.x, r);
         }
         const uint32_t out0 = h1.y + call * h0.z;
@@ -1282,14 +1282,21 @@ void launch_level(int nlimb, const GateOp* ops, const uint32_t* aseq, uint64_t n
                 static int tma_per_sm = 0;
                 static std::atomic<uint64_t> tma_attr_seen{0};
                 constexpr size_t smem = kTmaSmemBytes;
-                if (first_on_device(tma_attr_seen))
-                    cudaFuncSetAttribute(k_level_tma<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                if (first_on_device(tma_attr_seen)) {
+                    cudaFuncSetAttribute(k_level_tma<8, kMulFormGeneric>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                    cudaFuncSetAttribute(k_level_tma<8, kMulFormLow64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+                }
                 if (!tma_per_sm) {
                     const char* e = getenv("ZKB_TMA_GRID_PER_SM");
                     tma_per_sm = e ? std::max(1, atoi(e)) : 128;
                 }
                 grid = grid_for(n_ops << g.log2_wt, sm_count, tma_per_sm);
-                k_level_tma<8><<<grid, 256, smem, s>>>(ops, aseq, n_ops, store, consts_mont, first_fail, g, fp);
+                if (fp.mul_form == kMulFormLow64)
+                    k_level_tma<8, kMulFormLow64><<<grid, 256, smem, s>>>(ops, aseq, n_ops, store, consts_mont, first_fail, g, fp);
+                else
+                    k_level_tma<8, kMulFormGeneric><<<grid, 256, smem, s>>>(ops, aseq, n_ops, store, consts_mont, first_fail, g, fp);
+            } else if (nlimb == 8 && fp.mul_form == kMulFormLow64) {
+                k_level_pipe<8, 1, kMulFormLow64><<<grid, 256, 0, s>>>(ops, aseq, n_ops, store, consts_mont, first_fail, g, fp);
             } else {
                 ZKB_DISPATCH_N(nlimb, (k_level_pipe<N, 1><<<grid, 256, 0, s>>>(ops, aseq, n_ops, store, consts_mont, first_fail, g, fp)));
             }
@@ -1549,24 +1556,28 @@ uint32_t arith_group_threads(int nlimb, uint32_t n_regs) {
     while (t > 32 && (size_t)n_regs * nlimb * 4 * t > kArithGroupSmemPerCta) t >>= 1;
     return t;
 }
-template <int N>
+template <int N, uint32_t FORM>
 static void launch_arith_groups_n(const GroupDesc* descs, uint32_t n_groups, uint64_t total_calls, const GroupOp* gops, const uint32_t* tables,
                                   const uint32_t* hints, uint32_t* store, const uint32_t* consts_mont, uint32_t* first_fail, TileGeom g,
                                   const FieldParams& fp, uint32_t n_regs, int sm_count, cudaStream_t s) {
     static std::atomic<uint64_t> attr_seen{0};
-    if (first_on_device(attr_seen)) cudaFuncSetAttribute(k_arith_groups<N>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kArithGroupSmemPerCta);
+    if (first_on_device(attr_seen)) cudaFuncSetAttribute(k_arith_groups<N, FORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kArithGroupSmemPerCta);
     const uint32_t T = arith_group_threads(N, n_regs);
     const size_t smem = (size_t)std::max<uint32_t>(n_regs, 1) * N * 4 * T;
     const uint64_t blocks = ((total_calls << g.log2_wt) + T - 1) / T;
     const unsigned grid = (unsigned)std::min<uint64_t>(blocks, (uint64_t)sm_count * (2048 / T));
-    k_arith_groups<N><<<grid, T, smem, s>>>(descs, n_groups, total_calls, gops, tables, hints, store, consts_mont, first_fail, g, fp);
+    k_arith_groups<N, FORM><<<grid, T, smem, s>>>(descs, n_groups, total_calls, gops, tables, hints, store, consts_mont, first_fail, g, fp);
 }
 void launch_arith_groups(int nlimb, const GroupDesc* descs, uint32_t n_groups, uint64_t total_calls, const GroupOp* gops, const uint32_t* tables,
                          const uint32_t* hints, uint32_t* store, const uint32_t* consts_mont, uint32_t* first_fail, TileGeom g,
                          const FieldParams& fp, uint32_t n_regs, int sm_count, cudaStream_t s) {
     if (n_groups == 0 || total_calls == 0) return;
-    ZKB_DISPATCH_N(nlimb, (launch_arith_groups_n<N>(descs, n_groups, total_calls, gops, tables, hints, store, consts_mont, first_fail, g, fp,
-                                                    n_regs, sm_count, s)));
+    if (nlimb == 8 && fp.mul_form == kMulFormLow64)
+        launch_arith_groups_n<8, kMulFormLow64>(descs, n_groups, total_calls, gops, tables, hints, store, consts_mont, first_fail, g, fp, n_regs,
+                                                sm_count, s);
+    else
+        ZKB_DISPATCH_N(nlimb, (launch_arith_groups_n<N, kMulFormGeneric>(descs, n_groups, total_calls, gops, tables, hints, store, consts_mont,
+                                                                         first_fail, g, fp, n_regs, sm_count, s)));
 }
 
 void launch_bool_read_values(const uint32_t* slots, uint32_t n, const uint32_t* store, uint32_t lane, uint32_t log2_wt,

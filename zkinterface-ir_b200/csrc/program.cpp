@@ -59,6 +59,7 @@ bool Program::set_field(const uint8_t* mod_le, size_t len, uint32_t degree, std:
         uint32_t p0 = fp.p[0], inv = 1;
         for (int i = 0; i < 5; i++) inv *= 2 - p0 * inv;
         fp.n0inv = (uint32_t)(0u - inv);
+        fp.mul_form = (nlimb == 8 && fp.p[0] == 1u && fp.p[1] == 0xFFFFFFFFu) ? kMulFormLow64 : kMulFormGeneric;
         BigU R;
         R.w.assign((size_t)nlimb + 1, 0);
         R.w[nlimb] = 1;
