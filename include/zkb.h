@@ -197,10 +197,11 @@ typedef struct {
     uint32_t binary;        /* p == 2 */
     uint32_t tile_witnesses;/* witnesses resident per pass (after upload) */
     uint32_t n_tiles;
-    uint64_t n_call_groups; /* For loops over a plain function kept as ONE loop-structured descriptor each
-                             * (evaluator.rs:495-559 + :441-471; over a prime field: loops of >= 1024 calls whose body
-                             * holds Constant / Add / Mul / AddConstant / MulConstant and AssertZero on computed wires):
-                             * the device expands them, only the calls' outputs are SSA values (kind 11 in zkb_get_program) */
+    uint64_t n_call_groups; /* For loops over a plain function or an anonymous body of plain gates kept as ONE
+                             * loop-structured descriptor each (evaluator.rs:495-559 + :441-471; over a prime field: loops of
+                             * >= 1024 calls whose body holds Constant / Add / Mul / AddConstant / MulConstant and AssertZero
+                             * on computed wires, carried loops included): the device expands them, only the calls' outputs
+                             * are SSA values (kind 11 in zkb_get_program) */
     uint64_t n_group_calls; /* function calls those groups stand for */
     uint64_t n_group_launches;     /* after finalize: kernel launches that expand them (one per dependency depth) */
     uint64_t n_group_table_slots;  /* after finalize: operand slots listed explicitly (inputs whose slots are not an
@@ -210,6 +211,11 @@ typedef struct {
                                     * and in use */
     uint64_t n_sink_ops;           /* after finalize: stored results that no gate reads (only a read-back needs them; tiles
                                     * other than the last one run skip their stores) */
+    uint64_t n_carried_groups;     /* of n_call_groups, the carried loops (prime fields): call c reads output k of call c - d,
+                                    * 1 <= d <= 4 (over fields of at most 64 bits: loops of >= 2^20 calls), and calls c < d read seeds that are
+                                    * instance / witness / constant values or
+                                    * outputs of earlier groups.  Each runs as a chain, one thread per witness walking the calls
+                                    * in order; they count in n_group_calls and n_group_launches too */
 } zkb_stats;
 int zkb_get_stats(zkb_ctx* ctx, zkb_stats* out);
 

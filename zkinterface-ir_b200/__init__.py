@@ -52,7 +52,7 @@ class ZkbStats(C.Structure):
                 ("binary", C.c_uint32), ("tile_witnesses", C.c_uint32), ("n_tiles", C.c_uint32),
                 ("n_call_groups", C.c_uint64), ("n_group_calls", C.c_uint64),
                 ("n_group_launches", C.c_uint64), ("n_group_table_slots", C.c_uint64), ("group_jit_state", C.c_int64),
-                ("n_sink_ops", C.c_uint64)]
+                ("n_sink_ops", C.c_uint64), ("n_carried_groups", C.c_uint64)]
 
 
 class ZkbTiming(C.Structure):

@@ -66,6 +66,8 @@ int ctx_upload_groups(zkb_ctx* c) {
     if ((rc = upload_vec(c, c->d_group_ops, c->plan.group_ops)) != ZKB_OK) return rc;
     if ((rc = upload_vec(c, c->d_group_tables, c->plan.group_tables)) != ZKB_OK) return rc;
     if ((rc = upload_vec(c, c->d_group_hints, c->plan.group_hints)) != ZKB_OK) return rc;
+    if ((rc = upload_vec(c, c->d_chain_descs, c->plan.chain_descs)) != ZKB_OK) return rc;
+    if ((rc = upload_vec(c, c->d_chain_carry, c->plan.chain_carry)) != ZKB_OK) return rc;
     group_jit_start(c);  // the templates as straight-line code, compiled in the background (group_jit.cpp)
     return ZKB_OK;
 }
@@ -182,6 +184,8 @@ extern "C" void zkb_destroy(zkb_ctx* c) {
         cudaFree(c->d_group_ops);
         cudaFree(c->d_group_tables);
         cudaFree(c->d_group_hints);
+        cudaFree(c->d_chain_descs);
+        cudaFree(c->d_chain_carry);
         if (c->h_res) cudaFreeHost(c->h_res);
         cudaFree(c->d_const_flags);
         cudaFree(c->d_const_raw);
@@ -745,6 +749,14 @@ static void run_tile(zkb_ctx* c, uint32_t tile, bool full, uint32_t* d_fail, uin
     // call groups: one launch per dependency depth, before the first wavefront (their outputs are level-0 values)
     for (size_t d = 0; d + 1 < pl.depth_off.size(); d++) {
         const uint32_t lo = pl.depth_off[d], hi = pl.depth_off[d + 1];
+        if (!pl.chain_off.empty() && pl.chain_off[d + 1] > pl.chain_off[d]) {  // carried loops of this depth: a launch of their own
+            const uint32_t c0 = pl.chain_off[d];
+            launch_arith_chain(p.nlimb, c->d_chain_descs + c0, c->d_chain_carry + (size_t)c0 * kMaxGroupInputs, pl.chain_off[d + 1] - c0,
+                               c->d_group_ops, c->d_group_tables, c->d_store, c->d_consts, d_fail, g, p.fp, pl.chain_regs, c->sm_count,
+                               c->stream);
+            (*launches)++;
+            if (level_launches) (*level_launches)++;
+        }
         if (hi == lo) continue;
         const uint64_t calls = (uint64_t)pl.group_descs[hi - 1].first_call + pl.group_descs[hi - 1].n_calls;
         if (!p.binary)
@@ -1319,6 +1331,10 @@ extern "C" int zkb_debug_plan_hash(zkb_ctx* c, uint64_t* out) {
     mix(pl.group_ops.data(), pl.group_ops.size() * sizeof(GroupOp));
     mix(pl.group_hints.data(), pl.group_hints.size() * 4);
     mix(pl.group_tables.data(), pl.group_tables.size() * 4);
+    mix(pl.chain_descs.data(), pl.chain_descs.size() * sizeof(GroupDesc));
+    mix(pl.chain_carry.data(), pl.chain_carry.size() * 4);
+    mix(pl.chain_off.data(), pl.chain_off.size() * 4);
+    mix(&pl.chain_regs, 4);
     mix(&pl.callout_slot0, 4);
     mix(&pl.n_callouts, 4);
     mix(&pl.n_slots, 4);
@@ -1347,12 +1363,21 @@ extern "C" int zkb_get_stats(zkb_ctx* c, zkb_stats* s) {
         s->algo_bytes_per_witness = c->plan.algo_bytes_per_witness;
         s->n_sink_ops = c->plan.n_sink_ops;
     }
-    s->n_call_groups = c->plan.group_descs.empty() ? p.groups.size() : c->plan.group_descs.size();
-    for (const auto& g : p.groups) s->n_group_calls += g.n_calls;
-    if (p.groups.empty())
-        for (const auto& g : c->plan.group_descs) s->n_group_calls += g.n_calls;  // replica: only the plan came over
+    const Plan& pl = c->plan;
+    const bool replica_groups = p.groups.empty();  // replica: only the plan came over
+    s->n_call_groups = replica_groups ? pl.group_descs.size() + pl.chain_descs.size() : p.groups.size();
+    for (const auto& g : p.groups) {
+        s->n_group_calls += g.n_calls;
+        s->n_carried_groups += g.carried();
+    }
+    if (replica_groups) {
+        for (const auto& g : pl.group_descs) s->n_group_calls += g.n_calls;
+        for (const auto& g : pl.chain_descs) s->n_group_calls += g.n_calls;
+        s->n_carried_groups = pl.chain_descs.size();
+    }
     if (c->finalized) {
-        for (size_t d = 0; d + 1 < c->plan.depth_off.size(); d++) s->n_group_launches += c->plan.depth_off[d + 1] > c->plan.depth_off[d];
+        for (size_t d = 0; d + 1 < pl.depth_off.size(); d++)
+            s->n_group_launches += (pl.depth_off[d + 1] > pl.depth_off[d]) + (pl.chain_off[d + 1] > pl.chain_off[d]);
         s->n_group_table_slots = c->plan.group_tables.size();
     }
     s->group_jit_state = (int64_t)group_jit_state(c);

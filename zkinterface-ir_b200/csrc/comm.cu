@@ -224,6 +224,7 @@ struct ReplicaHeader {
     uint64_t n_dev_ops[D_OPS];
     uint64_t modulus_len, pending_len, const_raw_bytes;
     uint64_t n_group_descs, n_group_ops, n_group_tables, n_depth_off, group_regs, callout_slot0, n_callouts, n_group_hints;  // call groups (program.h)
+    uint64_t n_chain_descs, chain_regs;  // carried loops (Plan::chain_descs)
     uint32_t n_slots, max_level_ops, n_instance, n_witness;
     uint32_t nlimb, binary, is_boolean, has_pending, keep_all, const_raw_stride, has_const_flags, pad;
     FieldParams fp;
@@ -333,6 +334,11 @@ static int broadcast_program(zkb_ctx* c, int root) {
         put(blob, pl.depth_off.data(), pl.depth_off.size());
         put(blob, pl.group_hints.data(), pl.group_hints.size());
         put(blob, pl.hint_off.data(), pl.hint_off.size());
+        h.n_chain_descs = pl.chain_descs.size();
+        h.chain_regs = pl.chain_regs;
+        put(blob, pl.chain_descs.data(), pl.chain_descs.size());
+        put(blob, pl.chain_carry.data(), pl.chain_carry.size());
+        put(blob, pl.chain_off.data(), pl.chain_off.size());
         h.blob_bytes = blob.size();
     }
     // 1. the fixed-size header
@@ -387,6 +393,10 @@ static int broadcast_program(zkb_ctx* c, int root) {
         get(cur, pl.depth_off, h.n_depth_off);
         get(cur, pl.group_hints, h.n_group_hints);
         get(cur, pl.hint_off, h.n_depth_off);
+        get(cur, pl.chain_descs, h.n_chain_descs);
+        get(cur, pl.chain_carry, h.n_chain_descs * kMaxGroupInputs);
+        get(cur, pl.chain_off, h.n_depth_off);
+        pl.chain_regs = (uint32_t)h.chain_regs;
         pl.group_regs = (uint32_t)h.group_regs;
         pl.callout_slot0 = (uint32_t)h.callout_slot0;
         pl.n_callouts = (uint32_t)h.n_callouts;

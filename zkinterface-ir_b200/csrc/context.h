@@ -165,6 +165,8 @@ struct zkb_ctx {
     zkb::GroupOp* d_group_ops = nullptr;
     uint32_t* d_group_tables = nullptr;
     uint32_t* d_group_hints = nullptr;
+    zkb::GroupDesc* d_chain_descs = nullptr;  // carried loops (Plan::chain_descs / chain_carry)
+    uint32_t* d_chain_carry = nullptr;
     uint8_t* d_const_flags = nullptr;   // per constant: raw value >= p
     uint8_t* d_const_raw = nullptr;     // raw bytes of the constants (const_raw_stride each), when a bitwise gate may need them
     uint32_t const_raw_stride = 0;

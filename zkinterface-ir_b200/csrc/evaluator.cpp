@@ -16,6 +16,8 @@
 #include <chrono>
 #include <deque>
 #include <thread>
+#include <map>
+#include <tuple>
 #include <unordered_map>
 
 #include "context.h"
@@ -614,16 +616,54 @@ struct zkb_evaluator {
         return true;
     }
 
+    // The body of an IterExprAnonCall loop as a FunctionDecl, so that it qualifies under the rules of a named plain function:
+    // one per For gate and (output, input) count, its template cached like FunctionDecl::tmpl.  The entry holds the gate's
+    // Complex, so its address is not reused while the entry exists.  Its consts are the relation message's, which the
+    // entry does not own: they are set only while the template is built (anon_template) and cleared right after.
+    struct AnonKey {
+        const ir::Complex* cx;
+        uint64_t n_out, n_in;
+        bool operator<(const AnonKey& o) const { return std::tie(cx, n_out, n_in) < std::tie(o.cx, o.n_out, o.n_in); }
+    };
+    std::map<AnonKey, std::pair<std::shared_ptr<ir::Complex>, FunctionDecl>> anon_decls;
+    FunctionDecl* anon_decl(const std::shared_ptr<ir::Complex>& cx, uint64_t n_out, uint64_t n_in) {
+        if (cx->instance_count != 0 || cx->witness_count != 0) return nullptr;
+        auto it = anon_decls.find(AnonKey{cx.get(), n_out, n_in});
+        if (it == anon_decls.end()) {
+            FunctionDecl d;
+            d.body = std::shared_ptr<std::vector<ir::Gate>>(cx, &cx->body);
+            d.instance_nbr = d.witness_nbr = 0;
+            d.output_count = n_out;
+            d.input_count = n_in;
+            d.n_local = getenv("ZKB_NO_SIMPLE_CALLS") ? 0 : simple_body_locals(cx->body, n_out, n_in);
+            it = anon_decls.emplace(AnonKey{cx.get(), n_out, n_in}, std::make_pair(cx, std::move(d))).first;
+        }
+        return &it->second.second;
+    }
+    int anon_template(FunctionDecl& d, const std::vector<std::vector<uint8_t>>& consts) {
+        if (d.tmpl != -1) return d.tmpl;
+        d.consts = std::shared_ptr<std::vector<std::vector<uint8_t>>>(std::shared_ptr<void>(),
+                                                                      const_cast<std::vector<std::vector<uint8_t>>*>(&consts));
+        const int ti = template_of(d);
+        d.consts.reset();
+        return ti;
+    }
+
     // true: the whole loop has been recorded as one call group, with the state the gate-by-gate loop would leave (bindings,
     // callback counts, work accounting).  false: nothing was changed; the caller runs the loop gate by gate, which also
-    // reports every error where the reference does.
-    bool try_call_group(const ir::Complex& cx, const FunctionDecl& f, Scope& scope, Iters& iters, const uint32_t* weight) {
+    // reports every error where the reference does.  fn: the named callee; nullptr for an anonymous body (g.cx->body).
+    //
+    // An input may be CARRIED over a prime field: its wires move with the output stride S and call c reads output k of call
+    // c - d (1 <= d <= kMaxCarryLag).  Calls c < d read the d seed wires, which must be bound before the loop to level-0
+    // values or to outputs of earlier groups (groups run before the first wavefront: a gate-computed seed would not be ready).
+    bool try_call_group(const ir::Gate& gate, const FunctionDecl* fn, const std::vector<std::vector<uint8_t>>& consts, Scope& scope,
+                        Iters& iters, const uint32_t* weight) {
+        const ir::Complex& cx = *gate.cx;
         Program& p = prog();
         if (getenv("ZKB_NO_CALL_GROUPS") != nullptr || weight || p.keep_copies || p.expand_on || !p.field_set) return false;
         if (cx.last < cx.first || cx.last - cx.first < 3 || cx.last - cx.first >= (1ull << 28)) return false;
         if (!p.binary && cx.last - cx.first + 1 < kArithGroupMinCalls) return false;
-        const int ti = template_of(f);
-        if (ti < 0) return false;
+        if (fn && template_of(*fn) < 0) return false;
         const uint64_t n = cx.last - cx.first + 1;
         std::vector<AffineWire> wo, wi;
         Iters saved = iters;
@@ -634,8 +674,14 @@ struct zkb_evaluator {
         } catch (const EvalErr&) {
         }
         iters = saved;
+        if (!ok || (!fn && depth >= kMaxDepth)) return false;  // an anonymous body at the nesting limit: the unrolled loop reports it
+        FunctionDecl* anon = fn ? nullptr : anon_decl(gate.cx, wo.size(), wi.size());
+        const FunctionDecl* f = fn ? fn : anon;
+        if (!f) return false;
+        const int ti = fn ? template_of(*fn) : anon_template(*anon, consts);
+        if (ti < 0) return false;
         const Template& t = p.templates[ti];
-        if (!ok || wo.size() != t.n_out || wi.size() != t.n_in) return false;
+        if (wo.size() != t.n_out || wi.size() != t.n_in) return false;
         // outputs: every call writes its own block of unbound wires
         const uint64_t S = wo[0].stride;
         uint64_t lo = wo[0].w0, hi = wo[0].w0;
@@ -671,7 +717,31 @@ struct zkb_evaluator {
         cg.n_calls = (uint32_t)n;
         cg.n_out = t.n_out;
         cg.depth = 0;
+        uint32_t ring_regs = 0;
         for (const auto& a : wi) {
+            uint32_t lag = 0, k_out = 0;
+            if (a.stride == S)
+                for (uint32_t k = 0; k < t.n_out; k++)
+                    if (wo[k].w0 > a.w0 && (wo[k].w0 - a.w0) % S == 0 && (wo[k].w0 - a.w0) / S <= kMaxCarryLag) {
+                        lag = (uint32_t)((wo[k].w0 - a.w0) / S);
+                        k_out = k;
+                    }
+            if (lag) {  // carried: the seeds are call 0 .. lag-1's wires
+                if (p.binary) return false;
+                for (uint64_t c = 0; c < lag; c++) {
+                    const uint32_t h = scope.get(a.w0 + S * c);
+                    if (h == Scope::kNone) return false;
+                    if (is_callout(h)) cg.depth = std::max(cg.depth, p.group_of_callout(callout_index(h)).depth + 1);
+                    else if (p.kind[h] > V_WITNESS) return false;
+                    cg.seeds.push_back(h);
+                }
+                cg.carry.push_back(kCarried | (ring_regs << 16) | (lag << 8) | k_out);
+                ring_regs += lag;
+                cg.in_base.push_back(0);
+                cg.in_stride.push_back(0);
+                continue;
+            }
+            cg.carry.push_back(0);
             if (a.w0 >= (1ull << 40) || (a.stride >= (1ull << 32) && a.stride != 0)) return false;
             const uint32_t h0 = scope.get(a.w0);
             if (h0 == Scope::kNone) return false;
@@ -711,10 +781,16 @@ struct zkb_evaluator {
             cg.in_base.push_back(h0);
             cg.in_stride.push_back(st);
         }
+        if (ring_regs) {
+            if (t.n_regs + ring_regs > kMaxTemplateRegs || (p.nlimb <= 2 && n < kNarrowChainMinCalls)) return false;
+            cg.ring_regs = ring_regs;
+        } else {
+            cg.carry.clear();
+        }
         if (p.n_total_values() + n_new >= c->max_values || (uint64_t)p.n_callouts + n_new >= kMaxCallouts) return false;  // the gate-by-gate loop reports the limit
         const uint64_t n_group_asserts = n * t.assert_wire.size();
         if ((uint64_t)p.asserts.size() + n_group_asserts >= kNoSeq) return false;
-        step(n * (1 + f.body->size()));
+        step(n * (1 + f->body->size()));
         // ---- commit: the outputs are implicit values (program.h), only the scope learns about them
         c->max_values = std::min<uint64_t>(c->max_values, kCalloutBit - 256);  // explicit handles stay below the callout space
         cg.first_callout = p.n_callouts;
@@ -918,7 +994,7 @@ struct zkb_evaluator {
                     }
                     if (cnt >= 1024 && scope.sparse.empty()) scope.ensure_dense(hi, cnt);
                 }
-                if (callee && try_call_group(cx, *callee, scope, iters, weight)) {  // the whole loop as one call group
+                if ((callee || cx.body_is_anon) && try_call_group(g, callee, consts, scope, iters, weight)) {  // the whole loop as one call group
                     iters_remove(iters, cx.name);
                     break;
                 }

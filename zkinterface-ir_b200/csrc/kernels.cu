@@ -992,14 +992,71 @@ k_bool_groups(const GroupDesc* __restrict__ descs, uint32_t n_groups, uint64_t t
     }
 }
 
+// One call of a prime-field template over a thread's register file R (register r, chunk c at R[(r * NC + c) * T]), shared by
+// k_arith_groups and k_arith_chain: the body runs op by op (Montgomery arithmetic of field_ptx.cuh, constants from the
+// Montgomery const table), the previous op's result stays in registers (GroupOp::fwd), and an AssertZero tests its
+// register in place and reports seq0 + call * A + k.
+template <int N, uint32_t FORM, class V>
+__device__ __forceinline__ void arith_call(V* R, uint32_t T, const uint4* op, uint32_t n_ops, const uint32_t* __restrict__ consts_mont,
+                                           uint32_t seq0, uint32_t call, uint32_t lane, uint32_t* __restrict__ first_fail,
+                                           const TileGeom& g, const FieldParams& fp) {
+    constexpr int CW = Elem<N>::CW, NC = Elem<N>::NC;
+    auto ld_reg = [&](uint32_t* x, uint32_t r) {
+#pragma unroll
+        for (int c = 0; c < NC; c++) unpack(R[(r * NC + c) * T], x + c * CW);
+    };
+    auto st_reg = [&](uint32_t r, const uint32_t* x) {
+#pragma unroll
+        for (int c = 0; c < NC; c++) {
+            V v;
+            pack(v, x + c * CW);
+            R[(r * NC + c) * T] = v;
+        }
+    };
+    uint32_t x[N], y[N], r[N];
+#pragma unroll
+    for (int k = 0; k < N; k++) r[k] = 0;
+    for (uint32_t i = 0; i < n_ops; i++) {
+        const uint4 o = __ldg(op + 2 * i);      // dst, a, b registers, fwd
+        const uint4 m = __ldg(op + 2 * i + 1);  // kind, const index, assertion ordinal, assertions per call
+        if (m.x == AG_CONST) {
+#pragma unroll
+            for (int k = 0; k < N; k++) r[k] = __ldg(consts_mont + (size_t)m.y * N + k);
+            st_reg(o.x, r);
+            continue;
+        }
+        if (o.w & 1) {
+#pragma unroll
+            for (int k = 0; k < N; k++) x[k] = r[k];
+        } else {
+            ld_reg(x, o.y);
+        }
+        if (m.x == AG_ASSERT) {
+            const bool fail = !fe_is_zero<N>(x) && lane < g.n_valid;
+            report_fail(fail, seq0 + call * m.w + m.z, first_fail, g.batch0 + lane, false);
+            continue;
+        }
+        if (m.x == AG_ADDC || m.x == AG_MULC) {
+#pragma unroll
+            for (int k = 0; k < N; k++) y[k] = __ldg(consts_mont + (size_t)m.y * N + k);
+        } else if (o.w & 2) {
+#pragma unroll
+            for (int k = 0; k < N; k++) y[k] = r[k];
+        } else {
+            ld_reg(y, o.z);
+        }
+        if (m.x == AG_ADD || m.x == AG_ADDC) fe_add<N>(r, x, y, fp.p);
+        else fe_mont_mul_form<N, FORM>(r, x, y, fp.p, fp.n0inv);
+        st_reg(o.x, r);
+    }
+}
+
 // Call groups over a prime field: thread <-> (call, witness lane), lane fastest, so for tiles of >= 32 lanes a warp loads
 // and stores one coalesced row per 16-byte chunk of the wire store, and for narrower tiles a warp spans calls.  A call's
 // inputs are read into a register file in dynamic shared memory, laid out like the wire store with the CTA's threads as
 // lanes (chunk c of register r of thread t at ((r * NC + c) * T + t) * CW limbs: a thread's 16-byte chunks are
-// conflict-free), the body runs over it op by op (Montgomery arithmetic of field_ptx.cuh, constants from the Montgomery
-// const table), the previous op's result stays in registers (GroupOp::fwd), an AssertZero tests its register in place and
-// reports seq0 + call * A + k, and only the outputs go back to the wire store (always stored: a group output is a level-0
-// value).  thread -> group as in k_bool_groups.
+// conflict-free), arith_call runs the body over it, and only the outputs go back to the wire store (always stored: a group
+// output is a level-0 value).  thread -> group as in k_bool_groups.
 template <int N, uint32_t FORM>
 __global__ void __launch_bounds__(kGroupThreads)
 k_arith_groups(const GroupDesc* __restrict__ descs, uint32_t n_groups, uint64_t total_calls, const GroupOp* __restrict__ gops,
@@ -1033,48 +1090,108 @@ k_arith_groups(const GroupDesc* __restrict__ descs, uint32_t n_groups, uint64_t 
         const uint4 h0 = __ldg(reinterpret_cast<const uint4*>(d));      // tmpl_off, n_ops, n_out, n_in
         const uint4 h1 = __ldg(reinterpret_cast<const uint4*>(d) + 1);  // n_calls, out_slot, first_call, seq0
         const uint32_t call = call_g - h1.z;
-        uint32_t x[N], y[N], r[N];
+        uint32_t x[N];
         for (uint32_t k = 0; k < h0.w; k++) {
             const uint32_t base = __ldg(d->in_base + k), st = __ldg(d->in_stride + k);
             const uint32_t slot = st == kTableStride ? __ldg(tables + base + call) : base + st * call;
             load_elem<N>(x, store, slot, lane, g.log2_wt);
             st_reg(h0.z + k, x);
         }
-        const uint4* op = reinterpret_cast<const uint4*>(gops + h0.x);
+        arith_call<N, FORM>(R, T, reinterpret_cast<const uint4*>(gops + h0.x), h0.y, consts_mont, h1.w, call, lane, first_fail, g, fp);
+        const uint32_t out0 = h1.y + call * h0.z;
+        for (uint32_t k = 0; k < h0.z; k++) {
+            ld_reg(x, k);
+            store_elem<N>(store, out0 + k, lane, g.log2_wt, x);
+        }
+    }
+}
+
+template <int BYTES>
+__device__ __forceinline__ void chain_cp_async(void* smem_dst, const void* gmem_src) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], %2;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src), "n"(BYTES)
+                 : "memory");
+}
+
+// Carried loops over a prime field (Plan::chain_descs): thread <-> (chain, witness lane), lane fastest, and the thread walks
+// its chain's calls in order.  A chain takes at least a whole warp (lanes past the tile's idle): chains run different
+// templates, and two of them sharing a warp would take turns at every divergent op.  The register file is k_arith_groups' (shared memory, same layout), with two areas past the
+// template's registers: each carried input's ring of its last lag values (ring register + c % lag holds the value call c
+// reads: a seed for c < lag, then output k of call c - lag, written there when that call ends), and from stage0 (the
+// descriptor's first_call) kChainStages staging registers per input, which cp.async fills with the non-carried inputs of the next kChainStages
+// calls while the earlier ones run, so the wire store's latency stays off the chain.  Carried values never go through the
+// wire store; every call's outputs are stored.
+template <int N, uint32_t FORM>
+__global__ void __launch_bounds__(kGroupThreads)
+k_arith_chain(const GroupDesc* __restrict__ descs, const uint32_t* __restrict__ carry, uint32_t n_chains, const GroupOp* __restrict__ gops,
+              const uint32_t* __restrict__ tables, uint32_t* __restrict__ store, const uint32_t* __restrict__ consts_mont,
+              uint32_t* __restrict__ first_fail, TileGeom g, FieldParams fp) {
+    constexpr int CW = Elem<N>::CW, NC = Elem<N>::NC;
+    using V = typename Vec<CW>::T;
+    extern __shared__ __align__(16) uint8_t s_regs[];
+    const uint32_t T = blockDim.x;
+    V* R = reinterpret_cast<V*>(s_regs) + threadIdx.x;
+    auto ld_reg = [&](uint32_t* x, uint32_t r) {
 #pragma unroll
-        for (int k = 0; k < N; k++) r[k] = 0;
-        for (uint32_t i = 0; i < h0.y; i++) {
-            const uint4 o = __ldg(op + 2 * i);      // dst, a, b registers, fwd
-            const uint4 m = __ldg(op + 2 * i + 1);  // kind, const index, assertion ordinal, assertions per call
-            if (m.x == AG_CONST) {
+        for (int c = 0; c < NC; c++) unpack(R[(r * NC + c) * T], x + c * CW);
+    };
+    auto st_reg = [&](uint32_t r, const uint32_t* x) {
 #pragma unroll
-                for (int k = 0; k < N; k++) r[k] = __ldg(consts_mont + (size_t)m.y * N + k);
-                st_reg(o.x, r);
-                continue;
-            }
-            if (o.w & 1) {
+        for (int c = 0; c < NC; c++) {
+            V v;
+            pack(v, x + c * CW);
+            R[(r * NC + c) * T] = v;
+        }
+    };
+    const uint32_t log2_span = g.log2_wt > 5 ? g.log2_wt : 5;  // threads per chain
+    const uint64_t tid = blockIdx.x * (uint64_t)T + threadIdx.x;
+    const uint32_t lane = (uint32_t)tid & ((1u << log2_span) - 1);
+    if (tid >= ((uint64_t)n_chains << log2_span) || lane >> g.log2_wt) return;
+    const uint32_t gi = (uint32_t)(tid >> log2_span);
+    const GroupDesc* d = descs + gi;
+    const uint32_t* cw = carry + (size_t)gi * kMaxGroupInputs;
+    const uint4 h0 = __ldg(reinterpret_cast<const uint4*>(d));      // tmpl_off, n_ops, n_out, n_in
+    const uint4 h1 = __ldg(reinterpret_cast<const uint4*>(d) + 1);  // n_calls, out_slot, stage0, seq0
+    const uint32_t stage0 = h1.z;
+    const uint4* ops = reinterpret_cast<const uint4*>(gops + h0.x);
+    const V* gstore = reinterpret_cast<const V*>(store);
+    // call c's non-carried inputs -> its staging registers, asynchronously (one commit group per call, empty past the end)
+    auto stage = [&](uint32_t call) {
+        for (uint32_t k = 0; k < h0.w && call < h1.x; k++) {
+            if (__ldg(cw + k)) continue;
+            const uint32_t base = __ldg(d->in_base + k), st = __ldg(d->in_stride + k);
+            const uint32_t slot = st == kTableStride ? __ldg(tables + base + call) : base + st * call;
 #pragma unroll
-                for (int k = 0; k < N; k++) x[k] = r[k];
-            } else {
-                ld_reg(x, o.y);
-            }
-            if (m.x == AG_ASSERT) {
-                const bool fail = !fe_is_zero<N>(x) && lane < g.n_valid;
-                report_fail(fail, h1.w + call * m.w + m.z, first_fail, g.batch0 + lane, false);
-                continue;
-            }
-            if (m.x == AG_ADDC || m.x == AG_MULC) {
-#pragma unroll
-                for (int k = 0; k < N; k++) y[k] = __ldg(consts_mont + (size_t)m.y * N + k);
-            } else if (o.w & 2) {
-#pragma unroll
-                for (int k = 0; k < N; k++) y[k] = r[k];
-            } else {
-                ld_reg(y, o.z);
-            }
-            if (m.x == AG_ADD || m.x == AG_ADDC) fe_add<N>(r, x, y, fp.p);
-            else fe_mont_mul_form<N, FORM>(r, x, y, fp.p, fp.n0inv);
-            st_reg(o.x, r);
+            for (int c = 0; c < NC; c++)
+                chain_cp_async<CW * 4>(&R[((stage0 + k * kChainStages + call % kChainStages) * NC + c) * T],
+                                       gstore + ((((size_t)slot * NC + c) << g.log2_wt) + lane));
+        }
+        asm volatile("cp.async.commit_group;" ::: "memory");
+    };
+    uint32_t x[N];
+    for (uint32_t k = 0; k < h0.w; k++) {  // the seeds -> the rings
+        const uint32_t w = __ldg(cw + k);
+        if (!w) continue;
+        const uint32_t base = __ldg(d->in_base + k), ring = (w >> 16) & 0x7FFF, lag = (w >> 8) & 0xFF;
+        for (uint32_t s = 0; s < lag; s++) {
+            load_elem<N>(x, store, __ldg(tables + base + s), lane, g.log2_wt);
+            st_reg(ring + s, x);
+        }
+    }
+    for (uint32_t s = 0; s < kChainStages; s++) stage(s);
+    for (uint32_t call = 0; call < h1.x; call++) {
+        asm volatile("cp.async.wait_group %0;" ::"n"(kChainStages - 1) : "memory");  // this call's group has landed
+        for (uint32_t k = 0; k < h0.w; k++) {
+            const uint32_t w = __ldg(cw + k);
+            ld_reg(x, w ? ((w >> 16) & 0x7FFF) + call % ((w >> 8) & 0xFF) : stage0 + k * kChainStages + call % kChainStages);
+            st_reg(h0.z + k, x);
+        }
+        stage(call + kChainStages);
+        arith_call<N, FORM>(R, T, ops, h0.y, consts_mont, h1.w, call, lane, first_fail, g, fp);
+        for (uint32_t k = 0; k < h0.w; k++) {  // output k of this call is what call + lag reads
+            const uint32_t w = __ldg(cw + k);
+            if (!w) continue;
+            ld_reg(x, w & 0xFF);
+            st_reg(((w >> 16) & 0x7FFF) + call % ((w >> 8) & 0xFF), x);
         }
         const uint32_t out0 = h1.y + call * h0.z;
         for (uint32_t k = 0; k < h0.z; k++) {
@@ -1578,6 +1695,32 @@ void launch_arith_groups(int nlimb, const GroupDesc* descs, uint32_t n_groups, u
     else
         ZKB_DISPATCH_N(nlimb, (launch_arith_groups_n<N, kMulFormGeneric>(descs, n_groups, total_calls, gops, tables, hints, store, consts_mont,
                                                                          first_fail, g, fp, n_regs, sm_count, s)));
+}
+
+// CTA size: as k_arith_groups' (two CTAs per SM), and smaller while that leaves SMs idle: each thread is a serial walk,
+// latency-bound, so the threads are spread over the SMs rather than stacked on a few
+template <int N, uint32_t FORM>
+static void launch_arith_chain_n(const GroupDesc* descs, const uint32_t* carry, uint32_t n_chains, const GroupOp* gops, const uint32_t* tables,
+                                 uint32_t* store, const uint32_t* consts_mont, uint32_t* first_fail, TileGeom g, const FieldParams& fp,
+                                 uint32_t n_regs, int sm_count, cudaStream_t s) {
+    static std::atomic<uint64_t> attr_seen{0};
+    if (first_on_device(attr_seen)) cudaFuncSetAttribute(k_arith_chain<N, FORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kArithGroupSmemPerCta);
+    const uint64_t threads = (uint64_t)n_chains << (g.log2_wt > 5 ? g.log2_wt : 5);  // a warp at least per chain
+    uint32_t T = arith_group_threads(N, n_regs);
+    while (T > 32 && (threads + T - 1) / T < (uint64_t)sm_count) T >>= 1;
+    const size_t smem = (size_t)n_regs * N * 4 * T;
+    k_arith_chain<N, FORM><<<(unsigned)((threads + T - 1) / T), T, smem, s>>>(descs, carry, n_chains, gops, tables, store, consts_mont, first_fail,
+                                                                            g, fp);
+}
+void launch_arith_chain(int nlimb, const GroupDesc* descs, const uint32_t* carry, uint32_t n_chains, const GroupOp* gops, const uint32_t* tables,
+                        uint32_t* store, const uint32_t* consts_mont, uint32_t* first_fail, TileGeom g, const FieldParams& fp, uint32_t n_regs,
+                        int sm_count, cudaStream_t s) {
+    if (n_chains == 0) return;
+    if (nlimb == 8 && fp.mul_form == kMulFormLow64)
+        launch_arith_chain_n<8, kMulFormLow64>(descs, carry, n_chains, gops, tables, store, consts_mont, first_fail, g, fp, n_regs, sm_count, s);
+    else
+        ZKB_DISPATCH_N(nlimb, (launch_arith_chain_n<N, kMulFormGeneric>(descs, carry, n_chains, gops, tables, store, consts_mont, first_fail, g,
+                                                                        fp, n_regs, sm_count, s)));
 }
 
 void launch_bool_read_values(const uint32_t* slots, uint32_t n, const uint32_t* store, uint32_t lane, uint32_t log2_wt,

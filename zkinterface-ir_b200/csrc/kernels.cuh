@@ -75,6 +75,11 @@ void launch_arith_groups(int nlimb, const GroupDesc* descs, uint32_t n_groups, u
                          const uint32_t* hints, uint32_t* store, const uint32_t* consts_mont, uint32_t* first_fail, TileGeom g,
                          const FieldParams& fp, uint32_t n_regs, int sm_count, cudaStream_t s);
 uint32_t arith_group_threads(int nlimb, uint32_t n_regs);  // its CTA size
+// carried loops of one depth (k_arith_chain, Plan::chain_descs): carry = their Plan::chain_carry rows, n_regs = Plan::chain_regs
+// (rings and staging registers included)
+void launch_arith_chain(int nlimb, const GroupDesc* descs, const uint32_t* carry, uint32_t n_chains, const GroupOp* gops, const uint32_t* tables,
+                        uint32_t* store, const uint32_t* consts_mont, uint32_t* first_fail, TileGeom g, const FieldParams& fp, uint32_t n_regs,
+                        int sm_count, cudaStream_t s);
 void launch_read_values(int nlimb, const uint32_t* slots, uint32_t n, const uint32_t* store, uint32_t lane, uint32_t log2_wt,
                         uint32_t* out, const FieldParams& fp, cudaStream_t s);
 

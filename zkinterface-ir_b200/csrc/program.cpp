@@ -275,14 +275,17 @@ void Plan::build(const Program& prog, bool keep_all, const std::vector<uint32_t>
         size_t operator()(const Progression& p) const { return ((size_t)p.base * 0x9E3779B97F4A7C15ull) ^ ((size_t)p.stride << 32) ^ p.n; }
     };
     std::unordered_map<Progression, std::pair<uint32_t, uint32_t>, ProgressionHash> progressions;  // -> (slot stride | kTableStride, table offset)
-    for (const CallGroup& cg : prog.groups)
+    for (const CallGroup& cg : prog.groups) {
+        for (uint32_t h : cg.seeds)
+            if (!is_callout(h)) used[h] = 1;
         for (size_t k = 0; k < cg.in_base.size(); k++) {
             const uint32_t b = cg.in_base[k], st = cg.in_stride[k];
-            if (is_callout(b)) continue;
+            if (is_callout(b) || (cg.carried() && cg.carry[k])) continue;
             if (!progressions.emplace(Progression{b, st, st ? cg.n_calls : 1}, std::make_pair(0u, 0u)).second) continue;
             if (st == 0) used[b] = 1;
             else for (uint32_t c = 0; c < cg.n_calls; c++) used[b + st * c] = 1;
         }
+    }
     lap("levels");
     // earliest assert per value (a value that is non-zero fails at its first assert)
     std::vector<uint32_t> aseq(n, kNoSeq);
@@ -709,6 +712,10 @@ void Plan::build(const Program& prog, bool keep_all, const std::vector<uint32_t>
     hint_off.clear();
     depth_off.clear();
     group_regs = 0;
+    chain_descs.clear();
+    chain_carry.clear();
+    chain_off.clear();
+    chain_regs = 0;
     if (!prog.groups.empty()) {
         std::vector<uint32_t> tmpl_off(prog.templates.size());
         for (size_t t = 0; t < prog.templates.size(); t++) {
@@ -765,10 +772,17 @@ void Plan::build(const Program& prog, bool keep_all, const std::vector<uint32_t>
         uint32_t max_depth = 0;
         for (const CallGroup& cg : prog.groups) max_depth = std::max(max_depth, cg.depth);
         depth_off.assign((size_t)max_depth + 2, 0);
-        for (const CallGroup& cg : prog.groups) depth_off[cg.depth + 1]++;
-        for (size_t d = 0; d + 1 < depth_off.size(); d++) depth_off[d + 1] += depth_off[d];
+        chain_off.assign((size_t)max_depth + 2, 0);
+        for (const CallGroup& cg : prog.groups) (cg.carried() ? chain_off : depth_off)[cg.depth + 1]++;
+        for (size_t d = 0; d + 1 < depth_off.size(); d++) {
+            depth_off[d + 1] += depth_off[d];
+            chain_off[d + 1] += chain_off[d];
+        }
         std::vector<uint32_t> cursor(depth_off.begin(), depth_off.end() - 1), calls_before((size_t)max_depth + 1, 0);
-        group_descs.resize(prog.groups.size());
+        std::vector<uint32_t> chain_cursor(chain_off.begin(), chain_off.end() - 1);
+        group_descs.resize(depth_off.back());
+        chain_descs.resize(chain_off.back());
+        chain_carry.assign(chain_descs.size() * kMaxGroupInputs, 0);
         for (const CallGroup& cg : prog.groups) {
             const Template& tp = prog.templates[cg.tmpl];
             GroupDesc gd{};
@@ -778,11 +792,25 @@ void Plan::build(const Program& prog, bool keep_all, const std::vector<uint32_t>
             gd.n_in = tp.n_in;
             gd.n_calls = cg.n_calls;
             gd.out_slot = callout_slot0 + cg.first_callout;
-            gd.first_call = calls_before[cg.depth];
             gd.pad = prog.binary ? 0 : cg.seq0;
-            calls_before[cg.depth] += cg.n_calls;
+            const uint32_t chain = cg.carried() ? chain_cursor[cg.depth]++ : 0;
+            if (cg.carried()) {
+                gd.first_call = tp.n_regs + cg.ring_regs;
+                chain_regs = std::max(chain_regs, gd.first_call + tp.n_in * kChainStages);
+            } else {
+                gd.first_call = calls_before[cg.depth];
+                calls_before[cg.depth] += cg.n_calls;
+            }
+            const uint32_t* seed = cg.seeds.data();
             for (uint32_t k = 0; k < tp.n_in; k++) {
                 const uint32_t b = cg.in_base[k], st = cg.in_stride[k];
+                if (cg.carried() && cg.carry[k]) {  // the seeds' slots, then the ring past the template's registers
+                    const uint32_t w = cg.carry[k], lag = (w >> 8) & 0xFF;
+                    gd.in_base[k] = (uint32_t)group_tables.size();
+                    for (uint32_t s = 0; s < lag; s++) group_tables.push_back(slot_of(*seed++));
+                    chain_carry[(size_t)chain * kMaxGroupInputs + k] = (w & ~(0x7FFFu << 16)) | ((tp.n_regs + ((w >> 16) & 0x7FFF)) << 16);
+                    continue;
+                }
                 if (is_callout(b)) {  // outputs of earlier groups: consecutive indices are consecutive slots
                     gd.in_base[k] = slot_of(b);
                     gd.in_stride[k] = st;
@@ -813,7 +841,8 @@ void Plan::build(const Program& prog, bool keep_all, const std::vector<uint32_t>
                     gd.in_stride[k] = kTableStride;
                 }
             }
-            group_descs[cursor[cg.depth]++] = gd;
+            if (cg.carried()) chain_descs[chain] = gd;
+            else group_descs[cursor[cg.depth]++] = gd;
         }
         // thread -> group: a hint per 2^kGroupHintShift calls of a launch, then a short forward walk over first_call
         group_hints.clear();

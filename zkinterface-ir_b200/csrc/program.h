@@ -85,7 +85,22 @@ struct CallGroup {
     std::vector<uint32_t> in_base, in_stride;  // per input position: handle of call c's input = base + stride * c
     uint32_t n_out = 0;
     uint32_t seq0 = 0;  // assertion sequence number of call 0's first AssertZero (templates with assertions)
+    // carried loops (prime fields): per input position, 0 or kCarried | ring << 16 | lag << 8 | output position (call c reads
+    // output k of call c - lag; ring = the input's first ring register past the template's own); empty when nothing is carried
+    std::vector<uint32_t> carry;
+    std::vector<uint32_t> seeds;  // handles that calls 0 .. lag-1 read, lag per carried input, in input order
+    uint32_t ring_regs = 0;
+    bool carried() const { return !carry.empty(); }
 };
+// A carried loop is a chain: call c needs call c - lag's output.  It runs in k_arith_chain, one thread per (group, lane)
+// walking the calls in order with the last lag outputs in registers of a ring, which count against kMaxTemplateRegs.
+constexpr uint32_t kMaxCarryLag = 4;
+constexpr uint32_t kCarried = 0x80000000u;
+// Over fields of one or two limbs a chain walks its calls no faster than the level path runs two one-gate wavefronts per call
+// at one witness (DESIGN.md section 5.0e: Goldilocks, 2^12 and 2^16 calls slower grouped, 2^20 faster): such carried loops
+// qualify only from kNarrowChainMinCalls calls on.  Wider fields were faster grouped at every measured size.
+constexpr uint64_t kNarrowChainMinCalls = 1ull << 20;
+constexpr uint32_t kChainStages = 8;  // calls whose non-carried inputs k_arith_chain has in flight ahead of the running one
 
 // callback counters (one per ZKBackend method that the Evaluator drives)
 enum CbKind { CB_CONSTANT = 0, CB_INSTANCE, CB_WITNESS, CB_ADD, CB_MUL, CB_ADDC, CB_MULC, CB_AND, CB_XOR,
@@ -323,6 +338,15 @@ struct Plan {
     std::vector<uint32_t> group_tables;
     std::vector<uint32_t> depth_off;
     uint32_t group_regs = 0;  // registers of the widest template
+    // carried loops (k_arith_chain), one launch per depth next to that depth's group launch: chain_off[d] .. chain_off[d + 1]
+    // are the chains of depth d (chain_off has depth_off's length).  A carried input k of chain i has chain_carry[i *
+    // kMaxGroupInputs + k] = kCarried | ring register << 16 | lag << 8 | output position, and its lag seed slots at
+    // group_tables[in_base[k]]; other inputs have 0 there and read as in a GroupDesc.  A chain's first_call is its first
+    // staging register (past its template's registers and rings), kChainStages of them per input
+    std::vector<GroupDesc> chain_descs;
+    std::vector<uint32_t> chain_carry;
+    std::vector<uint32_t> chain_off;
+    uint32_t chain_regs = 0;  // registers of the widest chain, its rings and staging registers included
     uint32_t callout_slot0 = 0, n_callouts = 0;  // group outputs: slot of implicit value i = callout_slot0 + i
     uint32_t slot_of(uint32_t h) const { return is_callout(h) ? callout_slot0 + callout_index(h) : slot_of_value[h]; }
     bool is_readable(uint32_t h) const { return is_callout(h) || readable[h]; }
