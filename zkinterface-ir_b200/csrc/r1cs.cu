@@ -559,6 +559,9 @@ extern "C" int zkb_debug_r1cs_layout(zkb_ctx* c, int kind, uint64_t counts[3], u
 extern "C" int zkb_r1cs_upload(zkb_ctx* c, const uint8_t* z_le, uint64_t z_set_stride, uint32_t value_stride, uint32_t n_batch) {
     R1csDev* r = c->r1cs;
     if (!r) return c->fail(ZKB_E_ARG, "zkb_r1cs_load must be called first");
+    // a failed upload leaves nothing to run: the device buffers may already hold the new bytes (build_layout can reject
+    // the new tile width's layout after the copy) while n_batch / stride / log2_wt still describe the previous upload
+    r->uploaded = false;
     if (!c->has_gpu) return c->fail(ZKB_E_CUDA, "no CUDA device in this context (there is no CPU fallback)");
     if (n_batch == 0 || value_stride == 0) return c->fail(ZKB_E_ARG, "n_batch and value_stride must be > 0");
     if (n_batch > 1 && z_set_stride < r->n_vars * value_stride) return c->fail(ZKB_E_ARG, "z_set_stride smaller than one assignment vector");
